@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: O1280 -> TriNodes(7) encoder / processor / decoder graph, edges per second.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 One STEP = one complete pass of the edge-construction path over the workload: hidden TriNodes generation
 (icosphere subdivision kernels + the host node ordering the reference defines), CutOffEdges 0.6 encoder
@@ -19,6 +19,8 @@ synthetic (octahedral reduced Gaussian grid, ``anemoi_graphs_b200.grids``) and a
   timed on this host's cores on a bounded sample of the same workload, with its error against a full pass stated.
 * ``--impl reference``: ONE full, unsampled pass of the UNMODIFIED reference (``oracle/_ref``, vendored byte for byte by
   ``oracle/build_ref.py``) through its own ``GraphCreator.update_graph`` on the box's host cores.
+* ``--dump-outputs DIR``: what the last timed ``value`` step returned, as ``DIR/<name>.npy`` (``dump_outputs``), so two
+  builds of the project can be compared output for output on identical inputs.
 
 Multi-GPU (torchrun, one rank per GPU): sharded OUTPUT mode - query (target) nodes are sharded by rank, reference nodes
 replicated, nothing is exchanged between the GPUs except the attribute statistics (8 doubles per rank).  ``value``
@@ -187,6 +189,34 @@ def output_bytes(graph) -> int:
     return n
 
 
+DUMP_EDGES_PER_SET = 1 << 19  # 28 bytes per dumped edge: the three edge sets stay below 64 MB together
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(graph, out_dir: pathlib.Path) -> None:
+    """Write the graph one step returned as ``out_dir/<name>.npy``: the hidden node coordinates and, for every edge set,
+    ``<src>_to_<dst>_edge_index`` (float64, exact for int32 ids), ``_edge_length`` and ``_edge_dirs`` (float32).  Edges
+    are in canonical (target, source) order, so the files do not depend on the order the kernels emit an edge set in; a
+    set larger than ``DUMP_EDGES_PER_SET`` is sampled at fixed seeded positions of that order."""
+    arrays = {"hidden_x": graph["hidden"].x.cpu().numpy()}
+    for key in EDGE_KEYS:
+        store = graph[key]
+        ei = store.edge_index
+        order = torch.argsort(ei[1].long() * graph[key[0]].x.shape[0] + ei[0].long())
+        n = int(order.numel())
+        if n > DUMP_EDGES_PER_SET:
+            pick = np.sort(np.random.default_rng(0).choice(n, size=DUMP_EDGES_PER_SET, replace=False))
+            order = order[torch.from_numpy(pick).to(order.device)]
+        name = f"{key[0]}_to_{key[2]}"
+        arrays[f"{name}_edge_index"] = ei[:, order].cpu().numpy().astype(np.float64)
+        arrays[f"{name}_edge_length"] = store["edge_length"][order].cpu().numpy()
+        arrays[f"{name}_edge_dirs"] = store["edge_dirs"][order].cpu().numpy()
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def sharding_note(world: int) -> str:
     if world == 1:
         return "single GPU"
@@ -226,6 +256,8 @@ def bench_b200(args) -> dict:
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the product path has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single process: a sharded device-resident graph holds one rank's block")
     torch.cuda.set_device(local_rank)
     shared_host = True
     if world > 1:
@@ -296,6 +328,8 @@ def bench_b200(args) -> dict:
     ms_per_step = ms_total / args.steps
     value = n_edges / (ms_per_step * 1e-3)
     n_data, n_hidden = int(x_dev.shape[0]), int(graph["hidden"].x.shape[0])
+    if args.dump_outputs:
+        dump_outputs(graph, pathlib.Path(args.dump_outputs))
     del graph
     if world > 1:
         t = torch.tensor([launches], dtype=torch.int64, device="cuda")
@@ -677,7 +711,12 @@ def main() -> None:
     ap.add_argument("--workload", default="o1280_res7", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=20.0, help="seconds of CPU work for the cpu_baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's graph as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the b200 arm's outputs")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     line = bench_reference(args) if args.impl == "reference" else bench_b200(args)
     if line:
