@@ -208,7 +208,7 @@ __global__ void __launch_bounds__(256) k_flagged_tiles(const uint8_t* __restrict
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n_tiles; t += (int64_t)gridDim.x * blockDim.x) {
         bool any = false;
         if (t * 32 + 32 <= nq) {
-            const uint4* w = (const uint4*)(flags + t * 32);  // 32-byte aligned: cudaMalloc'ed base, t * 32
+            const uint4* w = (const uint4*)(flags + t * 32);  // 16-byte aligned: base checked by the entry points, t * 32
             uint4 a = w[0], b = w[1];
             any = (a.x | a.y | a.z | a.w | b.x | b.y | b.z | b.w) != 0u;
         } else {
@@ -391,46 +391,30 @@ __global__ void __launch_bounds__(KNN_WARPS * 32) k_knn(KnnArgs a) {
             dk = top.d_at(k - 1);
             rest_lb = top.d_at(k);  // +inf when there is no (k+1)-th candidate
         }
-        if (limited) {
-            // fewer than k provable neighbours inside the search limit: report what was found there (-1 / +inf for
-            // the missing ones); anything reported is farther than max_radius or exact (see agx_b200.h)
-            if (active) {
-                int32_t* os = a.out_src + q * k;
-#pragma unroll
-                for (int s = 0; s < CAP - 1; ++s)
-                    if (s < k) {
-                        bool have = top.id[s] != 0x7fffffff;
-                        os[s] = have ? knn_out_label(a, top.id[s]) : -1;
-                        if (a.out_rdist)
-                            a.out_rdist[q * k + s] = have ? agx_rdist64(ql, a.ref_latlon[top.id[s]]) : __longlong_as_double(0x7ff0000000000000ll);
-                    }
-                if (a.out_dst) {
-                    int32_t* od = a.out_dst + q * k;
-                    for (int s = 0; s < k; ++s) od[s] = knn_dst_label(a, q);
-                }
-            }
-        }
         // ---- decide the set --------------------------------------------------------------------------
+        // A `limited` lane found fewer than k provable neighbours inside the search limit: it reports what it found
+        // there, every point within max_radius among them, and -1 / +inf for the missing slots (see agx_b200.h).
         float amb = dk + 2.5f * agx_chord2_margin(dk);  // d_k + 2 margins
-        bool ambiguous = (CAP > 1) && (rest_lb <= amb);
-        if (active && !limited) {
+        bool ambiguous = !limited && (CAP > 1) && (rest_lb <= amb);
+        if (active) {
             int32_t* os = a.out_src + q * k;
             if (!ambiguous) {
                 if (a.out_rdist == nullptr) {
 #pragma unroll
                     for (int s = 0; s < CAP - 1; ++s)
-                        if (s < k) os[s] = knn_out_label(a, top.id[s]);
-                } else {
+                        if (s < k) os[s] = top.id[s] != 0x7fffffff ? knn_out_label(a, top.id[s]) : -1;
+                } else {  // ascending (rdist, index), the missing slots last
                     TopD<CAP> fin;
                     fin.reset();
 #pragma unroll
                     for (int s = 0; s < CAP - 1; ++s)
-                        if (s < k) fin.insert(agx_rdist64(ql, a.ref_latlon[top.id[s]]), top.id[s]);
+                        if (s < k && top.id[s] != 0x7fffffff) fin.insert(agx_rdist64(ql, a.ref_latlon[top.id[s]]), top.id[s]);
 #pragma unroll
                     for (int s = 0; s < CAP - 1; ++s)
                         if (s < k) {
-                            os[s] = knn_out_label(a, fin.id[s]);
-                            a.out_rdist[q * k + s] = fin.r[s];
+                            bool have = fin.id[s] != 0x7fffffff;
+                            os[s] = have ? knn_out_label(a, fin.id[s]) : -1;
+                            a.out_rdist[q * k + s] = have ? fin.r[s] : __longlong_as_double(0x7ff0000000000000ll);
                         }
                 }
             } else {
@@ -569,6 +553,7 @@ extern "C" int agx_knn_flagged(const agx_index_t* ix, const float* q_latlon, int
 extern "C" int agx_knn_redecide(const agx_index_t* ix, const float* q_latlon, int64_t nq, int k, double max_radius,
                                 int32_t* out_src, const uint8_t* tie_flags, void* stream_) {
     AGX_REQUIRE(tie_flags != nullptr, AGX_ERR_ARG, "agx_knn_redecide: tie_flags is NULL");
+    AGX_REQUIRE(((uintptr_t)tie_flags & 15) == 0, AGX_ERR_ARG, "agx_knn_redecide: tie_flags must be 16-byte aligned");
     return agx_knn_ex(ix, q_latlon, nq, k, max_radius, out_src, nullptr, 0, nullptr, nullptr, (uint8_t*)tie_flags, 1, nullptr,
                       nullptr, stream_);
 }
@@ -577,6 +562,7 @@ extern "C" int agx_knn_redecide_ranked(const agx_index_t* ix, const float* q_lat
                                        int32_t* out_src, const uint8_t* tie_flags, const int64_t* rank,
                                        const int64_t* order, void* stream_) {
     AGX_REQUIRE(tie_flags != nullptr, AGX_ERR_ARG, "agx_knn_redecide_ranked: tie_flags is NULL");
+    AGX_REQUIRE(((uintptr_t)tie_flags & 15) == 0, AGX_ERR_ARG, "agx_knn_redecide_ranked: tie_flags must be 16-byte aligned");
     AGX_REQUIRE(rank != nullptr && order != nullptr, AGX_ERR_ARG, "agx_knn_redecide_ranked: rank / order is NULL");
     return agx_knn_ex(ix, q_latlon, nq, k, max_radius, out_src, nullptr, 0, nullptr, nullptr, (uint8_t*)tie_flags, 1, rank,
                       order, stream_);

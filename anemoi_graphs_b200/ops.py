@@ -125,10 +125,12 @@ class NeighbourIndex:
     ):
         """``edge_index`` (2, nq*k) int32 - row 0 the k nearest reference points of each query, row 1
         ``dst_base + query`` - and optionally the float64 ``rdist`` (nq, k).  With ``out`` (a larger
-        contiguous (2, E) int32 buffer) the block is written at column ``out_offset`` instead.  ``max_radius``
-        (radians, 0 = unlimited) bounds the search: exact for queries whose k-th neighbour is within it, otherwise
-        -1 / +inf or points beyond it (``agx_b200.h``).  ``tie_flags`` (zeroed uint8 (nq,)) marks the queries whose result
-        depends on the numbering of the reference points (``agx_knn_flagged``)."""
+        contiguous (2, E) int32 buffer) the block is written at column ``out_offset`` instead.  Each query's k sources
+        are a SET; only with ``return_rdist`` is a row ordered, ascending (rdist, index).  ``max_radius`` (radians,
+        0 = unlimited) bounds the search: exact for queries whose k-th neighbour is within it; any other query gets
+        every point within it, and -1 / +inf or points beyond it in the other slots (``agx_b200.h``).  ``tie_flags``
+        (zeroed uint8 (nq,)) marks the queries whose result depends on the numbering of the reference points
+        (``agx_knn_flagged``)."""
         q = _dev_x(q)
         nq = int(q.shape[0])
         if out is None:
@@ -160,6 +162,7 @@ class NeighbourIndex:
         nq = int(q.shape[0])
         assert out.shape == (2, nq * k) and out.dtype == torch.int32 and out.is_contiguous()
         assert tie_flags.shape == (nq,) and tie_flags.dtype == torch.uint8
+        assert tie_flags.is_cuda and tie_flags.is_contiguous()  # the library checks the 16-byte alignment
         with _span("knn_ties", nq):
             if rank is None:
                 check(self.lib.agx_knn_redecide(self.handle, ptr(q), nq, int(k), 0.0, out.data_ptr(), ptr(tie_flags), current_stream()))

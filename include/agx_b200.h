@@ -65,19 +65,22 @@ int agx_search_vectors(const float* latlon /*DEV n*2*/, int64_t n, float* xyz /*
 
 /* ---- KNN --------------------------------------------------------------------------------------
  * Replaces `kneighbors_graph(target, n_neighbors=k)` / `kneighbors(...)` (edges/builder.py:261-265,
- * utils.py:62, generate/masks.py:97).  For query q (0 <= q < nq) writes its k nearest reference
- * points, ascending (distance, index), to out_src[q*k .. q*k+k); if out_dst != NULL also
- * out_dst[q*k+j] = dst_base + q (so (out_src, out_dst) are the two rows of edge_index,
- * edges/builder.py:86-87).  Decisions are float64 haversine `rdist` on the float32 inputs
- * (sklearn _dist_metrics.pyx.tp:2639-2648); ties within 2^-40 relative go to the lower index.
- * out_rdist (optional, nq*k) receives the float64 rdist of every neighbour.
+ * utils.py:62, generate/masks.py:97).  For query q (0 <= q < nq) writes the SET of its k nearest
+ * reference points to out_src[q*k .. q*k+k); if out_dst != NULL also out_dst[q*k+j] = dst_base + q
+ * (so (out_src, out_dst) are the two rows of edge_index, edges/builder.py:86-87).  Decisions are
+ * float64 haversine `rdist` on the float32 inputs (sklearn _dist_metrics.pyx.tp:2639-2648); ties
+ * within 2^-40 relative go to the lower index.  out_rdist (optional, nq*k) receives the float64 rdist
+ * of every neighbour; with it each row is ascending (rdist, index) under that tie rule.  Without it
+ * only the set is defined: the order inside a row is the filter's (FP32 chord, truncated by up to
+ * 2^-14 relative) and may differ between runs that process the queries in a different order.
  * stats (optional, DEV int64[4]) += {queries refined in float64, queries with a tie at the k-th
  * boundary, queries needing a wider search, (query, candidate) pairs evaluated by the staged scans on the FP32 pipe}.
  * max_radius (radians; 0 = unlimited) bounds the search, for callers that only ask "is anything within r?"
  * (KNNAreaMaskBuilder.get_mask compares the distance with a margin, generate/masks.py:94-99 - without the bound a
  * query far from a clustered reference set walks the whole sphere): a query whose k-th neighbour lies within
- * max_radius is answered exactly; otherwise the slots hold reference points found inside the bound, each of them
- * farther than max_radius, or -1 with rdist = +inf.                                                          */
+ * max_radius is answered exactly.  For any other query the row holds EVERY reference point within max_radius
+ * (with its exact rdist); the remaining slots hold distinct points farther than max_radius, or -1 with
+ * rdist = +inf (with out_rdist: after the points, ascending as above).                                      */
 int agx_knn(const agx_index_t* index, const float* q_latlon /*DEV nq*2*/, int64_t nq, int k, double max_radius,
             int32_t* out_src /*DEV*/, int32_t* out_dst /*DEV or NULL*/, int64_t dst_base,
             double* out_rdist /*DEV or NULL*/, int64_t* stats /*DEV or NULL*/, void* stream);
@@ -93,9 +96,11 @@ int agx_knn_flagged(const agx_index_t* index, const float* q_latlon /*DEV nq*2*/
 
 /* The second half: searches ONLY the queries whose tie_flags byte is set (against an index built over the finally
  * numbered reference points) and overwrites their k slots of out_src; every other query is left untouched.  No
- * compaction and no read-back: a tile of 32 queries without a flagged one costs 32 bytes of traffic.              */
+ * compaction and no read-back: a tile of 32 queries without a flagged one costs 32 bytes of traffic, read as two
+ * 16-byte words - so tie_flags must be 16-byte aligned (AGX_ERR_ARG otherwise; a cudaMalloc'ed base is, and so is
+ * flags + 16 m).                                                                                                */
 int agx_knn_redecide(const agx_index_t* index, const float* q_latlon /*DEV nq*2*/, int64_t nq, int k, double max_radius,
-                     int32_t* out_src /*DEV nq*k*/, const uint8_t* tie_flags /*DEV nq*/, void* stream);
+                     int32_t* out_src /*DEV nq*k*/, const uint8_t* tie_flags /*DEV nq, 16-byte aligned*/, void* stream);
 
 /* The same re-decision WITHOUT a second index: `index` is still the one built over the provisionally numbered points
  * (the one agx_knn_flagged searched).  Ties go to the lower FINAL label rank[provisional label]; the k slots are
@@ -112,8 +117,9 @@ int agx_knn_redecide_list(const agx_index_t* index, const float* q_latlon /*DEV 
 int agx_compact_flags(const uint8_t* flags /*DEV n, 4-byte aligned*/, int64_t n, int32_t* list /*DEV n*/,
                       int64_t* count /*DEV 1*/, void* stream);
 int agx_knn_redecide_ranked(const agx_index_t* index, const float* q_latlon /*DEV nq*2*/, int64_t nq, int k,
-                            double max_radius, int32_t* out_src /*DEV nq*k*/, const uint8_t* tie_flags /*DEV nq*/,
-                            const int64_t* rank /*DEV*/, const int64_t* order /*DEV*/, void* stream);
+                            double max_radius, int32_t* out_src /*DEV nq*k*/,
+                            const uint8_t* tie_flags /*DEV nq, 16-byte aligned*/, const int64_t* rank /*DEV*/,
+                            const int64_t* order /*DEV*/, void* stream);
 
 /* Query order of the tile kernels.  agx_knn / agx_radius_* decide per call whether to walk the queries as given or in
  * a spatially binned order; for >= 262 144 queries the decision samples tile plans and synchronises the stream.
