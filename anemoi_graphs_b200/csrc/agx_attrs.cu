@@ -629,6 +629,9 @@ __global__ void k_attr_params(double* __restrict__ ws, const double* __restrict_
                 double sd = var > 0.0 ? sqrt(var) : 0.0;
                 div = sd == 0.0 ? 1.0 : sd;  // normalise.py:46-50: skipped when std == 0
             }
+            // a NaN value (an antipodal pair's length) makes numpy's sum, amax, amin and std NaN, so the reference
+            // returns NaN everywhere; the sum carries the NaN here, the minimum / maximum (fminf / fmaxf) do not
+            if (isnan(S[0])) div = __longlong_as_double(0x7ff8000000000000ll);
         }
         if (which == 0) {
             ws[0] = shift;
@@ -662,6 +665,13 @@ static int attrs_check(const int32_t* edge_src, const int32_t* edge_dst, int64_t
     AGX_REQUIRE(((uintptr_t)nd.src_rec & 15) == 0 && ((uintptr_t)nd.dst_rec & 15) == 0 && ((uintptr_t)nd.src_ll & 7) == 0 &&
                     ((uintptr_t)nd.dst_ll & 7) == 0,
                 AGX_ERR_ARG, "agx_edge_attrs: node records must be 16-byte, coordinates 8-byte aligned");
+    return AGX_OK;
+}
+
+// the per-edge kernels store a direction as one float2 (J = 1 lanes, k_edge_attrs_regular): a 4-byte aligned out_dir
+// (a view that starts at an odd float) would fault there, so every entry point refuses it before any device work
+static int attrs_check_dir(const float* out_dir) {
+    AGX_REQUIRE(((uintptr_t)out_dir & 7) == 0, AGX_ERR_ARG, "agx_edge_attrs: out_dir must be 8-byte aligned");
     return AGX_OK;
 }
 
@@ -821,7 +831,7 @@ extern "C" int agx_edge_attrs_stats_flagged(const int32_t* edge_src, const int32
                 AGX_ERR_ARG, "agx_edge_attrs_stats_flagged: flag_mode must be 0, 1 (skip) or 2 (only) with dst_flags");
     const AttrNodes nd = {src_rec, src_latlon, dst_rec, dst_latlon};
     int rc = attrs_check(edge_src, edge_dst, n_edges, nd, workspace);
-    if (rc) return rc;
+    if (rc || (rc = attrs_check_dir(out_dir))) return rc;
     bool write = (want_len && out_len) || (want_dir && out_dir);
     AGX_REQUIRE(!write || ((!want_len || out_len) && (!want_dir || out_dir)), AGX_ERR_ARG,
                 "agx_edge_attrs_stats: give every requested output buffer or none");
@@ -842,7 +852,7 @@ extern "C" int agx_edge_attrs_stats_list(const int32_t* edge_src, const int32_t*
     AGX_REQUIRE(regular_k > 0 && n_edges % regular_k == 0, AGX_ERR_ARG, "agx_edge_attrs_stats_list: n_edges is not a multiple of k");
     const AttrNodes nd = {src_rec, src_latlon, dst_rec, dst_latlon};
     int rc = attrs_check(edge_src, edge_dst, n_edges, nd, workspace);
-    if (rc) return rc;
+    if (rc || (rc = attrs_check_dir(out_dir))) return rc;
     AGX_REQUIRE((!want_len || out_len) && (!want_dir || out_dir), AGX_ERR_ARG,
                 "agx_edge_attrs_stats_list: give every requested output buffer");
     return attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, 0, out_len, want_dir, dir_rotated, out_dir, true, stats,
@@ -863,6 +873,7 @@ extern "C" int agx_edge_attrs_apply(const int32_t* edge_src, const int32_t* edge
         int rc = attrs_check(edge_src, edge_dst, n_edges, nd, workspace);
         if (rc) return rc;
     }
+    if (int rc = attrs_check_dir(out_dir)) return rc;
     AGX_REQUIRE(workspace != nullptr, AGX_ERR_ARG, "agx_edge_attrs_apply: workspace is NULL");
     AGX_REQUIRE(!want_len || out_len, AGX_ERR_ARG, "agx_edge_attrs: out_len is NULL");
     AGX_REQUIRE(!want_dir || out_dir, AGX_ERR_ARG, "agx_edge_attrs: out_dir is NULL");
@@ -890,7 +901,7 @@ extern "C" int agx_edge_attrs(const int32_t* edge_src, const int32_t* edge_dst, 
     AGX_REQUIRE(len_norm <= AGX_NORM_UNIT_STD && dir_norm <= AGX_NORM_UNIT_STD, AGX_ERR_ARG, "agx_edge_attrs: unknown norm code");
     const AttrNodes nd = {src_rec, src_latlon, dst_rec, dst_latlon};
     int rc = attrs_check(edge_src, edge_dst, n_edges, nd, workspace);
-    if (rc) return rc;
+    if (rc || (rc = attrs_check_dir(out_dir))) return rc;
     if (n_edges == 0 || (!want_len && !want_dir)) return AGX_OK;
     AGX_REQUIRE(!want_len || out_len, AGX_ERR_ARG, "agx_edge_attrs: out_len is NULL");
     AGX_REQUIRE(!want_dir || out_dir, AGX_ERR_ARG, "agx_edge_attrs: out_dir is NULL");

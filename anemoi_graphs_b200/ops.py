@@ -438,7 +438,10 @@ def edge_attributes(
     (its columns of ``edge_index`` are valid before the edge all-gather has finished) and every rank's block
     size; without it the edges are split evenly.  ``shard`` (``device.Shard``, sharded output mode): ``edge_index`` is
     this rank's own block and so are the results - only the statistics are exchanged.  ``regular_k`` > 0: the edges of the
-    i-th target are the columns [i k, (i + 1) k) (a KNN result) - evaluated by target instead of by edge."""
+    i-th target are the columns [i k, (i + 1) k) (a KNN result) - evaluated by target instead of by edge.
+
+    A NaN attribute value (an antipodal pair's length: ``a > 1`` in float32) makes every normalised value of that
+    attribute NaN, whatever the norm, as in the reference."""
     from . import device as _device
 
     for norm in (length_norm, direction_norm):

@@ -222,7 +222,10 @@ int agx_gate_open(uint32_t* gate /*HOST page-locked*/, void* stream);
  * agx_edge_attrs: replaces EdgeLength.compute / EdgeDirection.compute (edges/attributes.py:42-157):
  * raw values (float32 store) + global statistics in one pass over the edges, then - if a norm was asked for -
  * an in-place scaling pass.  len_norm / dir_norm = AGX_NORM_* or -1 to skip the attribute;
- * dir_rotated = luse_rotated_features.                                                          */
+ * dir_rotated = luse_rotated_features.  A NaN value (an antipodal pair's length) makes every normalised value of its
+ * attribute NaN, as numpy's sum / amax / amin / std do in the reference.
+ * out_dir, in this call and in _stats, _stats_flagged, _stats_list and _apply, must be 8-byte aligned (one float2
+ * store per edge; AGX_ERR_ARG otherwise, before any device work) - a view of an (E, 2) float32 array at any row is. */
 int agx_node_tables(const float* latlon /*DEV n*2*/, int64_t n, float* src_rec /*DEV n*8 or NULL*/,
                     double* dst_rec /*DEV n*4 or NULL, 32-byte aligned*/, void* stream);
 /* Node inputs of the attribute calls, per side EITHER a record table from agx_node_tables (src_rec / dst_rec; small node
@@ -234,7 +237,7 @@ int agx_edge_attrs(const int32_t* edge_src /*DEV E*/, const int32_t* edge_dst /*
                    const float* src_rec /*DEV or NULL*/, const float* src_latlon /*DEV ns*2 or NULL*/,
                    const double* dst_rec /*DEV or NULL*/, const float* dst_latlon /*DEV nt*2 or NULL*/,
                    int len_norm /*AGX_NORM_* or -1 = skip*/, int len_invert, float* out_len /*DEV E*/,
-                   int dir_norm /*AGX_NORM_* or -1 = skip*/, int dir_rotated, float* out_dir /*DEV E*2*/,
+                   int dir_norm /*AGX_NORM_* or -1 = skip*/, int dir_rotated, float* out_dir /*DEV E*2, 8-byte aligned*/,
                    double* workspace /*DEV, >= agx_edge_attrs_workspace() doubles*/,
                    int regular_k /*k > 0: the edges of the i-th target are columns [i k, (i+1) k) - a KNN result; 0: any list*/,
                    void* stream);

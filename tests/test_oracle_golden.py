@@ -113,6 +113,21 @@ def test_attr_vectors(golden):
     np.testing.assert_allclose(length[0], 0.053570323, rtol=1e-7)
 
 
+def test_reference_normalise_propagates_nan(golden):
+    """The reference's normalisation turns one NaN value (the antipodal pair of the golden vectors, row 9) into NaN
+    everywhere, for every norm - the behaviour the attribute kernel reproduces (tests/test_gpu_attr_paths.py)."""
+    g = golden("attr_vectors")
+    n = g["src"].shape[0]
+    ei = np.stack([np.arange(n), np.arange(n)])
+    values = np.array([[0.5, 1.0], [np.nan, 2.0], [3.0, 4.0]], dtype=np.float32)
+    with np.errstate(all="ignore"):
+        for norm in ("l1", "l2", "unit-max", "unit-range", "unit-std"):
+            assert np.isnan(R.edge_length(g["src"], g["dst"], ei, norm)).all(), norm
+            assert np.isnan(R.edge_length(g["src"], g["dst"], ei, norm, invert=True)).all(), norm
+            for v in (values, values.astype(np.float64)):
+                assert np.isnan(R.normalise(v, norm)).all(), norm
+        length = R.edge_length(g["src"], g["dst"], ei, None)
+    assert np.isnan(length[9]).all() and np.isfinite(np.delete(length, 9)).all()
 def test_o96_res5_matches_reference_and_published_counts(golden):
     g = golden("o96_res5")
     lat, lon = grids.octahedral_grid(96)
