@@ -63,6 +63,15 @@ SIGNATURES = {
     "agx_gate_open": (c_int, [c_void_p, c_void_p]),
     "agx_mark_nodes": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "agx_relabel_nodes": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
+    "agx_restrict_flags": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_double, c_void_p, c_void_p],
+    ),
+    "agx_sort_edges": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p]),
+    "agx_gather_edge_columns": (
+        c_int,
+        [c_int, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int64), c_void_p, c_int64, c_void_p],
+    ),
     "agx_set_output_maps": (None, [c_void_p, c_void_p]),
     "agx_concat_edges": (
         c_int,

@@ -50,6 +50,36 @@ void agx_note_order(int binned);  // what the last decision was  // raise the re
         }                                                                                   \
     } while (0)
 
+// The cut-off test of a radius (radians): a pair is inside iff rdist <= rdist_thr = sin^2(radius / 2) (sklearn
+// HaversineDistance64._dist_to_rdist, inclusive).  chord2_thr / margin are the FP32 pre-filter of the searches.  One
+// definition for CutOffEdges (agx_radius_*) and RestrictEdgeLength (agx_restrict_flags): the two agree bit for bit.
+static inline int agx_radius_params(double radius, float* chord2_thr, float* margin, double* rdist_thr) {
+    AGX_REQUIRE(radius >= 0.0, AGX_ERR_ARG, "radius must be non-negative (got %g)", radius);
+    double s = sin(0.5 * (radius < 3.141592653589793 ? radius : 3.141592653589793));
+    *rdist_thr = s * s;
+    double c2 = 4.0 * (*rdist_thr);
+    *chord2_thr = (float)c2;
+    // same bound as agx_chord2_margin plus the rounding of the threshold itself
+    *margin = (float)(4.2e-7 * sqrt(c2) + 1.2e-6 * c2 + 1.0e-13);
+    return AGX_OK;
+}
+
+// Packed 64-bit sort keys of edge columns, (hi << 32) | lo with non-negative int32 (hi, lo), so that unsigned key order
+// is lexicographic (hi, lo) column order (agx_concat.cu; shared by agx_concat_edges and agx_sort_edges).
+// agx_pack_keys writes the keys of list a followed by list b; with `bad` (DEV int, zeroed) it also sets *bad = 1 if
+// an entry is outside [0, n_hi_nodes) / [0, n_lo_nodes).  agx_key_passes: the radix passes over only the key bits the
+// node counts can set - one pass over [0, 32 + hi bits), or, when the lo field leaves >= 8 bits unused, the used lo
+// bits then the hi bits (LSD order: stable passes from the least significant field).
+int agx_pack_keys(const int32_t* a_hi, const int32_t* a_lo, int64_t na, const int32_t* b_hi, const int32_t* b_lo,
+                  int64_t nb, int64_t n_hi_nodes, int64_t n_lo_nodes, unsigned long long* keys, int* bad,
+                  cudaStream_t stream);
+struct AgxKeyPasses {
+    int count;
+    int begin[2], end[2];
+    int end_bit;  // the widest pass, [0, end_bit): what the CUB temporary storage is sized for
+};
+AgxKeyPasses agx_key_passes(int64_t n_hi_nodes, int64_t n_lo_nodes);
+
 static inline int agx_sm_count() {
     static int sms = 0;
     if (sms == 0) {

@@ -1,7 +1,7 @@
 // N1: utils.concat_edges on the device (/root/reference/src/anemoi/graphs/utils.py:66-81: `torch.unique(torch.cat([e1, e2],
 // dim=1), dim=1)` - the columns of both lists sorted lexicographically by (source, target), duplicates removed) - without
 // materialising the concatenated int64 list and torch.unique's temporaries:
-//   k_concat_pack      both (2, E) int32 lists -> ONE array of packed 64-bit keys (source << 32 | target); indices are
+//   k_pack_keys        both (2, E) int32 lists -> ONE array of packed 64-bit keys (source << 32 | target); indices are
 //                      non-negative, so unsigned key order = lexicographic column order
 //   cub::DeviceRadixSort::SortKeys on a double buffer, only the key bits the node counts can set (plain library sort)
 //   k_concat_heads     number of distinct keys per tile of 1024 (a key is a head if it differs from its predecessor)
@@ -15,16 +15,29 @@
 
 #define CONCAT_TILE 1024
 
-__global__ void __launch_bounds__(256) k_concat_pack(const int32_t* __restrict__ a_src, const int32_t* __restrict__ a_dst, int64_t na,
-                                                     const int32_t* __restrict__ b_src, const int32_t* __restrict__ b_dst, int64_t nb,
-                                                     unsigned long long* __restrict__ keys) {
+__global__ void __launch_bounds__(256) k_pack_keys(const int32_t* __restrict__ a_hi, const int32_t* __restrict__ a_lo, int64_t na,
+                                                   const int32_t* __restrict__ b_hi, const int32_t* __restrict__ b_lo, int64_t nb,
+                                                   int64_t n_hi_nodes, int64_t n_lo_nodes, unsigned long long* __restrict__ keys,
+                                                   int* __restrict__ bad) {
     const int64_t n = na + nb;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const bool first = i < na;
         const int64_t j = first ? i : i - na;
-        const unsigned s = (unsigned)(first ? a_src[j] : b_src[j]), d = (unsigned)(first ? a_dst[j] : b_dst[j]);
+        const unsigned s = (unsigned)(first ? a_hi[j] : b_hi[j]), d = (unsigned)(first ? a_lo[j] : b_lo[j]);
+        if (bad && ((int64_t)s >= n_hi_nodes || (int64_t)d >= n_lo_nodes)) *bad = 1;  // negative entries are >= 2^31 here
         keys[i] = ((unsigned long long)s << 32) | (unsigned long long)d;
     }
+}
+
+int agx_pack_keys(const int32_t* a_hi, const int32_t* a_lo, int64_t na, const int32_t* b_hi, const int32_t* b_lo,
+                  int64_t nb, int64_t n_hi_nodes, int64_t n_lo_nodes, unsigned long long* keys, int* bad,
+                  cudaStream_t stream) {
+    if (na + nb == 0) return AGX_OK;
+    k_pack_keys<<<agx_grid(na + nb, 256, 8), 256, 0, stream>>>(a_hi, a_lo, na, b_hi, b_lo, nb, n_hi_nodes, n_lo_nodes,
+                                                               keys, bad);
+    AGX_LAUNCH_OK();
+    agx_note_launch(1);
+    return AGX_OK;
 }
 
 __device__ __forceinline__ bool concat_is_head(const unsigned long long* __restrict__ keys, int64_t i) {
@@ -89,6 +102,21 @@ static int bits_for(int64_t max_value) {
     return b;
 }
 
+AgxKeyPasses agx_key_passes(int64_t n_hi_nodes, int64_t n_lo_nodes) {
+    AgxKeyPasses p;
+    p.end_bit = 32 + bits_for(n_hi_nodes - 1);
+    const int lo_bits = bits_for(n_lo_nodes - 1);
+    if ((32 - lo_bits) >= 8) {
+        p.count = 2;
+        p.begin[0] = 0, p.end[0] = lo_bits;
+        p.begin[1] = 32, p.end[1] = p.end_bit;
+    } else {
+        p.count = 1;
+        p.begin[0] = 0, p.end[0] = p.end_bit;
+    }
+    return p;
+}
+
 // `out` is the RESULT allocation, sized for the worst case (2 * (na + nb) int32 = as many bytes as one key buffer): it
 // doubles as the radix sort's alternate buffer, so the only scratch besides it is ONE key buffer (8 bytes per input
 // edge) + CUB's histograms.  On return the first 2 * n_unique int32 of `out` are the result, row-major (2, n_unique).
@@ -121,21 +149,18 @@ extern "C" int agx_concat_edges(const int32_t* a_src, const int32_t* a_dst, int6
         return AGX_ERR_CUDA;                                                                               \
     }
     CC_TRY(cudaMallocAsync(&keys, n * sizeof(unsigned long long), stream));
-    k_concat_pack<<<agx_grid(n, 256, 8), 256, 0, stream>>>(a_src, a_dst, na, b_src, b_dst, nb, keys);
-    agx_note_launch(1);
-    cub::DoubleBuffer<unsigned long long> buf(keys, alt);
-    const int end_bit = 32 + bits_for(n_src_nodes - 1);
-    const int dst_bits = bits_for(n_dst_nodes - 1);
-    size_t temp_bytes = 0;
-    CC_TRY(cub::DeviceRadixSort::SortKeys(nullptr, temp_bytes, buf, (long long)n, 0, end_bit, stream));
-    CC_TRY(cudaMallocAsync(&temp, temp_bytes > 0 ? temp_bytes : 16, stream));
-    if ((32 - dst_bits) >= 8) {
-        // LSD radix sort = stable passes from the least significant field: the used target bits, then the source bits
-        CC_TRY(cub::DeviceRadixSort::SortKeys(temp, temp_bytes, buf, (long long)n, 0, dst_bits, stream));
-        CC_TRY(cub::DeviceRadixSort::SortKeys(temp, temp_bytes, buf, (long long)n, 32, end_bit, stream));
-    } else {
-        CC_TRY(cub::DeviceRadixSort::SortKeys(temp, temp_bytes, buf, (long long)n, 0, end_bit, stream));
+    int rc = agx_pack_keys(a_src, a_dst, na, b_src, b_dst, nb, n_src_nodes, n_dst_nodes, keys, nullptr, stream);
+    if (rc) {
+        cudaFreeAsync(keys, stream);
+        return rc;
     }
+    cub::DoubleBuffer<unsigned long long> buf(keys, alt);
+    const AgxKeyPasses passes = agx_key_passes(n_src_nodes, n_dst_nodes);
+    size_t temp_bytes = 0;
+    CC_TRY(cub::DeviceRadixSort::SortKeys(nullptr, temp_bytes, buf, (long long)n, 0, passes.end_bit, stream));
+    CC_TRY(cudaMallocAsync(&temp, temp_bytes > 0 ? temp_bytes : 16, stream));
+    for (int p = 0; p < passes.count; ++p)
+        CC_TRY(cub::DeviceRadixSort::SortKeys(temp, temp_bytes, buf, (long long)n, passes.begin[p], passes.end[p], stream));
     agx_note_launch(2);
     if (buf.Current() != keys)  // the sorted keys must not live in the buffer the result is unpacked into
         CC_TRY(cudaMemcpyAsync(keys, alt, n * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, stream));
@@ -143,7 +168,7 @@ extern "C" int agx_concat_edges(const int32_t* a_src, const int32_t* a_dst, int6
     CC_TRY(cudaMallocAsync(&offsets, (n_tiles + 1) * sizeof(int64_t), stream));
     k_concat_heads<<<(unsigned)n_tiles, 256, 0, stream>>>(keys, n, counts);
     agx_note_launch(1);
-    int rc = agx_exclusive_scan(counts, n_tiles, offsets, n_unique, stream);  // reads the total back (one sync)
+    rc = agx_exclusive_scan(counts, n_tiles, offsets, n_unique, stream);  // reads the total back (one sync)
     if (rc == AGX_OK) {
         k_concat_fill<<<(unsigned)n_tiles, 256, 0, stream>>>(keys, n, offsets, out, out + *n_unique);
         agx_note_launch(1);

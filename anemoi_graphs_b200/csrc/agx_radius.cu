@@ -264,18 +264,6 @@ static int launch_radius_tile(const agx_index_t* ix, const float* q_latlon, int6
     return AGX_OK;
 }
 
-static int radius_params(double radius, float* chord2_thr, float* margin, double* rdist_thr) {
-    AGX_REQUIRE(radius >= 0.0, AGX_ERR_ARG, "radius must be non-negative (got %g)", radius);
-    // sklearn: reduced radius = sin(0.5 r)^2 (HaversineDistance64._dist_to_rdist)
-    double s = sin(0.5 * (radius < 3.141592653589793 ? radius : 3.141592653589793));
-    *rdist_thr = s * s;
-    double c2 = 4.0 * (*rdist_thr);
-    *chord2_thr = (float)c2;
-    // same bound as agx_chord2_margin plus the rounding of the threshold itself
-    *margin = (float)(4.2e-7 * sqrt(c2) + 1.2e-6 * c2 + 1.0e-13);
-    return AGX_OK;
-}
-
 extern "C" int agx_radius_count(const agx_index_t* ix, const float* q_latlon, int64_t nq, double radius,
                                 int32_t* counts, void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
@@ -283,7 +271,7 @@ extern "C" int agx_radius_count(const agx_index_t* ix, const float* q_latlon, in
     AGX_REQUIRE(nq >= 0, AGX_ERR_ARG, "agx_radius_count: nq < 0");
     float c2, m;
     double thr;
-    int rc = radius_params(radius, &c2, &m, &thr);
+    int rc = agx_radius_params(radius, &c2, &m, &thr);
     if (rc) return rc;
     if (nq == 0) return AGX_OK;
     AGX_REQUIRE(q_latlon && counts, AGX_ERR_ARG, "agx_radius_count: NULL buffer");
@@ -306,7 +294,7 @@ extern "C" int agx_radius_fill(const agx_index_t* ix, const float* q_latlon, int
     AGX_REQUIRE(dst_base + nq < (int64_t)2147483647, AGX_ERR_ARG, "agx_radius_fill: target index exceeds int32");
     float c2, m;
     double thr;
-    int rc = radius_params(radius, &c2, &m, &thr);
+    int rc = agx_radius_params(radius, &c2, &m, &thr);
     if (rc) return rc;
     if (nq == 0) return AGX_OK;
     AGX_REQUIRE(q_latlon && offsets && out_src && out_dst, AGX_ERR_ARG, "agx_radius_fill: NULL buffer");

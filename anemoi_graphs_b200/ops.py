@@ -573,6 +573,68 @@ def compact_flags(flags: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:
     return out, count
 
 
+def restrict_flags(
+    edge_index: torch.Tensor, src_x: torch.Tensor, dst_x: torch.Tensor, max_radius: float,
+    src_mask: torch.Tensor | None = None, dst_mask: torch.Tensor | None = None,
+) -> torch.Tensor:  # fmt: skip
+    """CUDA uint8 (E,): 0 for the edges of the CUDA int32 (2, E) ``edge_index`` that are subject to the restriction
+    (``src_mask[source]`` and ``dst_mask[target]``, CUDA uint8 per node, each optional) and longer than ``max_radius``
+    (radians) by CutOffEdges' test, 1 for the others (``agx_restrict_flags``).  ValueError for an endpoint outside
+    its node set."""
+    assert edge_index.is_cuda and edge_index.dtype == torch.int32 and edge_index.dim() == 2 and edge_index.shape[0] == 2
+    edge_index = edge_index.contiguous()
+    src_x, dst_x = _dev_x(src_x), _dev_x(dst_x)
+    for mask, x in ((src_mask, src_x), (dst_mask, dst_x)):
+        assert mask is None or (mask.is_cuda and mask.dtype == torch.uint8 and mask.shape == (x.shape[0],))
+    n = int(edge_index.shape[1])
+    keep = torch.empty(n, dtype=torch.uint8, device=edge_index.device)
+    with _span("restrict_flags", n):
+        check(
+            load_library().agx_restrict_flags(
+                ptr(edge_index[0]), ptr(edge_index[1]), n, ptr(src_x), int(src_x.shape[0]), ptr(dst_x),
+                int(dst_x.shape[0]), ptr(src_mask), ptr(dst_mask), float(max_radius), ptr(keep), current_stream(),
+            )
+        )  # fmt: skip
+    return keep
+
+
+def sort_permutation(key_row: torch.Tensor, other_row: torch.Tensor, n_key_nodes: int, n_other_nodes: int,
+                     descending: bool) -> torch.Tensor:  # fmt: skip
+    """CUDA int32 (E,): the stable permutation that orders the columns (key_row, other_row) lexicographically
+    (``agx_sort_edges``).  ValueError for an endpoint outside its node set."""
+    for row in (key_row, other_row):
+        assert row.is_cuda and row.dtype == torch.int32 and row.is_contiguous() and row.shape == key_row.shape
+    n = int(key_row.numel())
+    perm = torch.empty(n, dtype=torch.int32, device=key_row.device)
+    with _span("sort_edges", n):
+        check(
+            load_library().agx_sort_edges(
+                ptr(key_row), ptr(other_row), n, int(n_key_nodes), int(n_other_nodes), int(bool(descending)), ptr(perm),
+                current_stream(),
+            )
+        )  # fmt: skip
+    return perm
+
+
+def gather_rows(pairs: list[tuple[torch.Tensor, torch.Tensor]], index: torch.Tensor) -> None:
+    """``dst[j] = src[index[j]]`` along dim 0 for every (src, dst) pair of contiguous CUDA tensors of one dtype and row
+    shape, eight pairs per launch (``agx_gather_edge_columns``)."""
+    assert index.is_cuda and index.dtype == torch.int32 and index.is_contiguous()
+    m = int(index.numel())
+    pairs = [(s, d) for s, d in pairs if d.numel()]
+    lib = load_library()
+    for a in range(0, len(pairs), 8):
+        part = pairs[a : a + 8]
+        for s, d in part:
+            assert s.is_cuda and d.is_cuda and s.is_contiguous() and d.is_contiguous() and s.dtype == d.dtype
+            assert d.shape[0] == m and s.shape[1:] == d.shape[1:]
+        srcs = (c_void_p * len(part))(*[s.data_ptr() for s, _ in part])
+        dsts = (c_void_p * len(part))(*[d.data_ptr() for _, d in part])
+        row_bytes = (c_int64 * len(part))(*[d.numel() // m * d.element_size() for _, d in part])
+        with _span("gather_edges", m * len(part)):
+            check(lib.agx_gather_edge_columns(len(part), srcs, dsts, row_bytes, ptr(index), m, current_stream()))
+
+
 class DeferredEdgeAttributes:
     """EdgeLength / EdgeDirection of an edge set whose sources of a FEW targets are still to be re-decided (KNN edges
     searched while the source numbering was provisional; ``dst_flags`` marks those targets).

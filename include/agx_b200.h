@@ -168,6 +168,37 @@ int agx_relabel_nodes(int32_t* row /*DEV n, in place*/, int64_t n, const int64_t
 int agx_relabel_rows(int32_t* const* rows /*HOST n_rows x DEV*/, const int64_t* lens /*HOST n_rows*/, int n_rows,
                      const int64_t* new_index /*DEV*/, void* stream);
 
+/* ---- edge post-processors -----------------------------------------------------------------------------
+ * RestrictEdgeLength / SortEdgeIndexBySourceNodes / SortEdgeIndexByTargetNodes (processors/post_process.py of newer
+ * releases; replaces pulling edge_index and every attribute to the host, masking / argsorting them there and writing
+ * them back).  Each ends in ONE int32 index list applied to every per-edge array of an edge set.
+ * agx_restrict_flags: keep[i] = 0 iff edge i is subject to the restriction (src_mask[src] and dst_mask[dst], each mask
+ * optional: uint8 per node, non-zero = subject) and its rdist (agx_rdist64 of target, source) > sin^2(max_radius / 2) - the
+ * test CutOffEdges applies (agx_radius_*), so the two agree bit for bit; 1 otherwise.  max_radius in radians, >= 0.
+ * AGX_ERR_ARG (after the pass, one read-back) if an endpoint is outside [0, n_src_nodes) / [0, n_dst_nodes); keep is
+ * then undefined.  The list of kept positions is agx_compact_flags(keep) (keep from cudaMalloc: 4-byte aligned).     */
+int agx_restrict_flags(const int32_t* edge_src /*DEV E*/, const int32_t* edge_dst /*DEV E*/, int64_t n_edges,
+                       const float* src_latlon /*DEV ns*2*/, int64_t n_src_nodes, const float* dst_latlon /*DEV nt*2*/,
+                       int64_t n_dst_nodes, const uint8_t* src_mask /*DEV ns or NULL*/,
+                       const uint8_t* dst_mask /*DEV nt or NULL*/, double max_radius, uint8_t* keep /*DEV E*/,
+                       void* stream);
+/* agx_sort_edges: perm = the stable permutation that orders the columns lexicographically by (key_row, other_row),
+ * ascending or (descending != 0) descending; columns equal in both rows keep their input order.  The rows are packed
+ * into 64-bit keys as in agx_concat_edges (same kernel, same trimming to the bits the node counts can set) and
+ * sorted with CUB's radix SortPairs / SortPairsDescending, positions as values.  Scratch: 20 bytes per edge + CUB's.
+ * AGX_ERR_ARG if E >= 2^31 or an endpoint is outside [0, n_key_nodes) / [0, n_other_nodes) (checked by the packing
+ * pass, one read-back at the end; perm is then undefined).                                                         */
+int agx_sort_edges(const int32_t* key_row /*DEV E*/, const int32_t* other_row /*DEV E*/, int64_t n_edges,
+                   int64_t n_key_nodes, int64_t n_other_nodes, int descending, int32_t* perm /*DEV E*/, void* stream);
+/* agx_gather_edge_columns: for each of n_arrays <= 8 arrays (src / dst / row_bytes: HOST arrays of DEV pointers and
+ * sizes) row j of dst = row index[j] of src, j < n_index, in ONE launch; a caller with more arrays calls again.  An
+ * array is any row-major (rows, row_bytes) buffer - the two rows of an edge_index count as two arrays of E rows.  Rows
+ * of any byte size up to 2^20 are moved as the widest word (16, 8, 4, 2 or 1 bytes) that divides the row size and both
+ * pointers' alignment.  index entries must lie inside every src; dst must not overlap src.  No read-back.            */
+int agx_gather_edge_columns(int n_arrays, const void* const* src /*HOST n_arrays x DEV*/,
+                            void* const* dst /*HOST n_arrays x DEV*/, const int64_t* row_bytes /*HOST n_arrays*/,
+                            const int32_t* index /*DEV n_index*/, int64_t n_index, void* stream);
+
 /* ---- masked node sets -------------------------------------------------------------------------------------
  * NodeMaskingMixin.undo_masking (edges/builder.py:176-193: compact indices of the row-selected coordinates mapped back
  * to node indices through a python dict + np.vectorize) fused into the searches' writes: while maps are set (thread-
