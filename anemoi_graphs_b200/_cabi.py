@@ -105,6 +105,15 @@ SIGNATURES = {
         [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_int,
          c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p],
     ),  # fmt: skip
+    "agx_edge_azimuth": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p],
+    ),
+    "agx_gaussian_weights": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_double, c_int, c_void_p, c_void_p, c_void_p, c_void_p],
+    ),
+    "agx_gaussian_weights_scratch_bytes": (c_int64, [c_int64, c_int64]),
     "agx_icosphere": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "agx_multiscale_tri_count": (
         c_int,

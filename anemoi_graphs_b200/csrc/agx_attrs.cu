@@ -926,3 +926,82 @@ extern "C" int agx_edge_attrs(const int32_t* edge_src, const int32_t* edge_dst, 
                      workspace, stream, nullptr, 0, nullptr, nullptr, 0, workspace, want_len && len_norm > 0,
                      want_len && len_invert, want_dir && dir_norm > 0);
 }
+
+// ------------------------------------------------------------------------------------------------
+// Azimuth: the initial bearing at the target towards the source, clockwise from north, in [-pi, pi]
+// ------------------------------------------------------------------------------------------------
+// atan2(sin(dlon) cos(lat_s), cos(lat_t) sin(lat_s) - sin(lat_t) cos(lat_s) cos(dlon)), dlon = lon_s - lon_t, in float64
+// from the float32 coordinates, each operation rounded as numpy rounds it (no contraction), stored as float32.  The
+// statistics are those of EdgeLength (the float64 of the stored value) in the length slot of the K5 workspace, so the
+// global norm is k_attr_fold -> k_attr_params -> k_attr_scale with its NaN rule.  An endpoint outside its node set is
+// never read: it raises *bad (an int in workspace word 14, between the statistics and the block partials).
+__global__ void __launch_bounds__(ATTR_THREADS) k_edge_azimuth(const int32_t* __restrict__ esrc, const int32_t* __restrict__ edst,
+                                                               int64_t n, const float2* __restrict__ s_ll, int64_t n_src,
+                                                               const float2* __restrict__ t_ll, int64_t n_dst,
+                                                               float* __restrict__ out, double* __restrict__ ws, int stats) {
+    Stat4 st;
+    st.init();
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const int32_t s = __ldg(esrc + i), t = __ldg(edst + i);
+        if (s < 0 || s >= n_src || t < 0 || t >= n_dst) {
+            *reinterpret_cast<int*>(ws + 14) = 1;
+            continue;
+        }
+        const float2 ps = __ldg(s_ll + s), pt = __ldg(t_ll + t);
+        double sls, cls, slt, clt, sdl, cdl;
+        sincos((double)ps.x, &sls, &cls);
+        sincos((double)pt.x, &slt, &clt);
+        sincos(__dsub_rn((double)ps.y, (double)pt.y), &sdl, &cdl);
+        const double y = __dmul_rn(sdl, cls);
+        const double x = __dsub_rn(__dmul_rn(clt, sls), __dmul_rn(__dmul_rn(slt, cls), cdl));
+        const float v = (float)atan2(y, x);
+        out[i] = v;
+        if (stats) st.add((double)v, v);
+    }
+    if (stats) {
+        __shared__ Stat4 sm[ATTR_THREADS / 32];
+        st = warp_reduce(st);
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+        if (lane == 0) sm[warp] = st;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int w = 1; w < ATTR_THREADS / 32; ++w) st.merge(sm[w]);
+            double* p = ws + (int64_t)ATTR_STAT_FIELDS * (2 + blockIdx.x);
+            st.store(p);
+            Stat4 none;
+            none.init();
+            none.store(p + 4);  // the direction slot of the fold stays empty
+        }
+    }
+}
+
+extern "C" int agx_edge_azimuth(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, const float* src_latlon,
+                                int64_t n_src_nodes, const float* dst_latlon, int64_t n_dst_nodes, int norm, float* out,
+                                double* workspace, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    AGX_REQUIRE(n_edges >= 0 && n_src_nodes >= 0 && n_dst_nodes >= 0, AGX_ERR_ARG, "agx_edge_azimuth: negative size");
+    AGX_REQUIRE(norm >= 0 && norm <= AGX_NORM_UNIT_STD, AGX_ERR_ARG, "agx_edge_azimuth: unknown norm code");
+    if (n_edges == 0) return AGX_OK;
+    AGX_REQUIRE(edge_src && edge_dst && out && workspace, AGX_ERR_ARG, "agx_edge_azimuth: NULL buffer");
+    AGX_REQUIRE((n_src_nodes == 0 || src_latlon) && (n_dst_nodes == 0 || dst_latlon), AGX_ERR_ARG,
+                "agx_edge_azimuth: NULL coordinates");
+    AGX_REQUIRE((((uintptr_t)src_latlon | (uintptr_t)dst_latlon) & 7) == 0, AGX_ERR_ARG,
+                "agx_edge_azimuth: coordinates must be 8-byte aligned");
+    AGX_CUDA_OK(cudaMemsetAsync(workspace + 14, 0, sizeof(double), stream));
+    const int grid = attrs_grid(n_edges, 1);
+    k_edge_azimuth<<<grid, ATTR_THREADS, 0, stream>>>(edge_src, edge_dst, n_edges, (const float2*)src_latlon, n_src_nodes,
+                                                      (const float2*)dst_latlon, n_dst_nodes, out, workspace, norm > 0);
+    agx_note_launch(1);
+    if (norm > 0) {
+        k_attr_fold<<<1, 256, 0, stream>>>(workspace, grid, workspace + 6);
+        k_attr_params<<<1, 32, 0, stream>>>(workspace, workspace + 6, 1, n_edges, norm, 0);
+        k_attr_scale<<<agx_grid((n_edges + 3) / 4, 256, 8), 256, 0, stream>>>(out, n_edges, 1, 0, nullptr, 0, 0, 0, workspace);
+        agx_note_launch(3);
+    }
+    AGX_LAUNCH_OK();
+    long long bad = 0;
+    int rc = agx_readback(&bad, workspace + 14, 1, stream);
+    if (rc) return rc;
+    AGX_REQUIRE((int)bad == 0, AGX_ERR_ARG, "agx_edge_azimuth: an edge endpoint is outside [0, num_nodes) of its node set");
+    return AGX_OK;
+}

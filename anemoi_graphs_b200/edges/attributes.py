@@ -5,10 +5,17 @@ edges_name)`` contract (float32 ``(E, 1)`` / ``(E, 2)`` tensors, normalised over
 Raw values, the global reduction for the normalisation and the final float32 cast are one fused CUDA
 kernel pair (``ops.edge_attributes``); when both attributes are requested for an edge set
 (``compute_attributes``) they share a single pass over ``edge_index``.
+
+``Azimuth``, ``GaussianDistanceWeights``, ``AttributeFromSourceNode`` and ``AttributeFromTargetNode`` carry the names
+of edge attributes of newer anemoi-graphs releases, which the pinned reference does not have: their semantics follow
+the upstream classes as far as is known, unverified against their source (DESIGN.md).  They need the final node
+numbering (a canonical order by target, or rows of a node attribute) and are evaluated after ``EdgeLength`` /
+``EdgeDirection`` of the same edge set.
 """
 
 from __future__ import annotations
 
+import math
 from abc import ABC
 
 import torch
@@ -16,6 +23,7 @@ import torch
 from .. import device as _device
 from .. import ops
 from .._cabi import NORM_CODES
+from ..processors.post_process import _refuse_sharded
 
 
 def _check_norm(norm) -> None:
@@ -110,7 +118,20 @@ def compute_attributes(graph, edges_name: tuple[str, str, str], attrs: dict) -> 
 
     Pairs one ``EdgeLength`` with one ``EdgeDirection`` per kernel pass; foreign attribute objects (anything
     with a ``compute(graph, edges_name)`` method) are called as the reference would call them
-    (edges/builder.py:133)."""
+    (edges/builder.py:133).  The edge-list attributes (``EdgeListAttribute``) follow, in final numbering."""
+    listed = {k: a for k, a in attrs.items() if isinstance(a, EdgeListAttribute)}
+    if not listed:
+        return _fused_attributes(graph, edges_name, attrs)
+    if _device.sharded_output() or "edge_shard" in graph[tuple(edges_name)]:
+        _refuse_sharded(tuple(edges_name))
+    _check_nodes(graph, edges_name)
+    out = _fused_attributes(graph, edges_name, {k: a for k, a in attrs.items() if k not in listed})
+    out.update(_edge_list_attributes(graph, edges_name, listed))
+    return {k: out[k] for k in attrs}  # the recipe's order
+
+
+def _fused_attributes(graph, edges_name: tuple[str, str, str], attrs: dict) -> dict:
+    """``EdgeLength`` / ``EdgeDirection`` (K5) and foreign attribute objects."""
     ours = {k: a for k, a in attrs.items() if isinstance(a, (EdgeLength, EdgeDirection))}
     out: dict = {}
     for k, a in attrs.items():
@@ -218,3 +239,151 @@ def _deferred_attributes(prov, meta, edge_index, src, dst, lengths, dirs, host_s
 
     prov.add_finalizer(finalize)
     return results
+
+
+# ------------------------------------------------------------------------------------------------
+# attributes of newer anemoi-graphs releases: evaluated on the complete edge list in final numbering
+# ------------------------------------------------------------------------------------------------
+class EdgeListAttribute(BaseEdgeAttribute):
+    """An edge attribute that reads the complete device edge list of its edge set in final node numbering."""
+
+    def evaluate(self, graph, edges_name, edge_index: torch.Tensor) -> torch.Tensor:
+        """The CUDA result for the CUDA int32 (2, E) ``edge_index`` (final numbering, not yet checked)."""
+        raise NotImplementedError
+
+
+def _check_endpoints(edge_index: torch.Tensor, n_src: int, n_dst: int) -> None:
+    """ValueError unless every source is in [0, n_src) and every target in [0, n_dst) - one read-back."""
+    if edge_index.shape[1] == 0:
+        return
+    lo, hi = torch.aminmax(edge_index, dim=1)
+    (s_lo, d_lo), (s_hi, d_hi) = torch.stack([lo, hi]).tolist()
+    if s_lo < 0 or d_lo < 0 or s_hi >= n_src or d_hi >= n_dst:
+        raise ValueError("an edge endpoint is outside [0, num_nodes) of its node set")
+
+
+def _edge_list_attributes(graph, edges_name, attrs: dict) -> dict:
+    source_name, _, target_name = edges_name
+    store = graph[tuple(edges_name)]
+    reference_input = store["edge_index"]
+    edge_index = _device.device_edge_index(store)  # before the order resolves: it relabels this very tensor
+    meta = _device.edge_meta(edge_index)
+    for prov in (meta.fixup if meta is not None else None, *_device.row_tags(edge_index),
+                 _device.active_provisional(graph[source_name]), _device.active_provisional(graph[target_name])):  # fmt: skip
+        if prov is not None:
+            prov.resolve()
+    _device.wait_for(edge_index)
+    return {k: _device.like_input(a.evaluate(graph, edges_name, edge_index), reference_input) for k, a in attrs.items()}
+
+
+class Azimuth(EdgeListAttribute):
+    """Initial bearing at the target node towards the source node, in radians, clockwise from north, in [-pi, pi]:
+    ``atan2(sin(dlon) cos(lat_s), cos(lat_t) sin(lat_s) - sin(lat_t) cos(lat_s) cos(dlon))``, dlon = lon_s - lon_t,
+    in float64 from the float32 coordinates, stored as float32 (E, 1).  As the upstream ``Azimuth.compute(x_i, x_j)``
+    with i = target, j = source, as far as is known.
+
+    Attributes
+    ----------
+    norm : Optional[str]
+        Normalisation over the whole edge set, as for ``EdgeLength``. Options: None, "l1", "l2", "unit-max",
+        "unit-range", "unit-std".
+    """
+
+    def __init__(self, norm: str | None = None) -> None:
+        _check_norm(norm)
+        super().__init__(norm)
+
+    def evaluate(self, graph, edges_name, edge_index):
+        source_name, _, target_name = edges_name
+        src_x = _device.node_state(graph[source_name]).x
+        dst_x = _device.node_state(graph[target_name]).x
+        return ops.edge_azimuth(edge_index, src_x, dst_x, self.norm)
+
+
+class GaussianDistanceWeights(EdgeListAttribute):
+    """Gaussian weights of the edge lengths, normalised per target node: w = exp(-d^2 / (2 sigma^2)), d the float32
+    ``EdgeLength(norm=None)`` value on the unit sphere, in float64; ``norm`` is applied to the edges of each target
+    node as normalise.py applies it to a whole array (a NaN weight makes its group NaN; under "unit-std" a group of
+    bit-equal weights is left unnormalised), rounded to float32 (E, 1) once.  The result does not depend on the order
+    of the columns of ``edge_index``.  As the upstream class, as far as is known.
+
+    Attributes
+    ----------
+    sigma : float
+        Width of the Gaussian, in radians. Default 1.0.
+    norm : Optional[str]
+        Normalisation per target node. Options: None, "l1", "l2", "unit-max", "unit-range", "unit-std". Default "l1".
+    """
+
+    def __init__(self, sigma: float = 1.0, norm: str | None = "l1") -> None:
+        assert isinstance(sigma, (int, float)) and not isinstance(sigma, bool), "sigma must be a number"
+        assert sigma > 0, "sigma must be positive"
+        _check_norm(norm)
+        super().__init__(norm)
+        self.sigma = sigma
+
+    def evaluate(self, graph, edges_name, edge_index):
+        source_name, _, target_name = edges_name
+        n_src, n_dst = int(graph[source_name].num_nodes), int(graph[target_name].num_nodes)
+        perm = None
+        if self.norm is None:
+            _check_endpoints(edge_index, n_src, n_dst)
+        else:  # the canonical order; checks the endpoints
+            perm = ops.sort_permutation(edge_index[1], edge_index[0], n_dst, n_src, descending=False)
+        meta = _device.edge_meta(edge_index)
+        src = _device.node_tables(graph[source_name])
+        dst = _device.node_tables(graph[target_name])
+        lengths, _ = ops.edge_attributes(edge_index, src, dst, length=True, length_norm=None, direction=False,
+                                         regular_k=meta.regular_k if meta is not None else 0)  # fmt: skip
+        return ops.gaussian_weights(edge_index, n_src, n_dst, lengths, self.sigma, self.norm, perm)
+
+
+class _AttributeFromNode(EdgeListAttribute):
+    row: int
+
+    def __init__(self, node_attr_name: str) -> None:
+        assert isinstance(node_attr_name, str), "node_attr_name must be a str"
+        super().__init__(None)
+        self.node_attr_name = node_attr_name
+
+    def evaluate(self, graph, edges_name, edge_index):
+        nodes_name = edges_name[0] if self.row == 0 else edges_name[2]
+        nodes = graph[nodes_name]
+        n = int(nodes.num_nodes)
+        value = nodes.get(self.node_attr_name, None) if hasattr(nodes, "get") else None
+        if not isinstance(value, torch.Tensor) or value.dim() == 0 or value.shape[0] != n:
+            what = f"shape {tuple(value.shape)}" if isinstance(value, torch.Tensor) else "missing"
+            raise ValueError(f"The node attribute '{self.node_attr_name}' of {nodes_name} must be a tensor with {n} rows ({what}).")
+        _check_endpoints(edge_index, int(graph[edges_name[0]].num_nodes), int(graph[edges_name[2]].num_nodes))
+        rows = _device.to_device(value.reshape(n, math.prod(value.shape[1:]))).bool().view(torch.uint8).contiguous()
+        out = torch.empty((int(edge_index.shape[1]), int(rows.shape[1])), dtype=torch.bool, device=edge_index.device)
+        ops.gather_rows([(rows, out.view(torch.uint8))], edge_index[self.row])
+        return out
+
+
+class AttributeFromSourceNode(_AttributeFromNode):
+    """The source node's row of a node attribute, as a bool edge attribute: ``graph[source][node_attr_name]`` at
+    ``edge_index[0]``, (E, 1) for an (N,) attribute and (E, M) for an (N, M) one, cast as ``Tensor.bool()`` casts.
+    As the upstream class (a mask such as CutOutMask carried onto the edges), as far as is known.
+
+    Attributes
+    ----------
+    node_attr_name : str
+        Name of the source node attribute.
+    """
+
+    row = 0
+
+
+class AttributeFromTargetNode(_AttributeFromNode):
+    """The target node's row of a node attribute, as a bool edge attribute: ``graph[target][node_attr_name]`` at
+    ``edge_index[1]``, (E, 1) for an (N,) attribute and (E, M) for an (N, M) one, cast as ``Tensor.bool()`` casts.
+    As the upstream class, as far as is known.
+
+    Attributes
+    ----------
+    node_attr_name : str
+        Name of the target node attribute.
+    """
+
+    row = 1

@@ -635,6 +635,51 @@ def gather_rows(pairs: list[tuple[torch.Tensor, torch.Tensor]], index: torch.Ten
             check(lib.agx_gather_edge_columns(len(part), srcs, dsts, row_bytes, ptr(index), m, current_stream()))
 
 
+def edge_azimuth(edge_index: torch.Tensor, src_x: torch.Tensor, dst_x: torch.Tensor, norm: str | None) -> torch.Tensor:
+    """CUDA float32 (E, 1): the bearing at each edge's target towards its source, clockwise from north, in radians,
+    normalised over the whole edge set as ``EdgeLength`` is (``agx_edge_azimuth``).  ValueError for an endpoint outside
+    its node set."""
+    assert edge_index.is_cuda and edge_index.dtype == torch.int32 and edge_index.dim() == 2 and edge_index.shape[0] == 2
+    edge_index = edge_index.contiguous()
+    src_x, dst_x = _dev_x(src_x), _dev_x(dst_x)
+    n = int(edge_index.shape[1])
+    out = torch.empty((n, 1), dtype=torch.float32, device=edge_index.device)
+    with _span("edge_azimuth", n):
+        check(
+            load_library().agx_edge_azimuth(
+                ptr(edge_index[0]), ptr(edge_index[1]), n, ptr(src_x), int(src_x.shape[0]), ptr(dst_x),
+                int(dst_x.shape[0]), NORM_CODES[norm], ptr(out), ptr(_attr_workspace(edge_index.device)), current_stream(),
+            )
+        )  # fmt: skip
+    return out
+
+
+def gaussian_weights(edge_index: torch.Tensor, n_src_nodes: int, n_dst_nodes: int, lengths: torch.Tensor, sigma: float,
+                     norm: str | None, perm: torch.Tensor | None) -> torch.Tensor:  # fmt: skip
+    """CUDA float32 (E, 1): exp(-d^2 / (2 sigma^2)) of the float32 lengths d (E, 1), normalised within each target's
+    edges (``agx_gaussian_weights``).  ``perm``: ``sort_permutation(edge_index[1], edge_index[0], ..., False)`` (which
+    checks the endpoints); None with ``norm=None``."""
+    assert edge_index.is_cuda and edge_index.dtype == torch.int32 and edge_index.dim() == 2 and edge_index.shape[0] == 2
+    edge_index = edge_index.contiguous()
+    n = int(edge_index.shape[1])
+    assert lengths.is_cuda and lengths.dtype == torch.float32 and lengths.is_contiguous() and lengths.numel() == n
+    assert (perm is None) == (norm is None) and (perm is None or (perm.is_cuda and perm.dtype == torch.int32 and perm.numel() == n))
+    lib = load_library()
+    out = torch.empty((n, 1), dtype=torch.float32, device=edge_index.device)
+    scratch = None
+    if norm is not None and n:
+        size = int(lib.agx_gaussian_weights_scratch_bytes(n, int(n_dst_nodes)))
+        scratch = torch.empty(size, dtype=torch.uint8, device=edge_index.device)
+    with _span("gaussian_weights", n):
+        check(
+            lib.agx_gaussian_weights(
+                ptr(edge_index[0]), ptr(edge_index[1]), n, int(n_src_nodes), int(n_dst_nodes), ptr(lengths),
+                float(sigma), NORM_CODES[norm], ptr(perm), ptr(out), ptr(scratch), current_stream(),
+            )
+        )  # fmt: skip
+    return out
+
+
 class DeferredEdgeAttributes:
     """EdgeLength / EdgeDirection of an edge set whose sources of a FEW targets are still to be re-decided (KNN edges
     searched while the source numbering was provisional; ``dst_flags`` marks those targets).

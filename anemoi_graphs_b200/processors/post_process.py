@@ -161,11 +161,15 @@ class RemoveUnconnectedNodes(BaseMaskingProcessor):
 # ------------------------------------------------------------------------------------------------
 def _check_gathered(name, store) -> None:
     if "edge_shard" in store:
-        raise NotImplementedError(
-            f"edge set {name} is a sharded block of a device-resident graph: the edge post-processors work on complete "
-            "edge lists - build this recipe in the default output mode (AGX_OUTPUT=gather / "
-            "device.set_sharded_output(False))"
-        )
+        _refuse_sharded(name)
+
+
+def _refuse_sharded(name) -> None:
+    raise NotImplementedError(
+        f"edge set {name} is a sharded block of a device-resident graph: the edge post-processors work on complete "
+        "edge lists - build this recipe in the default output mode (AGX_OUTPUT=gather / "
+        "device.set_sharded_output(False))"
+    )
 
 
 def _select_edges(store, index: torch.Tensor, ei_dev: torch.Tensor) -> None:

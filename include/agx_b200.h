@@ -309,6 +309,32 @@ int agx_edge_attrs_apply(const int32_t* edge_src, const int32_t* edge_dst, int64
                          int len_invert, float* out_len, int dir_norm, int dir_rotated, float* out_dir,
                          const double* stats /*DEV n_stat_sets*8 or NULL if no norm*/, int n_stat_sets,
                          int64_t n_edges_global, int raw_present, double* workspace, void* stream);
+/* agx_edge_azimuth (Azimuth): out[e] = float32 of the initial bearing at the target towards the source, in radians,
+ * clockwise from north, in [-pi, pi]: atan2(sin(dlon) cos(lat_s), cos(lat_t) sin(lat_s) - sin(lat_t) cos(lat_s) cos(dlon)),
+ * dlon = lon_s - lon_t, in float64 from the float32 coordinates (8-byte aligned).  norm = AGX_NORM_*, over the whole
+ * edge set with EdgeLength's arithmetic and NaN rule (the K5 fold / parameter / scaling kernels).  AGX_ERR_ARG (after
+ * the pass, one read-back) if an endpoint is outside [0, n_src_nodes) / [0, n_dst_nodes): such an endpoint is never
+ * read and out is then undefined.                                                                                 */
+int agx_edge_azimuth(const int32_t* edge_src /*DEV E*/, const int32_t* edge_dst /*DEV E*/, int64_t n_edges,
+                     const float* src_latlon /*DEV ns*2*/, int64_t n_src_nodes, const float* dst_latlon /*DEV nt*2*/,
+                     int64_t n_dst_nodes, int norm, float* out /*DEV E*/,
+                     double* workspace /*DEV, >= agx_edge_attrs_workspace() doubles*/, void* stream);
+/* agx_gaussian_weights (GaussianDistanceWeights): w = exp(-d^2 / (2 sigma^2)) in float64 from lengths[e] (the float32
+ * EdgeLength values, unit sphere), normalised with norm = AGX_NORM_* within each group of edges that share a target
+ * (edge_dst), rounded to float32 once: out[e] = float32((w - shift[t]) / div[t]).  The statistics of a group are reduced
+ * over its edges in the order of perm - which must be agx_sort_edges(key = edge_dst, other = edge_src, ascending) of
+ * the same rows, so the endpoints are checked and the result does not depend on the column order - in one fixed tree.
+ * unit-std: two passes; a group whose weights are bit-equal is left unnormalised.  A NaN weight makes its group NaN.
+ * norm = AGX_NORM_NONE: out = float32(w), and perm / scratch / edge_dst may be NULL.  edge_src and n_src_nodes are not
+ * read: the weights depend on the lengths and the target row only.  sigma > 0.  No read-back.
+ * scratch: DEV, 16-byte aligned, >= agx_gaussian_weights_scratch_bytes(n_edges, n_dst_nodes) bytes
+ * = 32 n_dst + 64 + 48 (E / 1024 + 1) + 32 (2 (E / 1024) + 2) (a (shift, div) table and the group bounds per target, the
+ * groups of more than 1024 edges and their partial statistics).                                                    */
+int agx_gaussian_weights(const int32_t* edge_src /*DEV E*/, const int32_t* edge_dst /*DEV E*/, int64_t n_edges,
+                         int64_t n_src_nodes, int64_t n_dst_nodes, const float* lengths /*DEV E*/, double sigma, int norm,
+                         const int32_t* perm /*DEV E or NULL for norm None*/, float* out /*DEV E*/,
+                         void* scratch /*DEV or NULL for norm None*/, void* stream);
+int64_t agx_gaussian_weights_scratch_bytes(int64_t n_edges, int64_t n_dst_nodes);
 
 /* ---- icosphere + multi-scale edges -------------------------------------------------------------------
  * agx_icosphere: replaces trimesh.creation.icosphere (generate/tri_icosahedron.py:121,173):
