@@ -14,7 +14,7 @@ import torch
 
 LIB_PATH = Path(__file__).resolve().parent / "lib" / "libagx_b200.so"
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 AGX_OK = 0
 AGX_ERR_CUDA = -1
 AGX_ERR_ARG = -2
@@ -88,23 +88,12 @@ SIGNATURES = {
     "agx_edge_attrs_stats": (
         c_int,
         [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
-         c_void_p, c_void_p, c_void_p],
-    ),  # fmt: skip
-    "agx_edge_attrs_stats_flagged": (
-        c_int,
-        [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
-         c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p],
-    ),  # fmt: skip
-    "agx_edge_attrs_stats_list": (
-        c_int,
-        [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
-         c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+         c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p],
     ),  # fmt: skip
     "agx_edge_attrs_apply": (
         c_int,
-        [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_int,
-         c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p],
-    ),  # fmt: skip
+        [c_int64, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int64, c_void_p, c_void_p],
+    ),
     "agx_edge_azimuth": (
         c_int,
         [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p],

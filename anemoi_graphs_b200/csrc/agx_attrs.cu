@@ -17,8 +17,6 @@
 //    32 B written + 32 B gathered per node where the coordinates cost 8 B; the quaternion needs no trigonometry).
 // The per-edge kernel works on warp tiles of 64 consecutive edges, two ADJACENT edges per lane: 8-byte index loads,
 // all node gathers in flight before the arithmetic, one 8-byte (length) and one 128-bit (direction) store per lane.
-#include <stdlib.h>
-
 #include "agx_common.cuh"
 
 #define ATTR_THREADS 256
@@ -284,10 +282,6 @@ struct AttrArgs {
     const int32_t* only_list;  // with regular_k: the work items are the edges [t k, (t + 1) k) of the listed targets
     const int64_t* only_count;
     int regular_k;
-    // "recompute" second pass: the normalisation parameters (k_attr_params: ws[0..5]) are applied to the values as
-    // they are written, instead of an in-place scaling pass over raw values written earlier
-    const double* norm;  // NULL: write raw values
-    int len_scale, len_invert_final, dir_scale, dir_f64;
 };
 
 template <bool COORD>
@@ -308,12 +302,12 @@ __device__ __forceinline__ DstNode attr_load_dst(const AttrArgs& a, int i, bool 
     return n;
 }
 
-// STATS: reduce the raw values (a shard's statistics, or the first pass).  WRITE: store the raw float32 values - the
+// Stores the raw float32 values; STATS: also reduces them (a shard's statistics, or the first pass) - the
 // normalisation follows as an in-place scaling pass (k_attr_scale), so the trigonometry runs ONCE per edge.
 // J = 2: every lane owns TWO ADJACENT edges of a 64-edge warp tile: the index rows are read as one 8-byte load per lane
 // and row, the lengths leave as one 8-byte store and the directions as ONE 128-bit store (2 edges x 2 floats) - fully
 // coalesced 256 / 512-byte warp transactions.  J = 1 (unaligned rows, the list-driven patch pass): scalar accesses.
-template <bool STATS, bool WRITE, int J, bool SRC_COORD, bool DST_COORD>
+template <bool STATS, int J, bool SRC_COORD, bool DST_COORD>
 __global__ void __launch_bounds__(ATTR_THREADS, 3) k_edge_attrs(AttrArgs a) {
     Stat4 st_len, st_dir;
     st_len.init();
@@ -398,36 +392,16 @@ __global__ void __launch_bounds__(ATTR_THREADS, 3) k_edge_attrs(AttrArgs a) {
                 }
             }
         }
-        if (WRITE && a.norm != nullptr) {
-            // the same arithmetic as k_attr_scale on the float32 value that would have been stored
+        if (J == 2 && live[0] && live[J - 1] && eid[J - 1] == eid[0] + 1 && (eid[0] & 1) == 0) {
+            if (a.want_len) *reinterpret_cast<float2*>(a.out_len + eid[0]) = make_float2(vlen[0], vlen[J - 1]);
+            if (a.want_dir) *reinterpret_cast<float4*>(a.out_dir + 2 * eid[0]) = make_float4(d0[0], d1[0], d0[J - 1], d1[J - 1]);
+        } else {
 #pragma unroll
-            for (int j = 0; j < J; ++j) {
-                if (a.want_len && (a.len_scale || a.len_invert_final))
-                    vlen[j] = scale_one<false>(vlen[j], a.len_scale ? (float)a.norm[0] : 0.0f, a.len_scale ? (float)a.norm[1] : 1.0f,
-                                               0.0, 1.0, a.len_invert_final);
-                if (a.want_dir && a.dir_scale) {
-                    if (a.dir_f64) {
-                        d0[j] = scale_one<true>(d0[j], 0.0f, 1.0f, a.norm[2], a.norm[3], 0);
-                        d1[j] = scale_one<true>(d1[j], 0.0f, 1.0f, a.norm[2], a.norm[3], 0);
-                    } else {
-                        d0[j] = scale_one<false>(d0[j], (float)a.norm[4], (float)a.norm[5], 0.0, 1.0, 0);
-                        d1[j] = scale_one<false>(d1[j], (float)a.norm[4], (float)a.norm[5], 0.0, 1.0, 0);
-                    }
+            for (int j = 0; j < J; ++j)
+                if (live[j]) {
+                    if (a.want_len) a.out_len[eid[j]] = vlen[j];
+                    if (a.want_dir) reinterpret_cast<float2*>(a.out_dir)[eid[j]] = make_float2(d0[j], d1[j]);
                 }
-            }
-        }
-        if (WRITE) {
-            if (J == 2 && live[0] && live[J - 1] && eid[J - 1] == eid[0] + 1 && (eid[0] & 1) == 0) {
-                if (a.want_len) *reinterpret_cast<float2*>(a.out_len + eid[0]) = make_float2(vlen[0], vlen[J - 1]);
-                if (a.want_dir) *reinterpret_cast<float4*>(a.out_dir + 2 * eid[0]) = make_float4(d0[0], d1[0], d0[J - 1], d1[J - 1]);
-            } else {
-#pragma unroll
-                for (int j = 0; j < J; ++j)
-                    if (live[j]) {
-                        if (a.want_len) a.out_len[eid[j]] = vlen[j];
-                        if (a.want_dir) reinterpret_cast<float2*>(a.out_dir)[eid[j]] = make_float2(d0[j], d1[j]);
-                    }
-            }
         }
     }
     if (STATS) {
@@ -457,7 +431,7 @@ __global__ void __launch_bounds__(ATTR_THREADS, 3) k_edge_attrs(AttrArgs a) {
 // ONCE, evaluates its cos(lat) / rotation quaternion once and walks its k sources.  A third of the target-side
 // arithmetic and loads of the edge-centric kernel for k = 3, and the target row is read once per target (its first
 // column) instead of once per edge.
-template <bool STATS, bool WRITE, bool SRC_COORD, bool DST_COORD>
+template <bool STATS, bool SRC_COORD, bool DST_COORD>
 __global__ void __launch_bounds__(ATTR_THREADS, 3) k_edge_attrs_regular(AttrArgs a) {
     Stat4 st_len, st_dir;
     st_len.init();
@@ -482,7 +456,7 @@ __global__ void __launch_bounds__(ATTR_THREADS, 3) k_edge_attrs_regular(AttrArgs
             if (a.want_len) {
                 const float v = edge_length_raw(make_float2(sn.lat, sn.lon), sn.cl, make_float2(dn.lat, dn.lon), ct);
                 if (STATS && counted) st_len.add((double)v, v);
-                if (WRITE) a.out_len[e] = a.len_invert_now ? __fsub_rn(1.0f, v) : v;
+                a.out_len[e] = a.len_invert_now ? __fsub_rn(1.0f, v) : v;
             }
             if (a.want_dir) {
                 float f0, f1;
@@ -503,7 +477,7 @@ __global__ void __launch_bounds__(ATTR_THREADS, 3) k_edge_attrs_regular(AttrArgs
                         st_dir.add((double)f1, f1);
                     }
                 }
-                if (WRITE) reinterpret_cast<float2*>(a.out_dir)[e] = make_float2(f0, f1);
+                reinterpret_cast<float2*>(a.out_dir)[e] = make_float2(f0, f1);
             }
         }
     }
@@ -680,59 +654,45 @@ static inline int attrs_grid(int64_t n_edges, int j) {
     return grid > ATTR_MAX_BLOCKS ? ATTR_MAX_BLOCKS : grid;
 }
 
-template <bool STATS, bool WRITE, int J>
+template <bool STATS, int J>
 static void attrs_launch_modes(int grid, cudaStream_t stream, const AttrArgs& a) {
     const bool sc = a.s_rec == nullptr, dc = a.t_rec == nullptr;
     if (sc && dc)
-        k_edge_attrs<STATS, WRITE, J, true, true><<<grid, ATTR_THREADS, 0, stream>>>(a);
+        k_edge_attrs<STATS, J, true, true><<<grid, ATTR_THREADS, 0, stream>>>(a);
     else if (sc)
-        k_edge_attrs<STATS, WRITE, J, true, false><<<grid, ATTR_THREADS, 0, stream>>>(a);
+        k_edge_attrs<STATS, J, true, false><<<grid, ATTR_THREADS, 0, stream>>>(a);
     else if (dc)
-        k_edge_attrs<STATS, WRITE, J, false, true><<<grid, ATTR_THREADS, 0, stream>>>(a);
+        k_edge_attrs<STATS, J, false, true><<<grid, ATTR_THREADS, 0, stream>>>(a);
     else
-        k_edge_attrs<STATS, WRITE, J, false, false><<<grid, ATTR_THREADS, 0, stream>>>(a);
+        k_edge_attrs<STATS, J, false, false><<<grid, ATTR_THREADS, 0, stream>>>(a);
 }
 
-template <bool STATS, bool WRITE>
+template <bool STATS>
 static void attrs_launch_regular(int grid, cudaStream_t stream, const AttrArgs& a) {
     const bool sc = a.s_rec == nullptr, dc = a.t_rec == nullptr;
     if (sc && dc)
-        k_edge_attrs_regular<STATS, WRITE, true, true><<<grid, ATTR_THREADS, 0, stream>>>(a);
+        k_edge_attrs_regular<STATS, true, true><<<grid, ATTR_THREADS, 0, stream>>>(a);
     else if (sc)
-        k_edge_attrs_regular<STATS, WRITE, true, false><<<grid, ATTR_THREADS, 0, stream>>>(a);
+        k_edge_attrs_regular<STATS, true, false><<<grid, ATTR_THREADS, 0, stream>>>(a);
     else if (dc)
-        k_edge_attrs_regular<STATS, WRITE, false, true><<<grid, ATTR_THREADS, 0, stream>>>(a);
+        k_edge_attrs_regular<STATS, false, true><<<grid, ATTR_THREADS, 0, stream>>>(a);
     else
-        k_edge_attrs_regular<STATS, WRITE, false, false><<<grid, ATTR_THREADS, 0, stream>>>(a);
+        k_edge_attrs_regular<STATS, false, false><<<grid, ATTR_THREADS, 0, stream>>>(a);
 }
 
 template <int J>
-static void attrs_launch(bool stats, bool write, int grid, cudaStream_t stream, const AttrArgs& a) {
-    if (stats && write)
-        attrs_launch_modes<true, true, J>(grid, stream, a);
-    else if (stats)
-        attrs_launch_modes<true, false, J>(grid, stream, a);
+static void attrs_launch(bool stats, int grid, cudaStream_t stream, const AttrArgs& a) {
+    if (stats)
+        attrs_launch_modes<true, J>(grid, stream, a);
     else
-        attrs_launch_modes<false, true, J>(grid, stream, a);
+        attrs_launch_modes<false, J>(grid, stream, a);
 }
 
-// AGX_ATTR_RECOMPUTE=1: normalise by a second evaluation instead of an in-place scaling pass (measured alternative)
-static inline bool attrs_recompute() {
-    static int v = -1;
-    if (v < 0) {
-        const char* env = getenv("AGX_ATTR_RECOMPUTE");
-        v = (env && atoi(env) == 1) ? 1 : 0;
-    }
-    return v == 1;
-}
-
-// pass A: raw values of the local edges -> out_* (float32) and/or stats[8]
+// pass A: raw values of the local edges -> out_* (float32), and stats[8] when stats is given
 static int attrs_raw(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, const AttrNodes& nd, int want_len,
-                     int len_invert_now, float* out_len, int want_dir, int dir_rotated, float* out_dir, bool write,
-                     double* stats, double* workspace, cudaStream_t stream, const uint8_t* dst_flags = nullptr,
-                     int flag_mode = 0, const int32_t* only_list = nullptr, const int64_t* only_count = nullptr,
-                     int regular_k = 0, const double* norm = nullptr, int len_scale = 0, int len_invert_final = 0,
-                     int dir_scale = 0) {
+                     int len_invert_now, float* out_len, int want_dir, int dir_rotated, float* out_dir, double* stats,
+                     double* workspace, cudaStream_t stream, const uint8_t* dst_flags, int flag_mode,
+                     const int32_t* only_list, const int64_t* only_count, int regular_k) {
     int grid = 0;
     if (n_edges > 0 && (want_len || want_dir)) {
         AttrArgs a;
@@ -747,39 +707,32 @@ static int attrs_raw(const int32_t* edge_src, const int32_t* edge_dst, int64_t n
         a.len_invert_now = len_invert_now;
         a.want_dir = want_dir;
         a.dir_rotated = dir_rotated;
-        a.out_len = write ? out_len : nullptr;
-        a.out_dir = write ? out_dir : nullptr;
+        a.out_len = out_len;
+        a.out_dir = out_dir;
         a.ws = workspace;
         a.dst_flags = dst_flags;
         a.flag_mode = flag_mode;
         a.only_list = only_list;
         a.only_count = only_count;
         a.regular_k = regular_k;
-        a.norm = norm;
-        a.len_scale = len_scale;
-        a.len_invert_final = len_invert_final;
-        a.dir_scale = dir_scale;
-        a.dir_f64 = dir_rotated;
         // two adjacent edges per lane need 8-byte aligned index rows and 8 / 16-byte aligned outputs (a (2, E) list with
         // odd E, or a block that starts at an odd column, is not): scalar lanes then
         const bool aligned = (((uintptr_t)edge_src | (uintptr_t)edge_dst | (uintptr_t)out_len) & 7) == 0 &&
                              ((uintptr_t)out_dir & 15) == 0;
         const int j = (only_list == nullptr && aligned) ? 2 : 1;
-        if (only_list == nullptr && regular_k > 0 && norm == nullptr) {
+        if (only_list == nullptr && regular_k > 0) {
             // a regular-k list (KNN result) walked by target
             grid = attrs_grid(n_edges / regular_k, 1);
-            if (stats != nullptr && write)
-                attrs_launch_regular<true, true>(grid, stream, a);
-            else if (stats != nullptr)
-                attrs_launch_regular<true, false>(grid, stream, a);
+            if (stats != nullptr)
+                attrs_launch_regular<true>(grid, stream, a);
             else
-                attrs_launch_regular<false, true>(grid, stream, a);
+                attrs_launch_regular<false>(grid, stream, a);
         } else {
             grid = only_list ? 32 : attrs_grid(n_edges, j);
             if (j == 2)
-                attrs_launch<2>(stats != nullptr, write, grid, stream, a);
+                attrs_launch<2>(stats != nullptr, grid, stream, a);
             else
-                attrs_launch<1>(stats != nullptr, write, grid, stream, a);
+                attrs_launch<1>(stats != nullptr, grid, stream, a);
         }
         agx_note_launch(1);
     }
@@ -812,67 +765,39 @@ static int attrs_scale(int64_t n_edges, int len_norm, int len_invert, float* out
 extern "C" int agx_edge_attrs_stats(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges,
                                     const float* src_rec, const float* src_latlon, const double* dst_rec,
                                     const float* dst_latlon, int want_len, int want_dir, int dir_rotated, float* out_len,
-                                    float* out_dir, double* stats, double* workspace, void* stream_) {
-    return agx_edge_attrs_stats_flagged(edge_src, edge_dst, n_edges, src_rec, src_latlon, dst_rec, dst_latlon, want_len,
-                                        want_dir, dir_rotated, out_len, out_dir, stats, workspace, nullptr, 0, 0, stream_);
-}
-
-extern "C" int agx_edge_attrs_stats_flagged(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges,
-                                            const float* src_rec, const float* src_latlon, const double* dst_rec,
-                                            const float* dst_latlon, int want_len, int want_dir, int dir_rotated,
-                                            float* out_len, float* out_dir, double* stats, double* workspace,
-                                            const uint8_t* dst_flags, int flag_mode, int regular_k, void* stream_) {
+                                    float* out_dir, double* stats, double* workspace, const uint8_t* dst_flags,
+                                    int flag_mode, const int32_t* list, const int64_t* count, int regular_k,
+                                    void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
     AGX_REQUIRE(regular_k >= 0 && (regular_k == 0 || n_edges % regular_k == 0), AGX_ERR_ARG,
-                "agx_edge_attrs_stats_flagged: n_edges is not a multiple of regular_k");
+                "agx_edge_attrs_stats: n_edges is not a multiple of regular_k");
     AGX_REQUIRE(stats != nullptr, AGX_ERR_ARG, "agx_edge_attrs_stats: stats is NULL");
     AGX_REQUIRE(workspace != nullptr, AGX_ERR_ARG, "agx_edge_attrs_stats: workspace is NULL");
-    AGX_REQUIRE(flag_mode == 0 || ((flag_mode == AGX_ATTR_FLAGS_SKIP || flag_mode == AGX_ATTR_FLAGS_ONLY) && dst_flags),
-                AGX_ERR_ARG, "agx_edge_attrs_stats_flagged: flag_mode must be 0, 1 (skip) or 2 (only) with dst_flags");
+    AGX_REQUIRE(flag_mode == 0 || flag_mode == AGX_ATTR_FLAGS_SKIP || flag_mode == AGX_ATTR_FLAGS_ONLY, AGX_ERR_ARG,
+                "agx_edge_attrs_stats: flag_mode must be 0, 1 (skip) or 2 (only)");
+    AGX_REQUIRE((list != nullptr) == (count != nullptr), AGX_ERR_ARG, "agx_edge_attrs_stats: give list and count together");
+    AGX_REQUIRE(!list || (flag_mode == AGX_ATTR_FLAGS_ONLY && !dst_flags && regular_k > 0), AGX_ERR_ARG,
+                "agx_edge_attrs_stats: a target list replaces dst_flags in flag_mode 2 (only) with regular_k > 0");
+    AGX_REQUIRE(list || flag_mode == 0 || dst_flags, AGX_ERR_ARG,
+                "agx_edge_attrs_stats: flag_mode 1 (skip) needs dst_flags, 2 (only) dst_flags or a target list");
     const AttrNodes nd = {src_rec, src_latlon, dst_rec, dst_latlon};
     int rc = attrs_check(edge_src, edge_dst, n_edges, nd, workspace);
     if (rc || (rc = attrs_check_dir(out_dir))) return rc;
-    bool write = (want_len && out_len) || (want_dir && out_dir);
-    AGX_REQUIRE(!write || ((!want_len || out_len) && (!want_dir || out_dir)), AGX_ERR_ARG,
-                "agx_edge_attrs_stats: give every requested output buffer or none");
-    AGX_REQUIRE(write || flag_mode != AGX_ATTR_FLAGS_ONLY, AGX_ERR_ARG, "agx_edge_attrs_stats_flagged: the only-pass writes");
-    return attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, 0, out_len, want_dir, dir_rotated, out_dir, write, stats,
-                     workspace, stream, dst_flags, flag_mode, nullptr, nullptr, regular_k);
+    AGX_REQUIRE(n_edges == 0 || ((!want_len || out_len) && (!want_dir || out_dir)), AGX_ERR_ARG,
+                "agx_edge_attrs_stats: give every requested output buffer");
+    // the list IS the set of "only" targets: the kernel then reads no flags
+    return attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, 0, out_len, want_dir, dir_rotated, out_dir, stats,
+                     workspace, stream, dst_flags, list ? 0 : flag_mode, list, count, regular_k);
 }
 
-// Raw values + statistics of the edges of a LIST of targets of a regular-k edge list (a KNN result: the edges of target
-// t are [t k, (t + 1) k)); the list length lives in device memory.  One small launch, sized for a few thousand targets.
-extern "C" int agx_edge_attrs_stats_list(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, int regular_k,
-                                         const int32_t* list, const int64_t* count, const float* src_rec,
-                                         const float* src_latlon, const double* dst_rec, const float* dst_latlon,
-                                         int want_len, int want_dir, int dir_rotated, float* out_len, float* out_dir,
-                                         double* stats, double* workspace, void* stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
-    AGX_REQUIRE(stats && workspace && list && count, AGX_ERR_ARG, "agx_edge_attrs_stats_list: NULL buffer");
-    AGX_REQUIRE(regular_k > 0 && n_edges % regular_k == 0, AGX_ERR_ARG, "agx_edge_attrs_stats_list: n_edges is not a multiple of k");
-    const AttrNodes nd = {src_rec, src_latlon, dst_rec, dst_latlon};
-    int rc = attrs_check(edge_src, edge_dst, n_edges, nd, workspace);
-    if (rc || (rc = attrs_check_dir(out_dir))) return rc;
-    AGX_REQUIRE((!want_len || out_len) && (!want_dir || out_dir), AGX_ERR_ARG,
-                "agx_edge_attrs_stats_list: give every requested output buffer");
-    return attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, 0, out_len, want_dir, dir_rotated, out_dir, true, stats,
-                     workspace, stream, nullptr, 0, list, count, regular_k);
-}
-
-extern "C" int agx_edge_attrs_apply(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges,
-                                    const float* src_rec, const float* src_latlon, const double* dst_rec,
-                                    const float* dst_latlon, int len_norm, int len_invert, float* out_len, int dir_norm,
+extern "C" int agx_edge_attrs_apply(int64_t n_edges, int len_norm, int len_invert, float* out_len, int dir_norm,
                                     int dir_rotated, float* out_dir, const double* stats, int n_stat_sets,
-                                    int64_t n_edges_global, int raw_present, double* workspace, void* stream_) {
+                                    int64_t n_edges_global, double* workspace, void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
     int want_len = len_norm >= 0, want_dir = dir_norm >= 0;
     AGX_REQUIRE(len_norm <= AGX_NORM_UNIT_STD && dir_norm <= AGX_NORM_UNIT_STD, AGX_ERR_ARG, "agx_edge_attrs: unknown norm code");
+    AGX_REQUIRE(n_edges >= 0, AGX_ERR_ARG, "agx_edge_attrs_apply: n_edges < 0");
     if (n_edges == 0 || (!want_len && !want_dir)) return AGX_OK;
-    const AttrNodes nd = {src_rec, src_latlon, dst_rec, dst_latlon};
-    if (!raw_present) {
-        int rc = attrs_check(edge_src, edge_dst, n_edges, nd, workspace);
-        if (rc) return rc;
-    }
     if (int rc = attrs_check_dir(out_dir)) return rc;
     AGX_REQUIRE(workspace != nullptr, AGX_ERR_ARG, "agx_edge_attrs_apply: workspace is NULL");
     AGX_REQUIRE(!want_len || out_len, AGX_ERR_ARG, "agx_edge_attrs: out_len is NULL");
@@ -881,11 +806,6 @@ extern "C" int agx_edge_attrs_apply(const int32_t* edge_src, const int32_t* edge
     AGX_REQUIRE(!need_stats || (stats && n_stat_sets >= 1), AGX_ERR_ARG,
                 "agx_edge_attrs_apply: this normalisation needs the statistics of every shard");
     AGX_REQUIRE(n_edges_global >= n_edges, AGX_ERR_ARG, "agx_edge_attrs_apply: n_edges_global < n_edges");
-    if (!raw_present) {
-        int rc = attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, 0, out_len, want_dir, dir_rotated, out_dir, true,
-                           nullptr, workspace, stream);
-        if (rc) return rc;
-    }
     return attrs_scale(n_edges, len_norm, len_invert, out_len, dir_norm, dir_rotated, out_dir, stats, n_stat_sets,
                        n_edges_global, workspace, stream);
 }
@@ -908,23 +828,11 @@ extern "C" int agx_edge_attrs(const int32_t* edge_src, const int32_t* edge_dst, 
     bool need_stats = (want_len && len_norm > 0) || (want_dir && dir_norm > 0);
     double* stats = need_stats ? workspace + 6 : nullptr;  // ws[6..13]: between the parameters and the block partials
     // no normalisation: the raw pass writes the final values (an inversion needs no statistics)
-    if (!need_stats || !attrs_recompute())
-        rc = attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, need_stats ? 0 : len_invert, out_len, want_dir, dir_rotated,
-                       out_dir, true, stats, workspace, stream, nullptr, 0, nullptr, nullptr, regular_k);
+    rc = attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, need_stats ? 0 : len_invert, out_len, want_dir, dir_rotated,
+                   out_dir, stats, workspace, stream, nullptr, 0, nullptr, nullptr, regular_k);
     if (rc || !need_stats) return rc;
-    if (!attrs_recompute())
-        return attrs_scale(n_edges, len_norm, len_invert, out_len, dir_norm, dir_rotated, out_dir, stats, 1, n_edges,
-                           workspace, stream);
-    // "recompute" form (AGX_ATTR_RECOMPUTE=1): a statistics-only pass (nothing written), the parameters, then a second
-    // evaluation that writes the normalised values: 8 + 8 + 12 bytes per edge instead of 8 + 12 + 24, twice the arithmetic
-    rc = attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, 0, nullptr, want_dir, dir_rotated, nullptr, false, stats,
-                   workspace, stream);
-    if (rc) return rc;
-    k_attr_params<<<1, 32, 0, stream>>>(workspace, stats, 1, n_edges, want_len ? len_norm : 0, want_dir ? dir_norm : 0);
-    agx_note_launch(1);
-    return attrs_raw(edge_src, edge_dst, n_edges, nd, want_len, 0, out_len, want_dir, dir_rotated, out_dir, true, nullptr,
-                     workspace, stream, nullptr, 0, nullptr, nullptr, 0, workspace, want_len && len_norm > 0,
-                     want_len && len_invert, want_dir && dir_norm > 0);
+    return attrs_scale(n_edges, len_norm, len_invert, out_len, dir_norm, dir_rotated, out_dir, stats, 1, n_edges,
+                       workspace, stream);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -1539,31 +1539,16 @@ def all_gather_count_rows(mine: list[int], device: torch.device) -> list[list[in
 
 
 def all_gather_stats_raw(stats: torch.Tensor) -> torch.Tensor:
-    """Per-rank attribute statistics stacked in rank order: (W, 8) float64.  The attribute kernel folds them in
-    that order (``agx_edge_attrs_apply(n_stat_sets=W)``), so every rank applies bit-identical constants."""
+    """Per-rank attribute statistics stacked in rank order: (W, n) float64 for the n doubles of ``stats`` (one or more
+    sets of 8).  The attribute kernel folds the sets in that order (``agx_edge_attrs_apply``), so every rank applies
+    bit-identical constants."""
     import torch.distributed as dist
 
+    n = stats.numel()
+    assert n % 8 == 0, "attribute statistics come in sets of 8 doubles"
     _, w = world()
     if w == 1:
-        return stats.reshape(1, 8)
-    allst = torch.empty((w, 8), dtype=stats.dtype, device=stats.device)
-    dist.all_gather_into_tensor(allst, stats.reshape(1, 8))
+        return stats.reshape(1, n)
+    allst = torch.empty((w, n), dtype=stats.dtype, device=stats.device)
+    dist.all_gather_into_tensor(allst, stats.reshape(1, n))
     return allst
-
-
-def all_gather_stats(stats: torch.Tensor) -> torch.Tensor:
-    """Combine per-rank attribute statistics {sum, sumsq, min, max} x {len, dir} in rank order."""
-    import torch.distributed as dist
-
-    _, w = world()
-    if w == 1:
-        return stats
-    allst = torch.empty((w, 8), dtype=stats.dtype, device=stats.device)
-    dist.all_gather_into_tensor(allst, stats.reshape(1, 8))
-    out = torch.empty_like(stats)
-    for base in (0, 4):
-        out[base] = allst[:, base].sum()
-        out[base + 1] = allst[:, base + 1].sum()
-        out[base + 2] = allst[:, base + 2].min()
-        out[base + 3] = allst[:, base + 3].max()
-    return out

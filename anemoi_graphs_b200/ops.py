@@ -460,39 +460,15 @@ def edge_attributes(
     len_code = NORM_CODES[length_norm] if length else -1
     dir_code = NORM_CODES[direction_norm] if direction else -1
     rank, w = _device.world() if sharded else (0, 1)
-    if shard is not None and shard.world > 1 and not shard.replicated:
-        # sharded output mode: ``edge_index`` IS this rank's block.  One pass for the raw values and the block's
-        # statistics, the (W, 8) statistics all-gathered (folded in rank order inside the kernel), scaling in place;
-        # the attribute blocks stay on their ranks.
-        ws, stream = _attr_workspace(dev), current_stream()
-        e_src, e_dst = edge_index[0].data_ptr(), edge_index[1].data_ptr()
-        stats = None
-        if len_code > 0 or dir_code > 0:
-            stats = torch.empty(8, dtype=torch.float64, device=dev)
-            with _span("edge_attrs_stats", n_edges):
-                check(
-                    lib.agx_edge_attrs_stats(
-                        e_src, e_dst, n_edges, *nodes, int(length), int(direction),
-                        int(bool(direction_rotated)), ptr(out_len), ptr(out_dir), ptr(stats), ptr(ws), stream,
-                    )
-                )
-            stats = _device.all_gather_stats_raw(stats)
-        with _span("edge_attrs_apply", n_edges):
-            check(
-                lib.agx_edge_attrs_apply(
-                    e_src, e_dst, n_edges, *nodes, len_code, int(bool(length_invert)), ptr(out_len),
-                    dir_code, int(bool(direction_rotated)), ptr(out_dir), ptr(stats), shard.world if stats is not None else 0,
-                    shard.total, 1 if stats is not None else 0, ptr(ws), stream,
-                )
-            )
-        return out_len, out_dir
-    if shard is not None:
+    # sharded output mode: ``edge_index`` IS this rank's block, and the attribute blocks stay on their ranks
+    own_block = shard is not None and shard.world > 1 and not shard.replicated
+    if shard is not None and not own_block:
         w = 1  # a replicated set in sharded output mode: every rank evaluates all of it
-    if w > 1 and local is None and n_edges < ATTR_SHARD_MIN_EDGES:
+    if w > 1 and not own_block and local is None and n_edges < ATTR_SHARD_MIN_EDGES:
         w = 1  # small edge set: every rank evaluates all of it (identical results, no exchange)
     ws = _attr_workspace(dev)
     stream = current_stream()
-    if w == 1:
+    if w == 1 and not own_block:
         _device.wait_for(edge_index)
         with _span("edge_attrs", n_edges):
             check(
@@ -503,7 +479,11 @@ def edge_attributes(
                 )
             )  # fmt: skip
         return out_len, out_dir
-    if local is not None:
+    # this rank's block [lo, hi) of the edges and of the outputs; ``counts``: every rank's block size (all-gathered)
+    n_global, counts = n_edges, None
+    if own_block:
+        lo, hi, n_global, w = 0, n_edges, shard.total, shard.world
+    elif local is not None:
         lo, hi, counts = local
         assert sum(counts) == n_edges and hi - lo == counts[rank]
     else:
@@ -514,32 +494,38 @@ def edge_attributes(
     e_src, e_dst = edge_index[0].data_ptr() + 4 * lo, edge_index[1].data_ptr() + 4 * lo
     o_len = out_len.data_ptr() + 4 * lo if length else None
     o_dir = out_dir.data_ptr() + 8 * lo if direction else None
-    stats = None
-    raw_present = 0
     if len_code > 0 or dir_code > 0:
-        # one pass over the local edges: raw float32 values into this rank's slot + the local statistics
+        # one pass over the block: raw float32 values + the block's statistics; then every rank's statistics (folded
+        # in rank order inside the kernel) and the scaling in place
         stats = torch.empty(8, dtype=torch.float64, device=dev)
         with _span("edge_attrs_stats", m):
             check(
                 lib.agx_edge_attrs_stats(
-                    e_src, e_dst, m, *nodes, int(length), int(direction),
-                    int(bool(direction_rotated)), o_len, o_dir, ptr(stats), ptr(ws), stream,
+                    e_src, e_dst, m, *nodes, int(length), int(direction), int(bool(direction_rotated)), o_len, o_dir,
+                    ptr(stats), ptr(ws), None, 0, None, None, 0, stream,
                 )
             )  # fmt: skip
         stats = _device.all_gather_stats_raw(stats)
-        raw_present = 1
-    with _span("edge_attrs_apply", m):
-        check(
-            lib.agx_edge_attrs_apply(
-                e_src, e_dst, m, *nodes, len_code, int(bool(length_invert)), o_len, dir_code,
-                int(bool(direction_rotated)), o_dir, ptr(stats), w if stats is not None else 0, n_edges, raw_present,
-                ptr(ws), stream,
-            )
-        )  # fmt: skip
-    if length:
-        _device.all_gather_v(out_len, counts, 0, async_op=True)
-    if direction:
-        _device.all_gather_v(out_dir, counts, 0, async_op=True)
+        with _span("edge_attrs_apply", m):
+            check(
+                lib.agx_edge_attrs_apply(
+                    m, len_code, int(bool(length_invert)), o_len, dir_code, int(bool(direction_rotated)), o_dir,
+                    ptr(stats), w, n_global, ptr(ws), stream,
+                )
+            )  # fmt: skip
+    else:
+        with _span("edge_attrs_apply", m):  # no statistics: the raw pass writes the final values
+            check(
+                lib.agx_edge_attrs(
+                    e_src, e_dst, m, *nodes, len_code, int(bool(length_invert)), o_len, dir_code,
+                    int(bool(direction_rotated)), o_dir, ptr(ws), 0, stream,
+                )
+            )  # fmt: skip
+    if counts is not None:
+        if length:
+            _device.all_gather_v(out_len, counts, 0, async_op=True)
+        if direction:
+            _device.all_gather_v(out_dir, counts, 0, async_op=True)
     return out_len, out_dir
 
 
@@ -714,58 +700,43 @@ class DeferredEdgeAttributes:
         self.stats = torch.tensor([[0.0, 0.0, 1e300, -1e300] * 2] * 2, dtype=torch.float64, device=dev)  # "no value"
         self.ws = _attr_workspace(dev)
 
-    def _pass(self, which: int, mode: int, tag: str) -> None:
+    def _stats(self, which: int, tag: str, work: int, mode: int, regular_k: int, listed: bool = False) -> None:
+        """Raw values + statistics set ``which``; ``listed``: the flagged targets are ``flag_list`` / ``flag_count``."""
         if self.n_edges == 0:
             return
         ei = self.edge_index
-        with _span(tag, self.n_edges if mode == ATTR_FLAGS_SKIP else 0):
+        flags = None if listed else self.flags.data_ptr() - self.flag_base
+        with _span(tag, work):
             check(
-                load_library().agx_edge_attrs_stats_flagged(
+                load_library().agx_edge_attrs_stats(
                     ei[0].data_ptr(), ei[1].data_ptr(), self.n_edges, *self.nodes,
                     int(self.length), int(self.direction), int(self.rotated), ptr(self.out_len), ptr(self.out_dir),
-                    self.stats[which].data_ptr(), ptr(self.ws), self.flags.data_ptr() - self.flag_base, mode,
-                    self.regular_k if mode == ATTR_FLAGS_SKIP else 0, current_stream(),
+                    self.stats[which].data_ptr(), ptr(self.ws), flags, mode, ptr(self.flag_list) if listed else None,
+                    ptr(self.flag_count) if listed else None, regular_k, current_stream(),
                 )
             )
 
     def raw(self) -> None:
-        self._pass(0, ATTR_FLAGS_SKIP, "edge_attrs_raw")
+        self._stats(0, "edge_attrs_raw", self.n_edges, ATTR_FLAGS_SKIP, self.regular_k)
 
     def patch(self) -> None:
-        if self.flag_list is None or self.regular_k <= 0:
-            self._pass(1, ATTR_FLAGS_ONLY, "edge_attrs_patch")
-            return
-        if self.n_edges == 0:
-            return
-        ei = self.edge_index
-        with _span("edge_attrs_patch", 0):
-            check(
-                load_library().agx_edge_attrs_stats_list(
-                    ei[0].data_ptr(), ei[1].data_ptr(), self.n_edges, self.regular_k, ptr(self.flag_list),
-                    ptr(self.flag_count), *self.nodes, int(self.length), int(self.direction),
-                    int(self.rotated), ptr(self.out_len), ptr(self.out_dir), self.stats[1].data_ptr(), ptr(self.ws),
-                    current_stream(),
-                )
-            )
+        listed = self.flag_list is not None and self.regular_k > 0
+        self._stats(1, "edge_attrs_patch", 0, ATTR_FLAGS_ONLY, self.regular_k if listed else 0, listed)
 
     def apply(self) -> None:
-        stats, n_sets, n_global = self.stats, 2, self.n_edges
+        from . import device as _device
+
+        stats, n_global = self.stats, self.n_edges
         if self.shard is not None:
             # every rank's two statistics sets, in rank order (a collective: also ranks without edges take part)
-            import torch.distributed as dist
-
-            allst = torch.empty((self.shard.world, 16), dtype=torch.float64, device=self.stats.device)
-            dist.all_gather_into_tensor(allst, self.stats.reshape(1, 16))
-            stats, n_sets, n_global = allst, 2 * self.shard.world, self.shard.total
+            stats, n_global = _device.all_gather_stats_raw(self.stats), self.shard.total
         if self.n_edges == 0:
             return
-        ei = self.edge_index
         with _span("edge_attrs_scale", self.n_edges):
             check(
                 load_library().agx_edge_attrs_apply(
-                    ei[0].data_ptr(), ei[1].data_ptr(), self.n_edges, *self.nodes, self.len_code,
-                    int(self.invert), ptr(self.out_len), self.dir_code, int(self.rotated), ptr(self.out_dir),
-                    ptr(stats), n_sets, n_global, 1, ptr(self.ws), current_stream(),
+                    self.n_edges, self.len_code, int(self.invert), ptr(self.out_len), self.dir_code, int(self.rotated),
+                    ptr(self.out_dir), ptr(stats), stats.numel() // 8, n_global, ptr(self.ws), current_stream(),
                 )
             )
 

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define AGX_ABI_VERSION 3
+#define AGX_ABI_VERSION 4
 
 #define AGX_OK 0
 #define AGX_ERR_CUDA -1      /* CUDA runtime / launch failure (includes "no device") */
@@ -255,8 +255,8 @@ int agx_gate_open(uint32_t* gate /*HOST page-locked*/, void* stream);
  * an in-place scaling pass.  len_norm / dir_norm = AGX_NORM_* or -1 to skip the attribute;
  * dir_rotated = luse_rotated_features.  A NaN value (an antipodal pair's length) makes every normalised value of its
  * attribute NaN, as numpy's sum / amax / amin / std do in the reference.
- * out_dir, in this call and in _stats, _stats_flagged, _stats_list and _apply, must be 8-byte aligned (one float2
- * store per edge; AGX_ERR_ARG otherwise, before any device work) - a view of an (E, 2) float32 array at any row is. */
+ * out_dir, in this call and in _stats and _apply, must be 8-byte aligned (one float2 store per edge; AGX_ERR_ARG
+ * otherwise, before any device work) - a view of an (E, 2) float32 array at any row is.                           */
 int agx_node_tables(const float* latlon /*DEV n*2*/, int64_t n, float* src_rec /*DEV n*8 or NULL*/,
                     double* dst_rec /*DEV n*4 or NULL, 32-byte aligned*/, void* stream);
 /* Node inputs of the attribute calls, per side EITHER a record table from agx_node_tables (src_rec / dst_rec; small node
@@ -273,42 +273,37 @@ int agx_edge_attrs(const int32_t* edge_src /*DEV E*/, const int32_t* edge_dst /*
                    int regular_k /*k > 0: the edges of the i-th target are columns [i k, (i+1) k) - a KNN result; 0: any list*/,
                    void* stream);
 int64_t agx_edge_attrs_workspace(void);
-/* The two halves of agx_edge_attrs, for callers that hold only a SHARD of the edge set (one rank of a
- * multi-GPU build).  _stats evaluates the raw values of the local edges ONCE: it writes them (float32, not yet
- * normalised) to out_len / out_dir when those are given, and reduces them to
- * stats[8] = {len sum, sum of squares, min, max, dir sum, sum of squares, min, max} (float64; an empty shard
- * gives {0, 0, +1e300, -1e300}).  The caller gathers the shards' statistics and passes all n_stat_sets of them
- * (8 doubles each, in rank order; they are folded in that order, so every rank derives bit-identical constants),
- * with the global edge count, to _apply, which normalises the local block in place (raw_present = 1) or
- * evaluates the raw values first (raw_present = 0).  normalise.py:20-55.                                  */
+/* The two halves of agx_edge_attrs, for callers that normalise over more than one call: one rank's SHARD of a
+ * multi-GPU build, or KNN edges whose sources of a few targets are re-decided later.
+ * _stats evaluates the raw values of the edges ONCE, writes them (float32, not yet normalised) to out_len / out_dir -
+ * every requested output is required - and reduces them to
+ * stats[8] = {len sum, sum of squares, min, max, dir sum, sum of squares, min, max} (float64; an empty set of edges
+ * gives {0, 0, +1e300, -1e300}).  Which edges are evaluated and counted, by a per-TARGET flag byte
+ * (dst_flags: DEV uint8[n_target_nodes]):
+ *   flag_mode 0: every edge (dst_flags is not read);
+ *   flag_mode 1 ("skip"): every edge is evaluated and written, edges INTO a flagged target stay out of the statistics;
+ *   flag_mode 2 ("only"): only the edges into flagged targets are evaluated, written and counted.  Instead of dst_flags
+ *     (then NULL) the flagged targets may be given as a LIST of a regular-k edge list (list = ascending target ids,
+ *     *count = its length, both in device memory - agx_compact_flags; the edges of target t are [t k, (t+1) k)): the
+ *     few re-decided queries then cost one small launch instead of a pass over every target index.
+ * regular_k > 0 without a list: the edges of the i-th target are columns [i k, (i+1) k), walked by target.
+ * For KNN edges built while the source numbering was provisional (agx_knn_flagged): mode 1 right after the search,
+ * mode 2 after agx_knn_redecide_ranked, each into its own statistics set - the decoder's trigonometry then runs in the
+ * shadow of the host sort and only the scaling pass follows it.
+ * _apply is the scaling pass: it normalises the n_edges raw values at out_len / out_dir in place with the
+ * n_stat_sets statistics sets at stats (8 doubles each; every rank's sets, in rank order - they are folded in that
+ * order, so every rank derives bit-identical constants) and the global edge count.  normalise.py:20-55.          */
 int agx_edge_attrs_stats(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, const float* src_rec,
                          const float* src_latlon, const double* dst_rec, const float* dst_latlon, int want_len,
-                         int want_dir, int dir_rotated, float* out_len /*DEV E or NULL*/,
-                         float* out_dir /*DEV E*2 or NULL*/, double* stats /*DEV 8*/, double* workspace, void* stream);
-/* agx_edge_attrs_stats with a per-TARGET flag byte (dst_flags: DEV uint8[n_target_nodes]).  flag_mode 1 ("skip"): every
- * edge is evaluated and written, edges INTO a flagged target stay out of the statistics; flag_mode 2 ("only"): only
- * the edges into flagged targets are evaluated, written and counted.  For KNN edges built while the source numbering
- * was provisional (agx_knn_flagged): mode 1 right after the search, mode 2 after agx_knn_redecide_ranked; the two
- * statistics sets go to agx_edge_attrs_apply (n_stat_sets = 2) - the decoder's trigonometry then runs in the shadow
- * of the host sort and only the scaling pass follows it.                                                          */
-int agx_edge_attrs_stats_flagged(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges,
-                                 const float* src_rec, const float* src_latlon, const double* dst_rec,
-                                 const float* dst_latlon, int want_len, int want_dir, int dir_rotated, float* out_len,
-                                 float* out_dir, double* stats /*DEV 8*/, double* workspace,
-                                 const uint8_t* dst_flags /*DEV*/, int flag_mode, int regular_k, void* stream);
-/* The "only" pass driven by an explicit LIST of targets of a regular-k edge list (edges of target t = [t k, (t+1) k),
- * a KNN result; list = ascending target ids, *count = its length, both in device memory - agx_compact_flags): the few
- * re-decided queries cost one small launch instead of a pass over every target index.                            */
-int agx_edge_attrs_stats_list(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, int regular_k,
-                              const int32_t* list /*DEV*/, const int64_t* count /*DEV*/, const float* src_rec,
-                              const float* src_latlon, const double* dst_rec, const float* dst_latlon, int want_len,
-                              int want_dir, int dir_rotated, float* out_len, float* out_dir, double* stats /*DEV 8*/,
-                              double* workspace, void* stream);
-int agx_edge_attrs_apply(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, const float* src_rec,
-                         const float* src_latlon, const double* dst_rec, const float* dst_latlon, int len_norm,
-                         int len_invert, float* out_len, int dir_norm, int dir_rotated, float* out_dir,
+                         int want_dir, int dir_rotated, float* out_len /*DEV E if want_len*/,
+                         float* out_dir /*DEV E*2 if want_dir*/, double* stats /*DEV 8*/, double* workspace,
+                         const uint8_t* dst_flags /*DEV or NULL*/, int flag_mode /*0, 1 = skip, 2 = only*/,
+                         const int32_t* list /*DEV or NULL*/, const int64_t* count /*DEV or NULL*/, int regular_k,
+                         void* stream);
+int agx_edge_attrs_apply(int64_t n_edges, int len_norm, int len_invert, float* out_len /*DEV E*/, int dir_norm,
+                         int dir_rotated, float* out_dir /*DEV E*2, 8-byte aligned*/,
                          const double* stats /*DEV n_stat_sets*8 or NULL if no norm*/, int n_stat_sets,
-                         int64_t n_edges_global, int raw_present, double* workspace, void* stream);
+                         int64_t n_edges_global, double* workspace, void* stream);
 /* agx_edge_azimuth (Azimuth): out[e] = float32 of the initial bearing at the target towards the source, in radians,
  * clockwise from north, in [-pi, pi]: atan2(sin(dlon) cos(lat_s), cos(lat_t) sin(lat_s) - sin(lat_t) cos(lat_s) cos(dlon)),
  * dlon = lon_s - lon_t, in float64 from the float32 coordinates (8-byte aligned).  norm = AGX_NORM_*, over the whole

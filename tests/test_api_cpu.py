@@ -120,14 +120,14 @@ def test_compute_requires_cuda_no_cpu_fallback():
         KNNEdges("a", "b", 2).update_graph(graph)
 
 
-def test_cabi_exports_every_declared_symbol():
+def test_cabi_library_matches_the_header_and_abi_version():
     header = (_cabi.LIB_PATH.parents[2] / "include" / "agx_b200.h").read_text()
     declared = set(re.findall(r"\b(agx_[a-z0-9_]+)\s*\(", header)) - {"agx_index"}
     assert declared == set(_cabi.SIGNATURES), declared ^ set(_cabi.SIGNATURES)
     lib = _cabi.load_library()
     for name in declared:
         assert isinstance(getattr(lib, name), ctypes._CFuncPtr)
-    assert lib.agx_abi_version() == _cabi.ABI_VERSION == 3
+    assert lib.agx_abi_version() == _cabi.ABI_VERSION == 4
     assert lib.agx_edge_attrs_workspace() > 16
     assert lib.agx_multiscale_scratch_per_node(8, 1) == 9 * 7
 

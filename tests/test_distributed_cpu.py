@@ -1,5 +1,5 @@
 """World-size-2 gloo tests (CPU) of the host logic of the multi-GPU path: shard ranges, the in-place
-variable-length all-gather of per-rank edge blocks, and the rank-order combination of the attribute
+variable-length all-gather of per-rank edge blocks, and the rank-order exchange of the attribute
 statistics.  The kernels themselves need a GPU; here the per-rank blocks are produced with numpy."""
 
 import os
@@ -95,22 +95,24 @@ def _worker(rank: int, world: int, port: int, out_dir: str) -> None:
         lo, hi = agx_device.shard_range(1000)
         part = v[lo:hi]
         st = torch.tensor([part.sum(), (part**2).sum(), part.min(), part.max()] * 2, dtype=torch.float64)
-        tot = agx_device.all_gather_stats(st)
-        np.testing.assert_allclose(tot[0].item(), v.sum(), rtol=1e-14)
-        np.testing.assert_allclose(tot[5].item(), (v**2).sum(), rtol=1e-14)
-        assert tot[2].item() == v.min() and tot[7].item() == v.max()
         raw = agx_device.all_gather_stats_raw(st)  # what the kernel folds, in rank order
         assert raw.shape == (world, 8) and torch.equal(raw[rank], st)
         np.testing.assert_allclose(raw[:, 0].sum().item(), v.sum(), rtol=1e-14)
-        torch.save(tot, os.path.join(out_dir, f"stats{rank}.pt"))
+        np.testing.assert_allclose(raw[:, 5].sum().item(), (v**2).sum(), rtol=1e-14)
+        assert raw[:, 2].min().item() == v.min() and raw[:, 7].max().item() == v.max()
+        # two sets per rank (the deferred decoder's): (W, 16), still rank-major
+        two = agx_device.all_gather_stats_raw(torch.stack([st, 2 * st]))
+        assert two.shape == (world, 16) and torch.equal(two[rank], torch.cat([st, 2 * st]))
+        assert torch.equal(two[:, :8], raw)
+        torch.save(raw, os.path.join(out_dir, f"stats{rank}.pt"))
         dist.barrier()
     finally:
         dist.destroy_process_group()
 
 
 @pytest.mark.timeout(120)
-def test_two_rank_gather_and_stats(tmp_path):
+def test_two_rank_gather_and_statistics_tables(tmp_path):
     port = _free_port()
     mp.spawn(_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
     a, b = torch.load(tmp_path / "stats0.pt"), torch.load(tmp_path / "stats1.pt")
-    assert torch.equal(a, b)  # bitwise identical normalisation constants on every rank
+    assert torch.equal(a, b)  # bitwise identical statistics tables, so identical constants, on every rank

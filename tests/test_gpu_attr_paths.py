@@ -1,8 +1,8 @@
 """Adversarial parity of the edge attribute kernel (K5: ``EdgeLength`` / ``EdgeDirection`` and their normalisation)
 along every code path: both node forms per side, the paired (J = 2) and scalar (J = 1) lanes, the walk by target of a
 regular-k list, the split statistics -> apply form with several statistics sets (a multi-GPU build), the flag modes
-and the list-driven patch pass of the provisional-numbering decoder, the in-place scaling pass at every 16-byte
-misalignment, and the ``AGX_ATTR_RECOMPUTE=1`` form.
+and the list-driven patch pass of the provisional-numbering decoder, and the in-place scaling pass at every
+16-byte misalignment.
 
 Every result is compared with ``oracle/ref_path`` (the reference's own numpy / scipy arithmetic) at the DESIGN section 4
 tolerances: 1e-6 relative, absolute 1e-6 of the array's largest magnitude for ``unit-range`` and inverted lengths and
@@ -20,11 +20,6 @@ Listed exceptions:
 * near-constant attributes, whose standard deviation sits at rounding level, are not generated: ``np.std`` there is
   noise.  The exact ``std == 0`` cases (one edge, two equal edges) are tested."""
 
-import os
-import pathlib
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 import torch
@@ -33,7 +28,6 @@ from oracle import ref_path as R
 
 pytestmark = pytest.mark.gpu
 
-REPO = pathlib.Path(__file__).resolve().parents[1]
 ATTR_RTOL = 1e-6
 FOLD_RTOL = 3e-7  # the same statistics folded in a different association (sum-based norms only)
 NORMS = [None, "l1", "l2", "unit-max", "unit-range", "unit-std"]
@@ -333,31 +327,39 @@ class Call:
             regular_k, _stream()))  # fmt: skip
         return self.result()
 
-    def stats(self, lo, hi, st, rotated, write=True):
+    def stats(self, lo, hi, st, rotated):
         """agx_edge_attrs_stats over the columns [lo, hi) into the 8 doubles at st."""
         _check(self.lib.agx_edge_attrs_stats(
-            self.col(0, lo), self.col(1, lo), hi - lo, *self.nodes, 1, 1, int(rotated),
-            self.len_ptr(lo) if write else None, self.dir_ptr(lo) if write else None, st, self.ws.data_ptr(),
-            _stream()))  # fmt: skip
+            self.col(0, lo), self.col(1, lo), hi - lo, *self.nodes, 1, 1, int(rotated), self.len_ptr(lo),
+            self.dir_ptr(lo), st, self.ws.data_ptr(), None, 0, None, None, 0, _stream()))  # fmt: skip
 
-    def apply(self, lo, hi, len_norm, invert, dir_norm, rotated, stats, n_sets, raw_present):
+    def apply(self, lo, hi, len_norm, invert, dir_norm, rotated, stats, n_sets):
         codes = self.ops.NORM_CODES
         _check(self.lib.agx_edge_attrs_apply(
-            self.col(0, lo), self.col(1, lo), hi - lo, *self.nodes, codes[len_norm], int(invert), self.len_ptr(lo),
-            codes[dir_norm], int(rotated), self.dir_ptr(lo), stats.data_ptr(), n_sets, self.E, raw_present,
-            self.ws.data_ptr(), _stream()))  # fmt: skip
+            hi - lo, codes[len_norm], int(invert), self.len_ptr(lo), codes[dir_norm], int(rotated), self.dir_ptr(lo),
+            stats.data_ptr(), n_sets, self.E, self.ws.data_ptr(), _stream()))  # fmt: skip
 
-    def sharded(self, bounds, len_norm, invert, dir_norm, rotated, raw_present):
+    def sharded(self, bounds, len_norm, invert, dir_norm, rotated):
         """Blocks [bounds[r], bounds[r + 1]) evaluated as the ranks of a multi-GPU build would: statistics per block
         into a (W, 8) tensor, then every block normalised with all W sets."""
         w = len(bounds) - 1
         st = torch.full((w, 8), float("nan"), dtype=torch.float64, device="cuda")
         self.outputs()
         for r in range(w):
-            self.stats(bounds[r], bounds[r + 1], st[r].data_ptr(), rotated, write=bool(raw_present))
+            self.stats(bounds[r], bounds[r + 1], st[r].data_ptr(), rotated)
         for r in range(w):
-            self.apply(bounds[r], bounds[r + 1], len_norm, invert, dir_norm, rotated, st, w, raw_present)
+            self.apply(bounds[r], bounds[r + 1], len_norm, invert, dir_norm, rotated, st, w)
         return (*self.result(), st.cpu().numpy(), bounds)
+
+    def blocks(self, bounds, invert, rotated):
+        """Every block in its own agx_edge_attrs call without a norm: how the ranks of a multi-GPU build evaluate
+        an un-normalised edge set (no statistics to exchange)."""
+        self.outputs()
+        for lo, hi in zip(bounds[:-1], bounds[1:]):
+            _check(self.lib.agx_edge_attrs(
+                self.col(0, lo), self.col(1, lo), hi - lo, *self.nodes, 0, int(invert), self.len_ptr(lo), 0,
+                int(rotated), self.dir_ptr(lo), self.ws.data_ptr(), 0, _stream()))  # fmt: skip
+        return self.result()
 
 
 def check_all(got_len, got_dir, ref, len_norm, invert, dir_norm, rotated, msg, dir_defined=None):
@@ -454,7 +456,7 @@ def test_million_edges_fold_many_block_partials(ops):
 # ------------------------------------------------------------------------------------------------
 # NaN, std == 0, max == min
 # ------------------------------------------------------------------------------------------------
-def test_nan_length_propagates_through_every_norm(ops, golden):
+def test_nan_length_propagates_through_every_norm_and_shard(ops, golden):
     """An antipodal pair's NaN length makes every normalised length NaN, as numpy's sum / amax / amin / std do in
     the reference - for the golden vectors (row 9) and for a random set with a few such pairs, in every path."""
     g = golden("attr_vectors")
@@ -475,7 +477,7 @@ def test_nan_length_propagates_through_every_norm(ops, golden):
                 ln, _ = Call(ops, s, t, ei, off=off).one(norm, True, None, True)
                 assert_len(ln, ref.length(norm, True), norm, f"{name} inverted off={off}", invert=True)
             if norm is not None:
-                ln, _, _, _ = Call(ops, s, t, ei, off=1).sharded([0, 1, e // 2, e], norm, False, "l1", True, 1)
+                ln, _, _, _ = Call(ops, s, t, ei, off=1).sharded([0, 1, e // 2, e], norm, False, "l1", True)
                 assert np.isnan(ln).all(), f"{name} {norm}: sharded"
 
 
@@ -544,9 +546,9 @@ def shard_bounds(e: int, w: int, rng) -> list[int]:
 
 
 @pytest.mark.parametrize("w", [2, 3, 7, "E+1"])
-def test_sharded_statistics_fold(ops, adversarial, w):
-    """Blocks at odd column boundaries, empty ones included ({0, 0, 1e300, -1e300}); every norm, raw values kept
-    (raw_present = 1) and re-evaluated (raw_present = 0, the statistics-only pass).  Equal to the one-call result -
+def test_sharded_statistics_fold_and_unnormalised_blocks(ops, adversarial, w):
+    """Blocks at odd column boundaries, empty ones included ({0, 0, 1e300, -1e300}); every norm through
+    statistics -> apply, and the un-normalised blocks in one agx_edge_attrs call each.  Equal to the one-call result -
     bit for bit where no sum enters the parameters - and to the reference."""
     sx, tx, ei = adversarial
     if w == "E+1":
@@ -566,19 +568,25 @@ def test_sharded_statistics_fold(ops, adversarial, w):
     for norm in norms:
         for inv, rot in ((False, True), (True, False)):
             one = call.one(norm, inv, norm, rot)
-            for raw_present in (1, 0):
-                ln, dr, st, b = call.sharded(bounds, norm, inv, norm, rot, raw_present)
-                msg = f"W={w} {norm} inv={inv} rot={rot} raw_present={raw_present}"
-                close_or_bits(ln, one[0], norm, msg)
-                close_or_bits(dr, one[1], norm, msg)
-                check_all(ln, dr, ref, norm, inv, norm, rot, msg)
-                empty = [r for r in range(len(b) - 1) if b[r] == b[r + 1]]
-                assert empty or w == 2
-                for r in empty:
-                    np.testing.assert_array_equal(st[r], NO_VALUE * 2)
-                np.testing.assert_allclose(st[:, [0, 1, 4, 5]].sum(0), whole[rot][[0, 1, 4, 5]], rtol=1e-12, err_msg=msg)
-                np.testing.assert_array_equal(st[:, [2, 6]].min(0), whole[rot][[2, 6]], err_msg=msg)
-                np.testing.assert_array_equal(st[:, [3, 7]].max(0), whole[rot][[3, 7]], err_msg=msg)
+            ln, dr, st, b = call.sharded(bounds, norm, inv, norm, rot)
+            msg = f"W={w} {norm} inv={inv} rot={rot}"
+            close_or_bits(ln, one[0], norm, msg)
+            close_or_bits(dr, one[1], norm, msg)
+            check_all(ln, dr, ref, norm, inv, norm, rot, msg)
+            empty = [r for r in range(len(b) - 1) if b[r] == b[r + 1]]
+            assert empty or w == 2
+            for r in empty:
+                np.testing.assert_array_equal(st[r], NO_VALUE * 2)
+            np.testing.assert_allclose(st[:, [0, 1, 4, 5]].sum(0), whole[rot][[0, 1, 4, 5]], rtol=1e-12, err_msg=msg)
+            np.testing.assert_array_equal(st[:, [2, 6]].min(0), whole[rot][[2, 6]], err_msg=msg)
+            np.testing.assert_array_equal(st[:, [3, 7]].max(0), whole[rot][[3, 7]], err_msg=msg)
+    for inv, rot in ((False, True), (True, False)):
+        ln, dr = call.blocks(bounds, inv, rot)
+        one = call.one(None, inv, None, rot)
+        msg = f"W={w} un-normalised blocks inv={inv} rot={rot}"
+        bits_equal(ln, one[0], msg)
+        bits_equal(dr, one[1], msg)
+        check_all(ln, dr, ref, None, inv, None, rot, msg)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -590,7 +598,7 @@ def _flag_lists(n_t: int, rng) -> dict:
 
 
 @pytest.mark.parametrize("k", [3, 7])
-def test_flag_modes_and_list_pass(ops, lib, k):
+def test_flag_modes_and_target_list_of_one_stats_entry_point(ops, lib, k):
     """"skip" with regular_k, then the list pass (lists of 0, 1 = the last target, every target, some) with a flag
     pointer offset as in a sharded decoder; also "only" without a list.  The two statistics sets add up to the whole
     set's, and apply(n_stat_sets = 2) equals the one-call result and the reference."""
@@ -616,20 +624,20 @@ def test_flag_modes_and_list_pass(ops, lib, k):
             for norm, inv, rot in ((n, i, r) for n, i, r in CONFIGS if i == (n in ("l1", "unit-range"))):
                 st = torch.tensor([NO_VALUE * 2] * 2, dtype=torch.float64, device="cuda")
                 call.outputs()
-                _check(lib.agx_edge_attrs_stats_flagged(
+                _check(lib.agx_edge_attrs_stats(
                     call.col(0), call.col(1), e, *call.nodes, 1, 1, int(rot), call.len_ptr(), call.dir_ptr(),
-                    st[0].data_ptr(), ws, flags.data_ptr() - base, 1, k, _stream()))  # fmt: skip
+                    st[0].data_ptr(), ws, flags.data_ptr() - base, 1, None, None, k, _stream()))  # fmt: skip
                 fe = torch.from_numpy(flagged_edges).cuda()
                 call.out_len[fe] = float("nan")  # what the second pass must overwrite
                 call.out_dir[fe] = float("nan")
                 if mode == "list":
-                    _check(lib.agx_edge_attrs_stats_list(
-                        call.col(0), call.col(1), e, k, f_list.data_ptr(), f_count.data_ptr(), *call.nodes, 1, 1,
-                        int(rot), call.len_ptr(), call.dir_ptr(), st[1].data_ptr(), ws, _stream()))  # fmt: skip
-                else:
-                    _check(lib.agx_edge_attrs_stats_flagged(
+                    _check(lib.agx_edge_attrs_stats(
                         call.col(0), call.col(1), e, *call.nodes, 1, 1, int(rot), call.len_ptr(), call.dir_ptr(),
-                        st[1].data_ptr(), ws, flags.data_ptr() - base, 2, k if mode == "only_k" else 0,
+                        st[1].data_ptr(), ws, None, 2, f_list.data_ptr(), f_count.data_ptr(), k, _stream()))  # fmt: skip
+                else:
+                    _check(lib.agx_edge_attrs_stats(
+                        call.col(0), call.col(1), e, *call.nodes, 1, 1, int(rot), call.len_ptr(), call.dir_ptr(),
+                        st[1].data_ptr(), ws, flags.data_ptr() - base, 2, None, None, k if mode == "only_k" else 0,
                         _stream()))  # fmt: skip
                 s = st.cpu().numpy()
                 w = whole_rot if rot else whole_norot
@@ -639,7 +647,7 @@ def test_flag_modes_and_list_pass(ops, lib, k):
                 np.testing.assert_array_equal(np.maximum(s[0, [3, 7]], s[1, [3, 7]]), w[[3, 7]], err_msg=msg)
                 if listed.size == 0:
                     np.testing.assert_array_equal(s[1], NO_VALUE * 2)
-                call.apply(0, e, norm, inv, norm, rot, st, 2, 1)
+                call.apply(0, e, norm, inv, norm, rot, st, 2)
                 ln, dr = call.result()
                 one = call.one(norm, inv, norm, rot, regular_k=k)
                 close_or_bits(ln, one[0], norm, msg)
@@ -662,50 +670,9 @@ def test_flag_modes_and_list_pass(ops, lib, k):
 
 
 # ------------------------------------------------------------------------------------------------
-# AGX_ATTR_RECOMPUTE=1 (the setting is read once per process: a child process)
-# ------------------------------------------------------------------------------------------------
-_CHILD = """
-import sys
-import numpy as np, torch
-sys.path.insert(0, {repo!r})
-from anemoi_graphs_b200 import ops
-d = np.load({inp!r})
-ei = torch.from_numpy(d["ei"]).cuda()
-src, dst = ops.NodeTables(torch.from_numpy(d["sx"]).cuda()), ops.NodeTables(torch.from_numpy(d["tx"]).cuda())
-out = {{}}
-for i, (norm, inv, rot) in enumerate({configs!r}):
-    ln, dr = ops.edge_attributes(ei, src, dst, length_norm=norm, length_invert=inv, direction_norm=norm,
-                                 direction_rotated=rot)
-    out[f"len{{i}}"], out[f"dir{{i}}"] = ln.cpu().numpy(), dr.cpu().numpy()
-np.savez({out!r}, **out)
-"""
-
-
-def test_recompute_mode_is_bit_identical(ops, adversarial, tmp_path):
-    sx, tx, ei = adversarial
-    ei = np.ascontiguousarray(ei[:, :-1])  # an odd count: the scalar lanes
-    inp, out = tmp_path / "in.npz", tmp_path / "out.npz"
-    np.savez(inp, sx=sx, tx=tx, ei=ei)
-    code = _CHILD.format(repo=str(REPO), inp=str(inp), out=str(out), configs=CONFIGS)
-    env = dict(os.environ, AGX_ATTR_RECOMPUTE="1")
-    run = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert run.returncode == 0, run.stderr[-3000:]
-    got = np.load(out)
-    e = dev(ei)
-    src, dst = ops.NodeTables(dev(sx)), ops.NodeTables(dev(tx))
-    ref = Ref(sx, tx, ei)
-    for i, (norm, inv, rot) in enumerate(CONFIGS):
-        ln, dr = ops.edge_attributes(e, src, dst, length_norm=norm, length_invert=inv, direction_norm=norm,
-                                     direction_rotated=rot)  # fmt: skip
-        bits_equal(got[f"len{i}"], ln.cpu().numpy(), f"recompute {norm} inv={inv} rot={rot}")
-        bits_equal(got[f"dir{i}"], dr.cpu().numpy(), f"recompute {norm} inv={inv} rot={rot}")
-        check_all(got[f"len{i}"], got[f"dir{i}"], ref, norm, inv, norm, rot, "recompute")
-
-
-# ------------------------------------------------------------------------------------------------
 # argument checks
 # ------------------------------------------------------------------------------------------------
-def test_out_dir_must_be_8_byte_aligned(ops, lib, adversarial):
+def test_out_dir_must_be_8_byte_aligned_in_every_work_set(ops, lib, adversarial):
     """A direction output 4 bytes off an 8-byte boundary is refused by every entry point before any device work
     (the kernels store each direction as one float2)."""
     from anemoi_graphs_b200._cabi import AGX_ERR_ARG
@@ -724,17 +691,16 @@ def test_out_dir_must_be_8_byte_aligned(ops, lib, adversarial):
     rcs = {
         "agx_edge_attrs": lib.agx_edge_attrs(a, b, e, *call.nodes, 3, 0, call.len_ptr(), 3, 1, bad, ws, 0, s),
         "agx_edge_attrs regular": lib.agx_edge_attrs(a, b, e, *call.nodes, 0, 0, call.len_ptr(), 0, 1, bad, ws, 1, s),
-        "agx_edge_attrs_stats": lib.agx_edge_attrs_stats(a, b, e, *call.nodes, 1, 1, 1, call.len_ptr(), bad,
-                                                         st[0].data_ptr(), ws, s),
-        "agx_edge_attrs_stats_flagged": lib.agx_edge_attrs_stats_flagged(
-            a, b, e, *call.nodes, 1, 1, 1, call.len_ptr(), bad, st[0].data_ptr(), ws, flags.data_ptr(), 2, 0, s),
-        "agx_edge_attrs_stats_list": lib.agx_edge_attrs_stats_list(
-            a, b, e, 1, f_list.data_ptr(), f_count.data_ptr(), *call.nodes, 1, 1, 1, call.len_ptr(), bad,
-            st[1].data_ptr(), ws, s),
-        "agx_edge_attrs_apply raw": lib.agx_edge_attrs_apply(a, b, e, *call.nodes, 3, 0, call.len_ptr(), 3, 1, bad,
-                                                             st.data_ptr(), 2, e, 0, ws, s),
-        "agx_edge_attrs_apply in place": lib.agx_edge_attrs_apply(a, b, e, *call.nodes, 3, 0, call.len_ptr(), 3, 1,
-                                                                  bad, st.data_ptr(), 2, e, 1, ws, s),
+        "agx_edge_attrs_stats all": lib.agx_edge_attrs_stats(
+            a, b, e, *call.nodes, 1, 1, 1, call.len_ptr(), bad, st[0].data_ptr(), ws, None, 0, None, None, 0, s),
+        "agx_edge_attrs_stats skip": lib.agx_edge_attrs_stats(
+            a, b, e, *call.nodes, 1, 1, 1, call.len_ptr(), bad, st[0].data_ptr(), ws, flags.data_ptr(), 1, None, None, 0, s),
+        "agx_edge_attrs_stats only": lib.agx_edge_attrs_stats(
+            a, b, e, *call.nodes, 1, 1, 1, call.len_ptr(), bad, st[0].data_ptr(), ws, flags.data_ptr(), 2, None, None, 0, s),
+        "agx_edge_attrs_stats list": lib.agx_edge_attrs_stats(
+            a, b, e, *call.nodes, 1, 1, 1, call.len_ptr(), bad, st[1].data_ptr(), ws, None, 2, f_list.data_ptr(),
+            f_count.data_ptr(), 1, s),
+        "agx_edge_attrs_apply": lib.agx_edge_attrs_apply(e, 3, 0, call.len_ptr(), 3, 1, bad, st.data_ptr(), 2, e, ws, s),
     }  # fmt: skip
     assert rcs == {name: AGX_ERR_ARG for name in rcs}
     torch.cuda.synchronize()

@@ -525,8 +525,8 @@ def _prov_coords(hx: np.ndarray, perm: np.ndarray) -> np.ndarray:
     return hx[perm]
 
 
-def test_attribute_flag_modes_split_the_statistics(ops, golden):
-    """``agx_edge_attrs_stats_flagged``: "skip" + "only" partition the statistics of an edge set by target flag, and
+def test_attribute_flag_modes_of_the_stats_entry_point_split_the_statistics(ops, golden):
+    """``agx_edge_attrs_stats`` flag modes: "skip" + "only" partition the statistics of an edge set by target flag, and
     the deferred three-step evaluation (raw / patch / apply) equals the one-call result."""
     g = golden("toy")
     dx, hx = g["data_x"], g["hidden_x"]
@@ -549,7 +549,8 @@ def test_attribute_flag_modes_split_the_statistics(ops, golden):
         check = __import__("anemoi_graphs_b200._cabi", fromlist=["check"]).check
         check(ops.load_library().agx_edge_attrs_stats(ei[0].data_ptr(), ei[1].data_ptr(), int(ei.shape[1]), src.src_rec.data_ptr(),
               None, dst.dst_rec.data_ptr(), None, 1, 1, 1, raw_len.data_ptr(), raw_dir.data_ptr(), whole.data_ptr(),
-              ops._attr_workspace(ei.device).data_ptr(), torch.cuda.current_stream().cuda_stream))  # fmt: skip
+              ops._attr_workspace(ei.device).data_ptr(), None, 0, None, None, 0,
+              torch.cuda.current_stream().cuda_stream))  # fmt: skip
         st = job.stats.cpu().numpy()
         w = whole.cpu().numpy()
         np.testing.assert_allclose(st[0, [0, 1, 4, 5]] + st[1, [0, 1, 4, 5]], w[[0, 1, 4, 5]], rtol=1e-12)
