@@ -80,14 +80,32 @@ class GraphCreator:
         walk(self.config.get("nodes", {}))
         walk(self.config.get("edges", []))
         walk(self.config.get("post_processors", []))
+        from .edges.builder import check_scale_levels
+        from .edges.builder import scale_levels
+
         for edges_cfg in self.config.get("edges", []):
             for b in edges_cfg.get("edge_builders", []):
                 target = str(b.get("_target_", ""))
+                name = target.rsplit(".", 1)[-1]
                 k, hops = b.get("num_nearest_neighbours"), b.get("x_hops")
-                if target.endswith(".KNNEdges") and isinstance(k, int) and k > self.MAX_KNN_K:
-                    raise NotImplementedError(f"KNNEdges: num_nearest_neighbours = {k} > {self.MAX_KNN_K} is not built")
-                if target.endswith(".MultiScaleEdges") and isinstance(hops, int) and hops > self.MAX_X_HOPS:
+                if name in ("KNNEdges", "ReversedKNNEdges") and isinstance(k, int) and k > self.MAX_KNN_K:
+                    raise NotImplementedError(f"{name}: num_nearest_neighbours = {k} > {self.MAX_KNN_K} is not built")
+                if name == "MultiScaleEdges" and isinstance(hops, int) and hops > self.MAX_X_HOPS:
                     raise NotImplementedError(f"MultiScaleEdges: x_hops = {hops} > {self.MAX_X_HOPS} is not built")
+                if name == "MultiScaleEdges" and b.get("scale_resolutions") is not None:
+                    levels = scale_levels(b.get("scale_resolutions"))
+                    check_scale_levels(levels, self._finest_level(edges_cfg.get("source_name")))
+
+    def _finest_level(self, nodes_name) -> int | None:
+        """The finest refinement level of a node set the recipe builds (``resolution`` / ``lam_resolution`` of its node
+        builder), or None when the recipe does not say."""
+        node_builder = self.config.get("nodes", {}).get(nodes_name, {}).get("node_builder", {})
+        res = node_builder.get("lam_resolution", node_builder.get("resolution"))
+        if isinstance(res, int) and not isinstance(res, bool):
+            return res
+        if isinstance(res, (list, tuple)) and res and all(isinstance(r, int) for r in res):
+            return max(res)
+        return None
 
     def update_graph(self, graph):
         """Instantiate the node and edge builders of the recipe and apply them to the graph (create.py:62-92)."""

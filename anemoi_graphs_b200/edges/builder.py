@@ -171,6 +171,14 @@ class NodeMaskingMixin:
     remap) is applied by the search kernels as they write (``masked_outputs``), so no pass over the edge list follows.
     ``undo_masking`` itself remains for callers that hold compact indices."""
 
+    # A reversed builder searches the other way round: the TARGETS are indexed and every source node is a query.  Its
+    # searches write the query side to row 0 (``swap_rows``), so the edge list still reads (source, target).
+    _reversed = False
+
+    def search_roles(self, of_source, of_target) -> tuple:
+        """``(indexed side, query side)`` of a (source, target) pair - and, applied to that, the (source, target) pair."""
+        return (of_target, of_source) if self._reversed else (of_source, of_target)
+
     @staticmethod
     def _selection(nodes, mask_attr_name: str | None, device) -> torch.Tensor | None:
         if mask_attr_name is None:
@@ -188,7 +196,7 @@ class NodeMaskingMixin:
         src_st = _device.node_state(source_nodes, provisional_ok=ok and self.provisional_source_ok)
         dst_st = _device.node_state(target_nodes, provisional_ok=ok and self.provisional_target_ok)
         self._row_provs = (src_st.prov, dst_st.prov)  # rows of the result that will be in provisional numbering
-        self._src_state = src_st  # its neighbour index is shared between the builders of a recipe (unmasked, small sets)
+        self._node_states = (src_st, dst_st)  # the indexed side's index is shared between the builders of a recipe
         src, dst = src_st.x, dst_st.x
         src_sel = self._selection(source_nodes, self.source_mask_attr_name, src.device)
         dst_sel = self._selection(target_nodes, self.target_mask_attr_name, dst.device)
@@ -199,10 +207,10 @@ class NodeMaskingMixin:
         return src, dst, src_sel, dst_sel
 
     @staticmethod
-    def masked_outputs(src_sel, dst_sel, lo: int, hi: int):
-        """``with self.masked_outputs(src_sel, dst_sel, lo, hi):`` - searches over the query rows [lo, hi) of the masked
+    def masked_outputs(ref_sel, query_sel, lo: int, hi: int):
+        """``with self.masked_outputs(ref_sel, query_sel, lo, hi):`` - searches over the query rows [lo, hi) of the masked
         coordinates write ORIGINAL node indices (``undo_masking`` fused into the kernels' stores, ``ops.output_maps``)."""
-        return ops.output_maps(src_sel, None if dst_sel is None else dst_sel[lo:hi].contiguous())
+        return ops.output_maps(ref_sel, None if query_sel is None else query_sel[lo:hi].contiguous())
 
     @staticmethod
     def undo_masking(edge_index: torch.Tensor, src_sel, dst_sel) -> torch.Tensor:
@@ -256,17 +264,19 @@ class KNNEdges(BaseEdgeBuilder, NodeMaskingMixin):
         self.num_nearest_neighbours = num_nearest_neighbours
         self.stats = None  # optional CUDA int64[4]: {float64-refined, tied at the k-th boundary, widened, 0}
 
-    # Ties at the k-th boundary go to the lower SOURCE index, so the result depends on the final numbering of the
-    # sources - but only for the queries that have such a tie.  With provisionally numbered sources the search runs
-    # at once, flags those queries (agx_knn_flagged), and re-decides exactly them when the order is known
-    # (``_redecide_ties``); everything else is a relabel.
+    # Ties at the k-th boundary go to the lower index of the indexed side (the SOURCES; the targets for
+    # ReversedKNNEdges), so the result depends on the final numbering of that side - but only for the queries that have
+    # such a tie.  With a provisionally numbered indexed side the search runs at once, flags those queries
+    # (agx_knn_flagged), and re-decides exactly them when the order is known (``_redecide_ties``); everything else is a
+    # relabel.
     provisional_source_ok = True
 
     @staticmethod
-    def _redecide_ties(prov, index, out: torch.Tensor, tie_list, queries: torch.Tensor, k: int) -> None:
+    def _redecide_ties(prov, index, out: torch.Tensor, tie_list, queries: torch.Tensor, k: int, swap_rows: bool) -> None:
         """Runs inside ``Provisional.resolve`` before the rows are relabelled: ``index`` is the one the search used
         (provisional labels); ties go to the lower FINAL label ``prov.rank[label]``, provisional labels are written."""
-        index.knn_redecide_list(queries, k, out, tie_list[0], tie_list[1], rank=prov.rank, order=prov.order_dev)
+        index.knn_redecide_list(queries, k, out, tie_list[0], tie_list[1], rank=prov.rank, order=prov.order_dev,
+                                swap_rows=swap_rows)  # fmt: skip
         meta = _device.edge_meta(out)
         if meta is not None:
             meta.fixup = None
@@ -274,54 +284,65 @@ class KNNEdges(BaseEdgeBuilder, NodeMaskingMixin):
     def compute_edge_index(self, source_nodes, target_nodes) -> torch.Tensor:
         src, dst, src_sel, dst_sel = self.get_node_coordinates(source_nodes, target_nodes)
         assert self.num_nearest_neighbours is not None, "number of neighbors required for knn encoder"
+        rev = self._reversed
         LOGGER.info(
-            "Using KNN-Edges (with %d nearest neighbours) between %s and %s.",
+            "Using %sKNN-Edges (with %d nearest neighbours) between %s and %s.",
+            "Reversed-" if rev else "",
             self.num_nearest_neighbours,
             self.source_name,
             self.target_name,
         )
         k = self.num_nearest_neighbours
-        nq = int(dst.shape[0])
+        ref, qry = self.search_roles(src, dst)
+        ref_sel, qry_sel = self.search_roles(src_sel, dst_sel)
+        ref_state = self.search_roles(*self._node_states)[0]
+        nq = int(qry.shape[0])
         # sharded output mode: this rank's queries only and nothing to exchange, so sharding always pays; otherwise
         # every rank needs the complete list and small searches are replicated (``shard_world``)
         sharded_out = _device.sharded_output()
         rank, w = _device.world() if sharded_out else _device.shard_world(nq)
-        src_prov, dst_prov = self._row_provs
-        if src_prov is not None and ((w > 1 and not sharded_out) or dst_prov is not None):
-            # flag-and-redecide is built for final target numbering and rank-local results: order first
-            src = _device.node_state(source_nodes).x
-            dst = _device.node_state(target_nodes).x
+        ref_prov, qry_prov = self.search_roles(*self._row_provs)
+        if ref_prov is not None and ((w > 1 and not sharded_out) or qry_prov is not None):
+            # flag-and-redecide is built for final query numbering and rank-local results: order first
+            ref, qry = self.search_roles(_device.node_state(source_nodes).x, _device.node_state(target_nodes).x)
             self._row_provs = (None, None)
-            src_prov = dst_prov = None
+            ref_prov = qry_prov = None
         lo, hi = _device.shard_range(nq, rank, w)
         shard = None
         if sharded_out:
             shard = _device.Shard(rank, w, [(b - a) * k for a, b in (_device.shard_range(nq, r, w) for r in range(w))])
-        if src_prov is not None:
-            q = dst[lo:hi]  # all queries on one rank
-            flags = torch.zeros(hi - lo, dtype=torch.uint8, device=dst.device)
-            with _device.neighbour_index(self._src_state, src, hint_k=k) as index:
-                out = index.knn(q, k, dst_base=lo, stats=self.stats, tie_flags=flags)
-            out = _device.tag_rows(out, src_prov, None)
+        if ref_prov is not None:
+            q = qry[lo:hi]  # all queries on one rank
+            flags = torch.zeros(hi - lo, dtype=torch.uint8, device=qry.device)
+            with _device.neighbour_index(ref_state, ref, hint_k=k) as index:
+                out = index.knn(q, k, dst_base=lo, stats=self.stats, tie_flags=flags, swap_rows=rev)
+            out = _device.tag_rows(out, *self.search_roles(ref_prov, None))
             meta = _device.edge_meta(out, create=True)
             tie_list = ops.compact_flags(flags)  # ascending ids of the tied queries, count on the device: no read-back
-            meta.fixup, meta.tie_flags, meta.tie_list, meta.regular_k, meta.shard = src_prov, flags, tie_list, k, shard
-            meta.flag_base = lo  # ``flags`` is indexed by target id - lo
-            meta.regular_targets = not sharded_out and (lo, hi) == (0, nq)  # unmasked by construction (provisional source)
+            meta.fixup, meta.shard = ref_prov, shard
+            if not rev:
+                # the attribute kernel evaluates the un-flagged targets' edges before the re-decision; its flag modes
+                # are keyed by row-1 targets, so a reversed list (flagged SOURCES) leaves them unset: its attributes
+                # are evaluated on the final edges
+                meta.tie_flags, meta.tie_list, meta.regular_k = flags, tie_list, k
+                meta.flag_base = lo  # ``flags`` is indexed by target id - lo
+                meta.regular_targets = not sharded_out and (lo, hi) == (0, nq)  # unmasked by construction
             # ``index`` stays alive in the closure: the re-decision searches it again, no second index
-            src_prov.add_fixup(lambda prov, index=index, out=out, tl=tie_list, q=q, k=k: self._redecide_ties(prov, index, out, tl, q, k))  # fmt: skip
+            ref_prov.add_fixup(lambda prov, index=index, out=out, tl=tie_list, q=q, k=k: self._redecide_ties(prov, index, out, tl, q, k, rev))  # fmt: skip
             return out
         if sharded_out:
-            # rank-local block, global target ids; no exchange
-            with _device.neighbour_index(self._src_state if src_sel is None else None, src, hint_k=k) as index:
-                with self.masked_outputs(src_sel, dst_sel, lo, hi):
-                    out = index.knn(dst[lo:hi], k, dst_base=lo, stats=self.stats)
+            # rank-local block, global query ids; no exchange
+            with _device.neighbour_index(ref_state if ref_sel is None else None, ref, hint_k=k) as index:
+                with self.masked_outputs(ref_sel, qry_sel, lo, hi):
+                    out = index.knn(qry[lo:hi], k, dst_base=lo, stats=self.stats, swap_rows=rev)
             out = _device.tag_rows(out, *self._row_provs)
             meta = _device.edge_meta(out, create=True)
-            meta.shard, meta.regular_k = shard, k
+            meta.shard = shard
+            if not rev:
+                meta.regular_k = k
             return out
-        with _device.neighbour_index(self._src_state if src_sel is None else None, src, hint_k=k) as index:
-            out = torch.empty((2, nq * k), dtype=torch.int32, device=dst.device)
+        with _device.neighbour_index(ref_state if ref_sel is None else None, ref, hint_k=k) as index:
+            out = torch.empty((2, nq * k), dtype=torch.int32, device=qry.device)
             masked = src_sel is not None or dst_sel is not None
             if w > 1 and not masked and _device.VMM_PUSH:
                 # opt-in: chunks pushed into peer-mapped staging buffers by the copy engines while the next chunk is
@@ -333,7 +354,7 @@ class KNNEdges(BaseEdgeBuilder, NodeMaskingMixin):
                 try:
                     for c, (a, b) in enumerate(ranges[rank]):
                         if b > a:
-                            index.knn(dst[a:b], k, dst_base=a, stats=self.stats, out=out, out_offset=a * k)
+                            index.knn(qry[a:b], k, dst_base=a, stats=self.stats, out=out, out_offset=a * k, swap_rows=rev)
                             if c == 0:  # the first chunk decided the query order (one sync): pin it for the rest
                                 lib.agx_set_query_order_mode(lib.agx_last_query_order())
                         marks.append(gather.mark())
@@ -348,17 +369,44 @@ class KNNEdges(BaseEdgeBuilder, NodeMaskingMixin):
                 # equal blocks: one in-place NCCL all-gather after the search (640 GB/s per rank; chunking the search
                 # to overlap an NCCL exchange was measured and does not pay: the persistent search kernel leaves no
                 # room for the collective's CTAs until it ends - 40 M queries, N = 2: 4.8 ms chunked against 4.5 ms)
-                with self.masked_outputs(src_sel, dst_sel, lo, hi):  # original node indices straight from the kernel
-                    index.knn(dst[lo:hi], k, dst_base=lo, stats=self.stats, out=out, out_offset=lo * k)
+                with self.masked_outputs(ref_sel, qry_sel, lo, hi):  # original node indices straight from the kernel
+                    index.knn(qry[lo:hi], k, dst_base=lo, stats=self.stats, out=out, out_offset=lo * k, swap_rows=rev)
         if w > 1:
             counts = [(b - a) * k for a, b in (_device.shard_range(nq, r, w) for r in range(w))]
             out = _gather_blocks(out, counts, rank, src_sel is not None or dst_sel is not None)
         local = _device.edge_meta(out).local if _device.edge_meta(out) is not None else None
         out = _device.tag_rows(out, *self._row_provs)
         meta = _device.edge_meta(out, create=True)
-        meta.regular_k, meta.local = k, local  # k edges per target, target after target: attributes walk it by target
-        meta.regular_targets = src_sel is None and dst_sel is None  # complete list, row 1 = column // k
+        meta.local = local
+        if not rev:
+            meta.regular_k = k  # k edges per target, target after target: attributes walk it by target
+            meta.regular_targets = src_sel is None and dst_sel is None  # complete list, row 1 = column // k
         return out
+
+
+class ReversedKNNEdges(KNNEdges):
+    """KNN edges in the other direction: for every (masked) source node, its k nearest (masked) target nodes.
+
+    The same edges as ``KNNEdges(target_name, source_name, ...)`` with its two rows swapped (and the masks swapped with
+    them), column for column: the targets are indexed and the sources are the queries, grouped by source, k columns per
+    source.  Exact float64 distance ties at the k-th boundary go to the lower TARGET index.  The class of newer
+    anemoi-graphs releases; parity with them is unverified (the pinned reference has no such class).
+
+    Attributes
+    ----------
+    source_name : str
+        The name of the source nodes.
+    target_name : str
+        The name of the target nodes.
+    num_nearest_neighbours : int
+        Number of nearest target nodes of each source node.
+    source_mask_attr_name : str | None
+        The name of the source mask attribute to filter edge connections.
+    target_mask_attr_name : str | None
+        The name of the target mask attribute to filter edge connections.
+    """
+
+    _reversed = True
 
 
 class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
@@ -393,13 +441,14 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
         self.stats = None  # optional CUDA int64[4]: {pairs decided in float64, pairs within 2^-40 of the radius, 0, 0}
 
     def get_cutoff_radius(self, graph, mask_attr: torch.Tensor | None = None) -> float:
-        """Cut-off radius = reference distance of the TARGET nodes x cut-off factor (edges/builder.py:312-334)."""
-        target_nodes = graph[self.target_name]
-        mask = target_nodes[mask_attr] if mask_attr is not None else None
+        """Cut-off radius = reference distance of the query nodes x cut-off factor (edges/builder.py:312-334): the
+        TARGET nodes, the sources for ``ReversedCutOffEdges``."""
+        query_nodes = graph[self.search_roles(self.source_name, self.target_name)[1]]
+        mask = query_nodes[mask_attr] if mask_attr is not None else None
         # the reference distance does not depend on the numbering of the nodes
-        state = _device.node_state(target_nodes, provisional_ok=True)
-        target_grid_reference_distance = get_grid_reference_distance(state.x, mask, state=state)
-        radius = target_grid_reference_distance * self.cutoff_factor
+        state = _device.node_state(query_nodes, provisional_ok=True)
+        query_grid_reference_distance = get_grid_reference_distance(state.x, mask, state=state)
+        radius = query_grid_reference_distance * self.cutoff_factor
         return radius
 
     def prepare_node_data(self, graph):
@@ -409,30 +458,34 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
 
     def compute_edge_index(self, source_nodes, target_nodes) -> torch.Tensor:
         src, dst, src_sel, dst_sel = self.get_node_coordinates(source_nodes, target_nodes)
+        rev = self._reversed
         LOGGER.info(
-            "Using CutOff-Edges (with radius = %.1f km) between %s and %s.",
+            "Using %sCutOff-Edges (with radius = %.1f km) between %s and %s.",
+            "Reversed-" if rev else "",
             self.radius * EARTH_RADIUS,
             self.source_name,
             self.target_name,
         )
-        nq = int(dst.shape[0])
+        ref, qry = self.search_roles(src, dst)
+        ref_sel, qry_sel = self.search_roles(src_sel, dst_sel)
+        nq = int(qry.shape[0])
         sharded_out = _device.sharded_output()
         rank, w = _device.world() if sharded_out else _device.shard_world(nq)
         lo, hi = _device.shard_range(nq, rank, w)
         if sharded_out:
-            # this rank's targets only; the blocks stay where they are (global target ids), only the counts travel
-            with ops.NeighbourIndex(src, hint_radius=self.radius) as index:
-                q = dst[lo:hi]
+            # this rank's queries only; the blocks stay where they are (global query ids), only the counts travel
+            with ops.NeighbourIndex(ref, hint_radius=self.radius) as index:
+                q = qry[lo:hi]
                 offsets, total = index.radius_count(q, self.radius)
-                out = torch.empty((2, total), dtype=torch.int32, device=dst.device)
-                with self.masked_outputs(src_sel, dst_sel, lo, hi):
-                    index.radius_fill(q, self.radius, offsets, total, out, 0, dst_base=lo, stats=self.stats)
-            counts = _device.exchange_counts(total, dst.device)
+                out = torch.empty((2, total), dtype=torch.int32, device=qry.device)
+                with self.masked_outputs(ref_sel, qry_sel, lo, hi):
+                    index.radius_fill(q, self.radius, offsets, total, out, 0, dst_base=lo, stats=self.stats, swap_rows=rev)
+            counts = _device.exchange_counts(total, qry.device)
             out = _device.tag_rows(out, *self._row_provs)
             _device.edge_meta(out, create=True).shard = _device.Shard(rank, w, counts)
             return out
-        with ops.NeighbourIndex(src, hint_radius=self.radius) as index:
-            q = dst[lo:hi]
+        with ops.NeighbourIndex(ref, hint_radius=self.radius) as index:
+            q = qry[lo:hi]
             offsets, total = index.radius_count(q, self.radius)
             masked = src_sel is not None or dst_sel is not None
             if w > 1 and not masked and torch.distributed.get_backend() == "nccl":
@@ -442,9 +495,9 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
                 chunks = _device.query_chunks(0, hi - lo, n_chunks)
                 bounds = offsets[[a for a, _ in chunks] + [hi - lo]].tolist()  # pair offsets at the chunk boundaries
                 mine = [o1 - o0 for o0, o1 in zip(bounds[:-1], bounds[1:])]
-                rows = _device.all_gather_count_rows(mine, dst.device)
+                rows = _device.all_gather_count_rows(mine, qry.device)
                 counts = [sum(r) for r in rows]
-                out = torch.empty((2, sum(counts)), dtype=torch.int32, device=dst.device)
+                out = torch.empty((2, sum(counts)), dtype=torch.int32, device=qry.device)
                 base = sum(counts[:rank])
                 gather = _device.make_gather(out, rows)
                 lib, marks = ops.load_library(), []
@@ -454,7 +507,7 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
                         if mine[c]:
                             # the offsets keep their block-relative values, so the chunk lands at its final columns
                             index.radius_fill(q[a:b], self.radius, offsets[a : b + 1], mine[c], out, base,
-                                              dst_base=lo + a, stats=self.stats)  # fmt: skip
+                                              dst_base=lo + a, stats=self.stats, swap_rows=rev)  # fmt: skip
                         marks.append(gather.mark())
                         if c > 0:
                             gather.chunk_done(c - 1, marks[c - 1])
@@ -465,14 +518,73 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
                 _device.edge_meta(out, create=True).local = (base, base + counts[rank], list(counts))
                 w = 1  # complete on every rank
             else:
-                counts = _device.all_gather_counts(total, dst.device) if w > 1 else [total]
-                out = torch.empty((2, sum(counts)), dtype=torch.int32, device=dst.device)
+                counts = _device.all_gather_counts(total, qry.device) if w > 1 else [total]
+                out = torch.empty((2, sum(counts)), dtype=torch.int32, device=qry.device)
                 base = sum(counts[:rank])
-                with self.masked_outputs(src_sel, dst_sel, lo, hi):  # original node indices straight from the kernel
-                    index.radius_fill(q, self.radius, offsets, total, out, base, dst_base=lo, stats=self.stats)
+                with self.masked_outputs(ref_sel, qry_sel, lo, hi):  # original node indices straight from the kernel
+                    index.radius_fill(q, self.radius, offsets, total, out, base, dst_base=lo, stats=self.stats,
+                                      swap_rows=rev)  # fmt: skip
         if w > 1:
             out = _gather_blocks(out, counts, rank, src_sel is not None or dst_sel is not None)
         return _device.tag_rows(out, *self._row_provs)
+
+
+class ReversedCutOffEdges(CutOffEdges):
+    """Cut-off edges in the other direction: every (masked) (source, target) pair with the target within the cut-off
+    radius of the source, grouped by source.
+
+    The radius is ``cutoff_factor`` x the grid reference distance of the SOURCE nodes (the query side, as the targets
+    are for ``CutOffEdges``), with the same inclusive test, so the edges are those of ``CutOffEdges(target_name,
+    source_name, ...)`` with its two rows swapped, column for column.  The class of newer anemoi-graphs releases;
+    parity with them is unverified (the pinned reference has no such class).
+
+    Attributes
+    ----------
+    source_name : str
+        The name of the source nodes.
+    target_name : str
+        The name of the target nodes.
+    cutoff_factor : float
+        Factor to multiply the grid reference distance of the source nodes to get the cut-off radius.
+    source_mask_attr_name : str | None
+        The name of the source mask attribute to filter edge connections.
+    target_mask_attr_name : str | None
+        The name of the target mask attribute to filter edge connections.
+    """
+
+    _reversed = True
+
+
+MULTISCALE_MAX_LEVELS = 16  # MS_MAX_LEVELS of the multi-scale edge kernel (agx_mesh.cu)
+
+
+def scale_levels(scale_resolutions) -> list[int] | None:
+    """The refinement levels a ``MultiScaleEdges(scale_resolutions=...)`` argument names, ascending and distinct: an int
+    ``n`` names 1..n, a list its own entries, None every level of the node set (returned as None)."""
+    assert not isinstance(scale_resolutions, str), "The scale_resolutions argument is not valid."
+    if scale_resolutions is None:
+        return None
+    if isinstance(scale_resolutions, int) and not isinstance(scale_resolutions, bool):
+        assert scale_resolutions > 0, "The scale_resolutions argument only supports positive integers."
+        return list(range(1, scale_resolutions + 1))
+    assert isinstance(scale_resolutions, (list, tuple)) and len(scale_resolutions) > 0, (
+        "The scale_resolutions argument is not valid."
+    )
+    assert all(isinstance(r, int) and not isinstance(r, bool) and r > 0 for r in scale_resolutions), (
+        "The scale_resolutions argument only supports positive integers."
+    )
+    return sorted(set(scale_resolutions))
+
+
+def check_scale_levels(levels: list[int], finest: int | None) -> None:
+    """Levels the multi-scale edge kernel can build on a node set whose finest level is ``finest`` (None: not known
+    yet); raised before any kernel runs."""
+    if len(levels) > MULTISCALE_MAX_LEVELS:
+        raise NotImplementedError(
+            f"MultiScaleEdges: {len(levels)} scale_resolutions > {MULTISCALE_MAX_LEVELS} levels is not built"
+        )
+    if finest is not None and max(levels) > finest:
+        raise ValueError(f"MultiScaleEdges: scale_resolutions {levels} go past the finest level {finest} of the nodes")
 
 
 class MultiScaleEdges(BaseEdgeBuilder):
@@ -487,25 +599,40 @@ class MultiScaleEdges(BaseEdgeBuilder):
     x_hops : int
         Number of hops (in the refined icosahedron) between two nodes to connect
         them with an edge.
+    scale_resolutions : int | list[int] | None
+        Refinement levels that contribute edges: ``n`` for the levels 1..n, a list for exactly those levels, None
+        (default) for every level of the node set (its ``_resolutions``).  As in newer anemoi-graphs releases, as far
+        as is known (the pinned reference has no such argument).
     """
 
     VALID_NODES = ["TriNodes", "HexNodes", "LimitedAreaTriNodes", "LimitedAreaHexNodes", "StretchedTriNodes"]
 
-    def __init__(self, source_name: str, target_name: str, x_hops: int, **kwargs):
+    def __init__(
+        self, source_name: str, target_name: str, x_hops: int, scale_resolutions: int | list[int] | None = None, **kwargs
+    ):
         super().__init__(source_name, target_name)
         assert source_name == target_name, f"{self.__class__.__name__} requires source and target nodes to be the same."
         assert isinstance(x_hops, int), "Number of x_hops must be an integer"
         assert x_hops > 0, "Number of x_hops must be positive"
         self.x_hops = x_hops
+        self.scale_resolutions = scale_levels(scale_resolutions)
+
+    def levels(self, nodes) -> list[int]:
+        """The refinement levels whose edges are built on ``nodes``."""
+        if self.scale_resolutions is None:
+            return nodes["_resolutions"]
+        check_scale_levels(self.scale_resolutions, max(int(r) for r in nodes["_resolutions"]))
+        return self.scale_resolutions
 
     def compute_edge_index(self, source_nodes, target_nodes) -> torch.Tensor:
         from ..generate import tri_icosahedron
 
         node_type = source_nodes["node_type"]
+        resolutions = self.levels(source_nodes)
         if node_type in ("TriNodes", "LimitedAreaTriNodes"):
             return tri_icosahedron.multiscale_edges(
                 source_nodes,
-                resolutions=source_nodes["_resolutions"],
+                resolutions=resolutions,
                 x_hops=self.x_hops,
                 area_mask_builder=source_nodes.get("_area_mask_builder", None),
                 allow_provisional=self._provisional_ok,
@@ -518,16 +645,16 @@ class MultiScaleEdges(BaseEdgeBuilder):
             all_points_mask_builder.fit_coords(_device.node_state(source_nodes).x)
             return tri_icosahedron.multiscale_edges(
                 source_nodes,
-                resolutions=source_nodes["_resolutions"],
+                resolutions=resolutions,
                 x_hops=self.x_hops,
                 area_mask_builder=all_points_mask_builder,
             )
         if node_type in ("HexNodes", "LimitedAreaHexNodes"):
             from ..generate import hex_icosahedron
 
-            return hex_icosahedron.multiscale_edges(
-                source_nodes, resolutions=source_nodes["_resolutions"], x_hops=self.x_hops
-            )
+            # the graph's nodes are the cells of the node set's finest level, whichever levels contribute edges
+            finest = None if self.scale_resolutions is None else max(int(r) for r in source_nodes["_resolutions"])
+            return hex_icosahedron.multiscale_edges(source_nodes, resolutions=resolutions, x_hops=self.x_hops, finest=finest)
         raise ValueError(f"Invalid node type {node_type}")
 
     def get_edge_index_device(self, graph) -> torch.Tensor:

@@ -68,6 +68,14 @@ def _dev_x(x: torch.Tensor) -> torch.Tensor:
     return x.contiguous()
 
 
+def _row_ptrs(out: torch.Tensor, col: int, swap_rows: bool) -> tuple[int, int]:
+    """Addresses of column ``col`` of the rows the search writes its reference points and its queries to: rows 0 and 1
+    of the (2, E) int32 ``out``, or rows 1 and 0."""
+    row0 = out.data_ptr() + 4 * col
+    row1 = row0 + 4 * out.shape[1]
+    return (row1, row0) if swap_rows else (row0, row1)
+
+
 class NeighbourIndex:
     """Cell-binned reference point set - the stand-in for a fitted ``NearestNeighbors(metric="haversine")``
     (/root/reference/src/anemoi/graphs/edges/builder.py:259-260, 364-365)."""
@@ -122,6 +130,7 @@ class NeighbourIndex:
         tag: str = "knn",
         max_radius: float = 0.0,
         tie_flags: torch.Tensor | None = None,
+        swap_rows: bool = False,
     ):
         """``edge_index`` (2, nq*k) int32 - row 0 the k nearest reference points of each query, row 1
         ``dst_base + query`` - and optionally the float64 ``rdist`` (nq, k).  With ``out`` (a larger
@@ -130,7 +139,8 @@ class NeighbourIndex:
         0 = unlimited) bounds the search: exact for queries whose k-th neighbour is within it; any other query gets
         every point within it, and -1 / +inf or points beyond it in the other slots (``agx_b200.h``).  ``tie_flags``
         (zeroed uint8 (nq,)) marks the queries whose result depends on the numbering of the reference points
-        (``agx_knn_flagged``)."""
+        (``agx_knn_flagged``).  ``swap_rows``: the kernel writes the queries to row 0 and the reference points to row 1
+        (reversed edge builders: the queries are the sources)."""
         q = _dev_x(q)
         nq = int(q.shape[0])
         if out is None:
@@ -139,13 +149,12 @@ class NeighbourIndex:
         assert out.dim() == 2 and out.shape[0] == 2 and out.dtype == torch.int32 and out.is_contiguous()
         assert 0 <= out_offset and out_offset + nq * k <= out.shape[1]
         rdist = torch.empty((nq, k), dtype=torch.float64, device=q.device) if return_rdist else None
-        row = out.shape[1] * 4
+        ref_row, q_row = _row_ptrs(out, out_offset, swap_rows)
         with _span(tag, nq * k):
             check(
                 self.lib.agx_knn_flagged(
-                    self.handle, ptr(q), nq, int(k), float(max_radius), out.data_ptr() + 4 * out_offset,
-                    out.data_ptr() + row + 4 * out_offset, int(dst_base), ptr(rdist), ptr(stats), ptr(tie_flags),
-                    current_stream(),
+                    self.handle, ptr(q), nq, int(k), float(max_radius), ref_row, q_row, int(dst_base), ptr(rdist),
+                    ptr(stats), ptr(tie_flags), current_stream(),
                 )
             )  # fmt: skip
         return (out, rdist) if return_rdist else out
@@ -177,10 +186,11 @@ class NeighbourIndex:
 
     def knn_redecide_list(
         self, q: torch.Tensor, k: int, out: torch.Tensor, flag_list: torch.Tensor, flag_count: torch.Tensor,
-        rank: torch.Tensor | None = None, order: torch.Tensor | None = None,
+        rank: torch.Tensor | None = None, order: torch.Tensor | None = None, swap_rows: bool = False,
     ) -> None:  # fmt: skip
         """``knn_redecide`` driven by the ascending list of flagged query ids (``compact_flags``): one thread per
-        listed query (``agx_knn_redecide_list``)."""
+        listed query (``agx_knn_redecide_list``).  ``swap_rows``: ``out`` came from ``knn(..., swap_rows=True)``, its
+        reference points are row 1."""
         q = _dev_x(q)
         nq = int(q.shape[0])
         assert out.shape == (2, nq * k) and out.dtype == torch.int32 and out.is_contiguous()
@@ -188,10 +198,10 @@ class NeighbourIndex:
         with _span("knn_ties", nq):
             check(
                 self.lib.agx_knn_redecide_list(
-                    self.handle, ptr(q), nq, int(k), 0.0, out.data_ptr(), ptr(flag_list), ptr(flag_count), ptr(rank),
-                    ptr(order), current_stream(),
+                    self.handle, ptr(q), nq, int(k), 0.0, _row_ptrs(out, 0, swap_rows)[0], ptr(flag_list),
+                    ptr(flag_count), ptr(rank), ptr(order), current_stream(),
                 )
-            )
+            )  # fmt: skip
 
     def radius_count(self, q: torch.Tensor, radius: float) -> tuple[torch.Tensor, int]:
         """Pass 1 of the cut-off search: ``(offsets (nq+1,) int64, total)``."""
@@ -208,20 +218,20 @@ class NeighbourIndex:
 
     def radius_fill(
         self, q: torch.Tensor, radius: float, offsets: torch.Tensor, total: int, out: torch.Tensor, out_offset: int = 0,
-        dst_base: int = 0, stats: torch.Tensor | None = None,
+        dst_base: int = 0, stats: torch.Tensor | None = None, swap_rows: bool = False,
     ) -> torch.Tensor:  # fmt: skip
-        """Pass 2: write the ``total`` pairs at column ``out_offset`` of the contiguous (2, E) int32 ``out``."""
+        """Pass 2: write the ``total`` pairs at column ``out_offset`` of the contiguous (2, E) int32 ``out``; with
+        ``swap_rows`` the queries go to row 0 and the reference points to row 1."""
         q = _dev_x(q)
         assert out.dim() == 2 and out.shape[0] == 2 and out.dtype == torch.int32 and out.is_contiguous()
         assert 0 <= out_offset and out_offset + total <= out.shape[1]
         if total:
-            row = out.shape[1] * 4
+            ref_row, q_row = _row_ptrs(out, out_offset, swap_rows)
             with _span("radius_fill", total):
                 check(
                     self.lib.agx_radius_fill(
-                        self.handle, ptr(q), int(q.shape[0]), float(radius), ptr(offsets),
-                        out.data_ptr() + 4 * out_offset, out.data_ptr() + row + 4 * out_offset, int(dst_base), ptr(stats),
-                        current_stream(),
+                        self.handle, ptr(q), int(q.shape[0]), float(radius), ptr(offsets), ref_row, q_row,
+                        int(dst_base), ptr(stats), current_stream(),
                     )
                 )  # fmt: skip
         return out
