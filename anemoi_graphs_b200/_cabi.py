@@ -120,6 +120,8 @@ SIGNATURES = {
     ),
     "agx_voronoi_areas_small": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_double, c_void_p, c_void_p, c_void_p]),
     "agx_healpix_nodes": (c_int, [c_int, c_void_p, c_void_p]),
+    "agx_gaussian_latitudes": (c_int, [c_int, c_void_p, c_void_p]),
+    "agx_octahedral_nodes": (c_int, [c_int, c_void_p, c_void_p, c_void_p]),
     "agx_hex_num_cells": (c_int64, [c_int]),
     "agx_hex_cells": (c_int, [c_int, c_void_p, c_void_p, c_void_p]),
     "agx_hex_adjacency": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),

@@ -64,7 +64,8 @@ class GraphCreator:
 
     def _validate(self) -> None:
         """Resolve every ``_target_`` of the recipe (an unknown or unbuilt class - the ICON builders,
-        ``PlanarAreaWeights`` - raises ImportError now) and check the limits of the kernels."""
+        ``PlanarAreaWeights`` - raises ImportError now), check the grid names of ``ReducedGaussianGridNodes`` and the
+        limits of the kernels."""
         from .config import resolve_target
 
         def walk(cfg):
@@ -82,7 +83,12 @@ class GraphCreator:
         walk(self.config.get("post_processors", []))
         from .edges.builder import check_scale_levels
         from .edges.builder import scale_levels
+        from .nodes.builders.from_reduced_gaussian import octahedral_number
 
+        for nodes_cfg in self.config.get("nodes", {}).values():
+            node_builder = nodes_cfg.get("node_builder", {})
+            if str(node_builder.get("_target_", "")).rsplit(".", 1)[-1] == "ReducedGaussianGridNodes":
+                octahedral_number(node_builder.get("grid"))
         for edges_cfg in self.config.get("edges", []):
             for b in edges_cfg.get("edge_builders", []):
                 target = str(b.get("_target_", ""))

@@ -408,3 +408,97 @@ extern "C" int agx_healpix_nodes(int order, float* latlon, void* stream_) {
     agx_note_launch(1);
     return AGX_OK;
 }
+
+// ------------------------------------------------------------------------------------------------
+// Octahedral reduced Gaussian grid O<n> (ReducedGaussianGridNodes of newer releases, grids.octahedral_grid): the 2n
+// Gaussian latitudes are the roots of the Legendre polynomial P_2n; row i (1-based from the nearer pole) holds 4i + 16
+// points at longitudes j * 360 / (4i + 16).
+// ------------------------------------------------------------------------------------------------
+namespace {
+constexpr double PIO2_HI = 1.5707963267948966;      // fl(pi / 2)
+constexpr double PIO2_LO = 6.123233995736766e-17;   // pi / 2 - PIO2_HI
+constexpr double RAD2DEG = 180.0 / M_PI_;           // numpy rad2deg
+
+// One thread per northern root k: Newton on f(theta) = P_m(cos theta), m = 2n, from Tricomi's guess
+// theta = pi (k + 3/4) / (m + 1/2) (k counted from 0).  P_m is evaluated through y = 1 - cos theta = 2 sin^2(theta/2) and
+// the differences D_j = P_j - P_{j-1} (j D_j = (j-1) D_{j-1} - (2j-1) y P_{j-1}): near the pole cos theta rounds away
+// most of theta (1 ulp of x is 1e-13 rad at O1280's first row), y keeps it, so the roots are good to 1e-14 degrees at
+// every row.  df/dtheta = m (x P_m - P_{m-1}) / sin theta, with x P_m - P_{m-1} = D_m - y P_m.  The loop stops after a
+// step below 1e-11: Newton's error after it is cot(theta) / 2 * step^2 < 1e-17.
+__global__ void k_gaussian_latitudes(int n, double* __restrict__ lat_deg) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const int m = 2 * n;
+    double theta = M_PI_ * ((double)k + 0.75) / ((double)m + 0.5);
+    for (int it = 0; it < 32; ++it) {
+        const double h = sin(0.5 * theta);
+        const double y = 2.0 * h * h;
+        double p = 1.0 - y, d = -y;  // P_1, D_1
+#pragma unroll 4
+        for (int j = 2; j <= m; ++j) {
+            const double r = __drcp_rn((double)j);
+            d = fma(1.0 - r, d, -((2.0 - r) * y) * p);
+            p += d;
+        }
+        const double step = p * sin(theta) / ((double)m * (d - y * p));
+        theta -= step;
+        if (fabs(step) < 1e-11) break;
+    }
+    const double lat = __dmul_rn(__dadd_rn(__dsub_rn(PIO2_HI, theta), PIO2_LO), RAD2DEG);
+    lat_deg[k] = lat;
+    lat_deg[m - 1 - k] = -lat;
+}
+
+// One point per thread.  q = the position counted from the nearer pole (from the last point in the southern half);
+// row r (0-based from that pole) starts at 2r(r + 9), so r is the largest with (2r + 9)^2 <= 2q + 81: an exact integer
+// square root (the double sqrt of an integer < 2^34, corrected by one either way).  Roundings as the oracle's:
+// lon = j * fl(360 / count), then numpy's deg2rad and one rounding to float32.
+__global__ void k_octahedral_nodes(int n, int64_t half, const double* __restrict__ lat_deg, float2* __restrict__ latlon) {
+    const int64_t total = 2 * half;
+    for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < total; p += (int64_t)gridDim.x * blockDim.x) {
+        const bool south = p >= half;
+        const int64_t q = south ? total - 1 - p : p;
+        const int64_t v = 2 * q + 81;
+        int64_t s = (int64_t)sqrt((double)v);
+        if (s * s > v) --s;
+        if ((s + 1) * (s + 1) <= v) ++s;
+        const int64_t r = (s - 9) >> 1;
+        const int64_t count = 4 * r + 20;
+        int64_t j = q - 2 * r * (r + 9);
+        if (south) j = count - 1 - j;
+        const double lat = lat_deg[south ? 2 * n - 1 - r : r];
+        const double lon = __dmul_rn((double)j, 360.0 / (double)count);
+        latlon[p] = make_float2((float)__dmul_rn(lat, NPY_DEG2RAD), (float)__dmul_rn(lon, NPY_DEG2RAD));
+    }
+}
+
+int octahedral_args(const char* fn, int n) {
+    AGX_REQUIRE(n >= 1, AGX_ERR_ARG, "%s: the grid number must be >= 1, got %d", fn, n);
+    AGX_REQUIRE(4ll * n * (n + 9ll) <= INT32_MAX, AGX_ERR_ARG, "%s: O%d has %lld points, more than int32 node indices hold",
+                fn, n, 4ll * n * (n + 9ll));
+    return AGX_OK;
+}
+}  // namespace
+
+extern "C" int agx_gaussian_latitudes(int n, double* lat_deg, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    int rc = octahedral_args("agx_gaussian_latitudes", n);
+    if (rc != AGX_OK) return rc;
+    AGX_REQUIRE(lat_deg != nullptr, AGX_ERR_ARG, "agx_gaussian_latitudes: lat_deg is NULL");
+    k_gaussian_latitudes<<<(n + 31) / 32, 32, 0, stream>>>(n, lat_deg);
+    AGX_LAUNCH_OK();
+    agx_note_launch(1);
+    return AGX_OK;
+}
+
+extern "C" int agx_octahedral_nodes(int n, const double* lat_deg, float* latlon, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    int rc = octahedral_args("agx_octahedral_nodes", n);
+    if (rc != AGX_OK) return rc;
+    AGX_REQUIRE(lat_deg != nullptr && latlon != nullptr, AGX_ERR_ARG, "agx_octahedral_nodes: NULL buffer");
+    const int64_t half = 2ll * n * (n + 9);
+    k_octahedral_nodes<<<agx_grid(2 * half, 256, 8), 256, 0, stream>>>(n, half, lat_deg, (float2*)latlon);
+    AGX_LAUNCH_OK();
+    agx_note_launch(1);
+    return AGX_OK;
+}

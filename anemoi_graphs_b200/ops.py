@@ -965,6 +965,26 @@ def healpix_nodes(resolution: int, device=None) -> torch.Tensor:
     return out
 
 
+def gaussian_latitudes(n: int, device=None) -> torch.Tensor:
+    """float64 (2n,) Gaussian latitudes in degrees, north to south: the roots of the Legendre polynomial P_2n
+    (``agx_gaussian_latitudes``).  ValueError for n < 1 or a grid O<n> past int32 node indices."""
+    _cabi.require_cuda()
+    device = torch.device("cuda") if device is None else device
+    out = torch.empty(max(2 * int(n), 0), dtype=torch.float64, device=device)
+    check(load_library().agx_gaussian_latitudes(int(n), ptr(out), current_stream()))
+    return out
+
+
+def octahedral_nodes(n: int, device=None) -> torch.Tensor:
+    """float32 (4n(n+9), 2) (lat, lon) radians of the octahedral reduced Gaussian grid O<n>, north to south and west to
+    east from 0 degrees (``agx_octahedral_nodes``); ``grids.latlon_deg_to_x(*grids.octahedral_grid(n))`` on the device."""
+    lat = gaussian_latitudes(n, device)  # checks n before the output is allocated
+    n = int(n)
+    out = torch.empty((4 * n * (n + 9), 2), dtype=torch.float32, device=lat.device)
+    check(load_library().agx_octahedral_nodes(n, ptr(lat), ptr(out), current_stream()))
+    return out
+
+
 # ----------------------------------------------------------------------------------------------
 # spherical Voronoi cell areas
 # ----------------------------------------------------------------------------------------------

@@ -395,6 +395,18 @@ int agx_multiscale_adj_count(int n_levels, const int32_t* const* nb /*HOST[n_lev
  * independent RING-scheme formulas (oracle/healpix_restated.py).                                             */
 int agx_healpix_nodes(int resolution /*log2 nside*/, float* latlon /*DEV npix*2*/, void* stream);
 
+/* ---- octahedral reduced Gaussian grid O<n> (ReducedGaussianGridNodes of newer releases) ---------------------------
+ * Upstream reads the grid from a downloaded file; O<n> is defined by its construction, which grids.octahedral_grid +
+ * latlon_deg_to_x restate on the host (the oracle).
+ * agx_gaussian_latitudes: the 2n Gaussian latitudes (roots of the Legendre polynomial P_2n) in float64 degrees, north to
+ * south, within 1e-13 degrees of the exact roots; row 2n-1-k is the exact negation of row k.
+ * agx_octahedral_nodes: float32 (lat, lon) radians of the 4n(n+9) points from those latitudes, north to south and west to
+ * east from 0 degrees; row i (1-based from the nearer pole) holds 4i + 16 points at lon = j * (360 / (4i + 16)) degrees.
+ * Bit for bit the oracle's float32 values wherever the latitudes are within float32 rounding (DESIGN section 4).
+ * Both: AGX_ERR_ARG for n < 1, for 4n(n+9) > INT32_MAX and for a NULL pointer.                                    */
+int agx_gaussian_latitudes(int n, double* lat_deg /*DEV 2n*/, void* stream);
+int agx_octahedral_nodes(int n, const double* lat_deg /*DEV 2n*/, float* latlon /*DEV 4n(n+9)*2*/, void* stream);
+
 /* ---- node attribute: spherical Voronoi cell areas (SURVEY section 8f, row N3) -------------------------------
  * Replaces `SphericalVoronoi(points, radius, centre).calculate_areas()` in SphericalAreaWeights.get_raw_values
  * (nodes/attributes.py:199-221), points = latlon_rad_to_cartesian(x) in float32 (generate/transforms.py:106-110).
