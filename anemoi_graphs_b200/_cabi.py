@@ -55,6 +55,9 @@ SIGNATURES = {
     "agx_radius_count": (c_int, [c_void_p, c_void_p, c_int64, c_double, c_void_p, c_void_p]),
     "agx_exclusive_scan": (c_int, [c_void_p, c_int64, c_void_p, POINTER(c_int64), c_void_p]),
     "agx_radius_fill": (c_int, [c_void_p, c_void_p, c_int64, c_double, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+    "agx_radius_cap_counts": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
+    "agx_radius_fill_capped": (c_int, [c_void_p, c_void_p, c_int64, c_double, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+    "agx_radius_select": (c_int, [c_void_p, c_void_p, c_int64, c_double, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "agx_max_positive": (c_int, [c_void_p, c_int64, POINTER(c_double), POINTER(c_int64), c_void_p]),
     "agx_host_reference_rdist": (c_int, [c_void_p, c_void_p, c_int64, c_int, POINTER(c_double)]),
     "agx_order_resolve": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -81,6 +81,7 @@ class GraphCreator:
         walk(self.config.get("nodes", {}))
         walk(self.config.get("edges", []))
         walk(self.config.get("post_processors", []))
+        from .edges.builder import check_max_num_neighbours
         from .edges.builder import check_scale_levels
         from .edges.builder import scale_levels
         from .nodes.builders.from_reduced_gaussian import octahedral_number
@@ -96,6 +97,8 @@ class GraphCreator:
                 k, hops = b.get("num_nearest_neighbours"), b.get("x_hops")
                 if name in ("KNNEdges", "ReversedKNNEdges") and isinstance(k, int) and k > self.MAX_KNN_K:
                     raise NotImplementedError(f"{name}: num_nearest_neighbours = {k} > {self.MAX_KNN_K} is not built")
+                if name in ("CutOffEdges", "ReversedCutOffEdges"):
+                    check_max_num_neighbours(b.get("max_num_neighbours"))
                 if name == "MultiScaleEdges" and isinstance(hops, int) and hops > self.MAX_X_HOPS:
                     raise NotImplementedError(f"MultiScaleEdges: x_hops = {hops} > {self.MAX_X_HOPS} is not built")
                 if name == "MultiScaleEdges" and b.get("scale_resolutions") is not None:

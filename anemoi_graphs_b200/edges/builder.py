@@ -424,6 +424,11 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
         The name of the source mask attribute to filter edge connections.
     target_mask_attr_name : str | None
         The name of the target mask attribute to filter edge connections.
+    max_num_neighbours : int | None
+        At most this many edges per target node: a target with more source nodes within the radius keeps its
+        ``max_num_neighbours`` nearest, exact float64 distance ties at the boundary going to the lower source index.
+        None (default): no cap.  The argument of newer anemoi-graphs releases, whose default is 64 as far as is known;
+        parity with them is unverified (DESIGN.md section 4).
     """
 
     def __init__(
@@ -433,12 +438,17 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
         cutoff_factor: float,
         source_mask_attr_name: str | None = None,
         target_mask_attr_name: str | None = None,
+        max_num_neighbours: int | None = None,
     ):
         super().__init__(source_name, target_name, source_mask_attr_name, target_mask_attr_name)
         assert isinstance(cutoff_factor, (int, float)), "Cutoff factor must be a float"
         assert cutoff_factor > 0, "Cutoff factor must be positive"
+        check_max_num_neighbours(max_num_neighbours)
         self.cutoff_factor = cutoff_factor
-        self.stats = None  # optional CUDA int64[4]: {pairs decided in float64, pairs within 2^-40 of the radius, 0, 0}
+        self.max_num_neighbours = max_num_neighbours
+        # optional CUDA int64[4]: {pairs decided in float64, pairs within 2^-40 of the radius, queries capped at
+        # max_num_neighbours, capped queries with a tie at the boundary}
+        self.stats = None
 
     def get_cutoff_radius(self, graph, mask_attr: torch.Tensor | None = None) -> float:
         """Cut-off radius = reference distance of the query nodes x cut-off factor (edges/builder.py:312-334): the
@@ -468,25 +478,41 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
         )
         ref, qry = self.search_roles(src, dst)
         ref_sel, qry_sel = self.search_roles(src_sel, dst_sel)
+        cap_m = self.max_num_neighbours
+        ref_prov, qry_prov = self.search_roles(*self._row_provs)
+        if cap_m is not None and ref_prov is not None:
+            # the nearest-M pick breaks ties by the numbering of the indexed side: final numbering first (provisional
+            # numbering implies no masks)
+            ref = _device.node_state(self.search_roles(source_nodes, target_nodes)[0]).x
+            self._row_provs = self.search_roles(None, qry_prov)
         nq = int(qry.shape[0])
         sharded_out = _device.sharded_output()
         rank, w = _device.world() if sharded_out else _device.shard_world(nq)
         lo, hi = _device.shard_range(nq, rank, w)
+
+        def count(index, q):
+            """``(offsets, total, cap)``: ``cap`` the keyword arguments ``radius_fill`` takes for query rows [a, b)."""
+            if cap_m is None:
+                return (*index.radius_count(q, self.radius), lambda a, b: {})
+            offsets, total, counts = index.radius_capped(q, self.radius, cap_m)
+            return offsets, total, lambda a, b: {"counts": counts[a:b], "max_neighbours": cap_m}
+
         if sharded_out:
             # this rank's queries only; the blocks stay where they are (global query ids), only the counts travel
             with ops.NeighbourIndex(ref, hint_radius=self.radius) as index:
                 q = qry[lo:hi]
-                offsets, total = index.radius_count(q, self.radius)
+                offsets, total, cap = count(index, q)
                 out = torch.empty((2, total), dtype=torch.int32, device=qry.device)
                 with self.masked_outputs(ref_sel, qry_sel, lo, hi):
-                    index.radius_fill(q, self.radius, offsets, total, out, 0, dst_base=lo, stats=self.stats, swap_rows=rev)
+                    index.radius_fill(q, self.radius, offsets, total, out, 0, dst_base=lo, stats=self.stats, swap_rows=rev,
+                                      **cap(0, hi - lo))  # fmt: skip
             counts = _device.exchange_counts(total, qry.device)
             out = _device.tag_rows(out, *self._row_provs)
             _device.edge_meta(out, create=True).shard = _device.Shard(rank, w, counts)
             return out
         with ops.NeighbourIndex(ref, hint_radius=self.radius) as index:
             q = qry[lo:hi]
-            offsets, total = index.radius_count(q, self.radius)
+            offsets, total, cap = count(index, q)
             masked = src_sel is not None or dst_sel is not None
             if w > 1 and not masked and torch.distributed.get_backend() == "nccl":
                 # uneven blocks: padded equal-block all-gathers, chunk by chunk (device.ChunkedGather); per-chunk pair
@@ -507,7 +533,7 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
                         if mine[c]:
                             # the offsets keep their block-relative values, so the chunk lands at its final columns
                             index.radius_fill(q[a:b], self.radius, offsets[a : b + 1], mine[c], out, base,
-                                              dst_base=lo + a, stats=self.stats, swap_rows=rev)  # fmt: skip
+                                              dst_base=lo + a, stats=self.stats, swap_rows=rev, **cap(a, b))  # fmt: skip
                         marks.append(gather.mark())
                         if c > 0:
                             gather.chunk_done(c - 1, marks[c - 1])
@@ -523,7 +549,7 @@ class CutOffEdges(BaseEdgeBuilder, NodeMaskingMixin):
                 base = sum(counts[:rank])
                 with self.masked_outputs(ref_sel, qry_sel, lo, hi):  # original node indices straight from the kernel
                     index.radius_fill(q, self.radius, offsets, total, out, base, dst_base=lo, stats=self.stats,
-                                      swap_rows=rev)  # fmt: skip
+                                      swap_rows=rev, **cap(0, hi - lo))  # fmt: skip
         if w > 1:
             out = _gather_blocks(out, counts, rank, src_sel is not None or dst_sel is not None)
         return _device.tag_rows(out, *self._row_provs)
@@ -550,9 +576,21 @@ class ReversedCutOffEdges(CutOffEdges):
         The name of the source mask attribute to filter edge connections.
     target_mask_attr_name : str | None
         The name of the target mask attribute to filter edge connections.
+    max_num_neighbours : int | None
+        At most this many edges per SOURCE node (the query side), chosen as for ``CutOffEdges``.  None (default): no cap.
     """
 
     _reversed = True
+
+
+def check_max_num_neighbours(max_num_neighbours) -> None:
+    """The ``max_num_neighbours`` argument of the cut-off builders: None (no cap) or a positive int."""
+    if max_num_neighbours is None:
+        return
+    assert isinstance(max_num_neighbours, int) and not isinstance(max_num_neighbours, bool), (
+        "Maximum number of neighbours must be an integer"
+    )
+    assert max_num_neighbours > 0, "Maximum number of neighbours must be positive"
 
 
 MULTISCALE_MAX_LEVELS = 16  # MS_MAX_LEVELS of the multi-scale edge kernel (agx_mesh.cu)

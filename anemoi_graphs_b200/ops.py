@@ -216,22 +216,60 @@ class NeighbourIndex:
         check(self.lib.agx_exclusive_scan(ptr(counts), nq, ptr(offsets), byref(total), stream))
         return offsets, int(total.value)
 
+    def radius_capped(self, q: torch.Tensor, radius: float, max_neighbours: int) -> tuple[torch.Tensor, int, torch.Tensor]:
+        """Pass 1 of the capped cut-off search: ``(offsets (nq+1,) int64, total, counts (nq,) int32)`` - the offsets
+        and total of at most ``max_neighbours`` pairs per query, and the uncapped counts ``radius_fill`` takes with
+        them."""
+        q = _dev_x(q)
+        nq = int(q.shape[0])
+        counts = torch.empty(nq, dtype=torch.int32, device=q.device)
+        capped = torch.empty(nq, dtype=torch.int32, device=q.device)
+        offsets = torch.empty(nq + 1, dtype=torch.int64, device=q.device)
+        stream = current_stream()
+        with _span("radius_count", nq):
+            check(self.lib.agx_radius_count(self.handle, ptr(q), nq, float(radius), ptr(counts), stream))
+        check(self.lib.agx_radius_cap_counts(ptr(counts), nq, int(max_neighbours), ptr(capped), stream))
+        total = c_int64()
+        check(self.lib.agx_exclusive_scan(ptr(capped), nq, ptr(offsets), byref(total), stream))
+        return offsets, int(total.value), counts
+
     def radius_fill(
         self, q: torch.Tensor, radius: float, offsets: torch.Tensor, total: int, out: torch.Tensor, out_offset: int = 0,
         dst_base: int = 0, stats: torch.Tensor | None = None, swap_rows: bool = False,
+        counts: torch.Tensor | None = None, max_neighbours: int | None = None,
     ) -> torch.Tensor:  # fmt: skip
         """Pass 2: write the ``total`` pairs at column ``out_offset`` of the contiguous (2, E) int32 ``out``; with
-        ``swap_rows`` the queries go to row 0 and the reference points to row 1."""
+        ``swap_rows`` the queries go to row 0 and the reference points to row 1.  With ``max_neighbours`` (and the
+        ``counts`` and ``offsets`` of ``radius_capped``) a query with more candidates keeps its ``max_neighbours``
+        nearest, ties at the boundary to the lower reference index (``agx_radius_select``)."""
         q = _dev_x(q)
         assert out.dim() == 2 and out.shape[0] == 2 and out.dtype == torch.int32 and out.is_contiguous()
         assert 0 <= out_offset and out_offset + total <= out.shape[1]
         if total:
             ref_row, q_row = _row_ptrs(out, out_offset, swap_rows)
+            nq, stream = int(q.shape[0]), current_stream()
+            if max_neighbours is None:
+                with _span("radius_fill", total):
+                    check(
+                        self.lib.agx_radius_fill(
+                            self.handle, ptr(q), nq, float(radius), ptr(offsets), ref_row, q_row, int(dst_base),
+                            ptr(stats), stream,
+                        )
+                    )  # fmt: skip
+                return out
+            assert counts is not None and counts.dtype == torch.int32 and counts.shape == (nq,)
             with _span("radius_fill", total):
                 check(
-                    self.lib.agx_radius_fill(
-                        self.handle, ptr(q), int(q.shape[0]), float(radius), ptr(offsets), ref_row, q_row,
-                        int(dst_base), ptr(stats), current_stream(),
+                    self.lib.agx_radius_fill_capped(
+                        self.handle, ptr(q), nq, float(radius), ptr(counts), int(max_neighbours), ptr(offsets),
+                        ref_row, q_row, int(dst_base), ptr(stats), stream,
+                    )
+                )  # fmt: skip
+            with _span("radius_select", nq):
+                check(
+                    self.lib.agx_radius_select(
+                        self.handle, ptr(q), nq, float(radius), ptr(counts), int(max_neighbours), ptr(offsets),
+                        ref_row, q_row, int(dst_base), ptr(stats), stream,
                     )
                 )  # fmt: skip
         return out

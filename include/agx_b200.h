@@ -142,6 +142,26 @@ int agx_exclusive_scan(const int32_t* counts /*DEV n*/, int64_t n, int64_t* offs
 int agx_radius_fill(const agx_index_t* index, const float* q_latlon /*DEV*/, int64_t nq, double radius,
                     const int64_t* offsets /*DEV nq+1*/, int32_t* out_src /*DEV*/, int32_t* out_dst /*DEV*/,
                     int64_t dst_base, int64_t* stats /*DEV or NULL*/, void* stream);
+/* Capped cut-off search (CutOffEdges(max_num_neighbours = M), M >= 1).  From the counts of agx_radius_count:
+ * agx_radius_cap_counts writes capped[q] = min(counts[q], M); `offsets` below is its exclusive scan.
+ * agx_radius_fill_capped writes every query with counts[q] <= M exactly as agx_radius_fill does and skips the others.
+ * agx_radius_select writes the M slots of each of those others: its M candidates nearest by float64 rdist, ties at the
+ * M-th boundary under the KNN rule (the tie group = the candidates within 2^-40 relative of the M-th smallest rdist;
+ * the ones below it are kept, the group is filled from the lowest reference index), in ascending (rdist, index) order
+ * with the kept group members last, by index.  It stages the candidates of those queries in scratch memory of
+ * 12 bytes per candidate and reads one total back (a stream sync).  stats (optional, DEV int64[4]) of the fill and
+ * the selection together: slots 0 and 1 as agx_radius_fill, += {.., .., capped queries, capped queries with a tie at
+ * the M-th boundary}.                                                                                            */
+int agx_radius_cap_counts(const int32_t* counts /*DEV nq*/, int64_t nq, int max_neighbours, int32_t* capped /*DEV nq*/,
+                          void* stream);
+int agx_radius_fill_capped(const agx_index_t* index, const float* q_latlon /*DEV*/, int64_t nq, double radius,
+                           const int32_t* counts /*DEV nq*/, int max_neighbours, const int64_t* offsets /*DEV nq+1*/,
+                           int32_t* out_src /*DEV*/, int32_t* out_dst /*DEV*/, int64_t dst_base,
+                           int64_t* stats /*DEV or NULL*/, void* stream);
+int agx_radius_select(const agx_index_t* index, const float* q_latlon /*DEV*/, int64_t nq, double radius,
+                      const int32_t* counts /*DEV nq*/, int max_neighbours, const int64_t* offsets /*DEV nq+1*/,
+                      int32_t* out_src /*DEV*/, int32_t* out_dst /*DEV*/, int64_t dst_base,
+                      int64_t* stats /*DEV or NULL*/, void* stream);
 
 /* ---- grid reference distance --------------------------------------------------------------------
  * Replaces `dists[dists > 0].max()` (utils.py:62-63) on the float64 rdist of a k=2 self query
