@@ -50,6 +50,26 @@ void agx_note_order(int binned);  // what the last decision was  // raise the re
         }                                                                                   \
     } while (0)
 
+// One pair of ints per call, zeroed: [0] is the flag a kernel raises on bad input, [1] is free for a count a kernel
+// leaves on the device.  agx_bad_flag_read reads both back with one synchronisation (the agx_mark_nodes pattern), frees
+// them, stores [1] in *second (may be NULL) and returns AGX_ERR_ARG with `msg` if the flag was raised.
+static inline int agx_bad_flag_alloc(int** bad, cudaStream_t stream) {
+    agx_pool_keep_warm();
+    AGX_CUDA_OK(cudaMallocAsync(bad, 2 * sizeof(int), stream));
+    AGX_CUDA_OK(cudaMemsetAsync(*bad, 0, 2 * sizeof(int), stream));
+    return AGX_OK;
+}
+
+static inline int agx_bad_flag_read(int* bad, const char* msg, int* second, cudaStream_t stream) {
+    int host2[2] = {0, 0};
+    int rc = agx_readback(host2, bad, 1, stream);
+    cudaFreeAsync(bad, stream);
+    if (rc) return rc;
+    if (second) *second = host2[1];
+    AGX_REQUIRE(host2[0] == 0, AGX_ERR_ARG, "%s", msg);
+    return AGX_OK;
+}
+
 // The cut-off test of a radius (radians): a pair is inside iff rdist <= rdist_thr = sin^2(radius / 2) (sklearn
 // HaversineDistance64._dist_to_rdist, inclusive).  chord2_thr / margin are the FP32 pre-filter of the searches.  One
 // definition for CutOffEdges (agx_radius_*) and RestrictEdgeLength (agx_restrict_flags): the two agree bit for bit.

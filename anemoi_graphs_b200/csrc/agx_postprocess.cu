@@ -30,23 +30,6 @@ __global__ void __launch_bounds__(256) k_restrict_flags(const int32_t* __restric
     }
 }
 
-// one int per launch, zeroed; read back after the kernel (the agx_mark_nodes pattern)
-static int bad_flag_alloc(int** bad, cudaStream_t stream) {
-    agx_pool_keep_warm();
-    AGX_CUDA_OK(cudaMallocAsync(bad, 2 * sizeof(int), stream));
-    AGX_CUDA_OK(cudaMemsetAsync(*bad, 0, 2 * sizeof(int), stream));
-    return AGX_OK;
-}
-
-static int bad_flag_read(int* bad, const char* what, cudaStream_t stream) {
-    int host2[2] = {0, 0};
-    int rc = agx_readback(host2, bad, 1, stream);
-    cudaFreeAsync(bad, stream);
-    if (rc) return rc;
-    AGX_REQUIRE(host2[0] == 0, AGX_ERR_ARG, "%s: an edge endpoint is outside [0, num_nodes) of its node set", what);
-    return AGX_OK;
-}
-
 extern "C" int agx_restrict_flags(const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, const float* src_latlon,
                                   int64_t n_src_nodes, const float* dst_latlon, int64_t n_dst_nodes, const uint8_t* src_mask,
                                   const uint8_t* dst_mask, double max_radius, uint8_t* keep, void* stream_) {
@@ -61,7 +44,7 @@ extern "C" int agx_restrict_flags(const int32_t* edge_src, const int32_t* edge_d
     AGX_REQUIRE((n_src_nodes == 0 || src_latlon) && (n_dst_nodes == 0 || dst_latlon), AGX_ERR_ARG,
                 "agx_restrict_flags: NULL coordinates");
     int* bad = nullptr;
-    rc = bad_flag_alloc(&bad, stream);
+    rc = agx_bad_flag_alloc(&bad, stream);
     if (rc) return rc;
     k_restrict_flags<<<agx_grid(n_edges, 256, 8), 256, 0, stream>>>(edge_src, edge_dst, n_edges, (const float2*)src_latlon,
                                                                     n_src_nodes, (const float2*)dst_latlon, n_dst_nodes,
@@ -72,7 +55,8 @@ extern "C" int agx_restrict_flags(const int32_t* edge_src, const int32_t* edge_d
         agx_set_error("agx_restrict_flags: kernel launch failed");
         return AGX_ERR_CUDA;
     }
-    return bad_flag_read(bad, "agx_restrict_flags", stream);
+    return agx_bad_flag_read(bad, "agx_restrict_flags: an edge endpoint is outside [0, num_nodes) of its node set", nullptr,
+                             stream);
 }
 
 __global__ void __launch_bounds__(256) k_iota(int32_t* __restrict__ out, int64_t n) {
@@ -91,7 +75,7 @@ extern "C" int agx_sort_edges(const int32_t* key_row, const int32_t* other_row, 
                 (long long)n_key_nodes, (long long)n_other_nodes);
     const int64_t n = n_edges;
     int* bad = nullptr;
-    int rc = bad_flag_alloc(&bad, stream);
+    int rc = agx_bad_flag_alloc(&bad, stream);
     if (rc) return rc;
     unsigned long long* keys = nullptr;  // both key buffers, back to back
     int32_t* vals_alt = nullptr;
@@ -138,7 +122,7 @@ extern "C" int agx_sort_edges(const int32_t* key_row, const int32_t* other_row, 
     cudaFreeAsync(keys, stream);
     cudaFreeAsync(vals_alt, stream);
     cudaFreeAsync(temp, stream);
-    return bad_flag_read(bad, "agx_sort_edges", stream);
+    return agx_bad_flag_read(bad, "agx_sort_edges: an edge endpoint is outside [0, num_nodes) of its node set", nullptr, stream);
 }
 
 // ------------------------------------------------------------------------------------------------

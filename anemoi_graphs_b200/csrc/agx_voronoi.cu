@@ -14,6 +14,9 @@
 // generator can reach the polygon ("security radius").  The polygon's vertices are then re-evaluated in 3-D as
 // normalised cross products of adjacent half-space normals - scipy's facet normals - and the area is scipy's sum of
 // |2 atan2(det[p, v_i, v_i+1], 1 + p.v_i + v_i.v_i+1 + v_i+1.p)| (Van Oosterom - Strackee, _voronoi.pyx).
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_run_length_encode.cuh>
+
 #include "agx_common.cuh"
 
 #include <math.h>
@@ -295,4 +298,113 @@ extern "C" int agx_voronoi_areas_small(const float* latlon, int64_t n, const int
     AGX_LAUNCH_OK();
     agx_note_launch(1);
     return AGX_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// Isolatitude area weights (IsolatitudeAreaWeights of newer releases; DESIGN section 4).  A row is one float32
+// latitude (-0.0 and +0.0 one row); with the distinct latitudes phi_0 > ... > phi_{R-1} in float64, row r is the band
+// between b_r = (phi_{r-1} + phi_r) / 2 and b_{r+1}, b_0 = pi/2 and b_R = -pi/2, and each of its c_r nodes weighs
+//     4 pi cos((b_r + b_{r+1}) / 2) sin((b_r - b_{r+1}) / 2) / c_r
+// (the product form: 2 pi (sin b_r - sin b_{r+1}) cancels near the poles).  Rows come from a radix sort of
+// order-preserving latitude keys and a run-length encoding of the sorted keys; every input takes this one path.
+// ------------------------------------------------------------------------------------------------------------------
+#define ISO_HALF_PI_F_BITS 0x3fc90fdbu  // float32(pi/2) = 1.5707963705 > pi/2: a node at a pole is valid
+
+// uint32 key whose unsigned order is the float order of the latitude; -0.0 and +0.0 give the key of +0.0
+__device__ __forceinline__ uint32_t iso_key(float lat) {
+    const uint32_t u = __float_as_uint(__fadd_rn(lat, 0.0f));
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+__device__ __forceinline__ double iso_lat(uint32_t key) {
+    return (double)__uint_as_float((key & 0x80000000u) ? (key & 0x7fffffffu) : ~key);
+}
+
+__global__ void __launch_bounds__(256) k_iso_keys(const float2* __restrict__ latlon, int64_t n, uint32_t* __restrict__ keys,
+                                                  int* __restrict__ bad) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const float lat = latlon[i].x;
+        if ((__float_as_uint(lat) & 0x7fffffffu) > ISO_HALF_PI_F_BITS) *bad = 1;  // NaN or beyond +-float32(pi/2)
+        keys[i] = iso_key(lat);
+    }
+}
+
+// one thread per row of the sorted distinct keys (ascending latitude: south to north); R = *n_rows on the device
+__global__ void __launch_bounds__(256) k_iso_bands(const uint32_t* __restrict__ row_keys, const int32_t* __restrict__ counts,
+                                                   const int* __restrict__ n_rows, double* __restrict__ row_weight) {
+    const int R = *n_rows;
+    for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < R; r += gridDim.x * blockDim.x) {
+        const double phi = iso_lat(row_keys[r]);
+        const double north = r + 1 < R ? (phi + iso_lat(row_keys[r + 1])) * 0.5 : 1.5707963267948966;
+        const double south = r > 0 ? (iso_lat(row_keys[r - 1]) + phi) * 0.5 : -1.5707963267948966;
+        const double area = __dmul_rn(__dmul_rn(12.566370614359172, cos((north + south) * 0.5)), sin((north - south) * 0.5));
+        row_weight[r] = area / (double)counts[r];
+    }
+}
+
+// one thread per node: its row by binary search among the R distinct keys
+__global__ void __launch_bounds__(256) k_iso_weights(const uint32_t* __restrict__ keys, int64_t n,
+                                                     const uint32_t* __restrict__ row_keys, const int* __restrict__ n_rows,
+                                                     const double* __restrict__ row_weight, double* __restrict__ areas) {
+    const int R = *n_rows;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const uint32_t key = keys[i];
+        int lo = 0, hi = R - 1;  // row_keys[lo] <= key <= row_keys[hi]: every key is one of the row keys
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (row_keys[mid] < key) lo = mid + 1;
+            else hi = mid;
+        }
+        areas[i] = row_weight[lo];
+    }
+}
+
+extern "C" int agx_isolatitude_areas(const float* latlon, int64_t n, double* areas, int32_t* n_rows, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    AGX_REQUIRE(n >= 0 && n < (int64_t)2147483647, AGX_ERR_ARG, "agx_isolatitude_areas: n out of [0, 2^31)");
+    if (n_rows) *n_rows = 0;
+    if (n == 0) return AGX_OK;
+    AGX_REQUIRE(latlon && areas, AGX_ERR_ARG, "agx_isolatitude_areas: NULL buffer");
+    int* flag = nullptr;  // [0] bad latitude, [1] R
+    int rc = agx_bad_flag_alloc(&flag, stream);
+    if (rc) return rc;
+    uint32_t* keys = nullptr;  // node keys, sorted keys, row keys: n each
+    int32_t* counts = nullptr;
+    double* row_weight = nullptr;
+    void* temp = nullptr;
+    cudaError_t e;
+#define ISO_TRY(expr)                                                                                      \
+    if ((e = (expr)) != cudaSuccess) {                                                                     \
+        agx_set_error("%s failed: %s", #expr, cudaGetErrorString(e));                                      \
+        cudaFreeAsync(keys, stream); cudaFreeAsync(counts, stream); cudaFreeAsync(row_weight, stream);     \
+        cudaFreeAsync(temp, stream); cudaFreeAsync(flag, stream);                                          \
+        return AGX_ERR_CUDA;                                                                               \
+    }
+    ISO_TRY(cudaMallocAsync(&keys, 3 * n * sizeof(uint32_t), stream));
+    ISO_TRY(cudaMallocAsync(&counts, n * sizeof(int32_t), stream));
+    ISO_TRY(cudaMallocAsync(&row_weight, n * sizeof(double), stream));
+    uint32_t* sorted = keys + n;
+    uint32_t* row_keys = keys + 2 * n;
+    size_t sort_bytes = 0, rle_bytes = 0;
+    ISO_TRY(cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, keys, sorted, (int)n, 0, 32, stream));
+    ISO_TRY(cub::DeviceRunLengthEncode::Encode(nullptr, rle_bytes, sorted, row_keys, counts, flag + 1, (int)n, stream));
+    size_t temp_bytes = sort_bytes > rle_bytes ? sort_bytes : rle_bytes;
+    ISO_TRY(cudaMallocAsync(&temp, temp_bytes > 0 ? temp_bytes : 16, stream));
+    const int grid = agx_grid(n, 256, 8);
+    k_iso_keys<<<grid, 256, 0, stream>>>((const float2*)latlon, n, keys, flag);
+    ISO_TRY(cudaGetLastError());
+    ISO_TRY(cub::DeviceRadixSort::SortKeys(temp, temp_bytes, keys, sorted, (int)n, 0, 32, stream));
+    ISO_TRY(cub::DeviceRunLengthEncode::Encode(temp, temp_bytes, sorted, row_keys, counts, flag + 1, (int)n, stream));
+    k_iso_bands<<<grid, 256, 0, stream>>>(row_keys, counts, flag + 1, row_weight);
+    ISO_TRY(cudaGetLastError());
+    k_iso_weights<<<grid, 256, 0, stream>>>(keys, n, row_keys, flag + 1, row_weight, areas);
+    ISO_TRY(cudaGetLastError());
+#undef ISO_TRY
+    agx_note_launch(3 + 5 + 2);  // the three kernels; CUB's histogram and four onesweep passes, and its encoding scan
+    cudaFreeAsync(keys, stream);
+    cudaFreeAsync(counts, stream);
+    cudaFreeAsync(row_weight, stream);
+    cudaFreeAsync(temp, stream);
+    return agx_bad_flag_read(flag, "agx_isolatitude_areas: a latitude is NaN or its magnitude exceeds float32(pi/2)", n_rows,
+                             stream);
 }

@@ -165,6 +165,18 @@ class SphericalAreaWeights(BaseNodeAttribute):
         return result
 
 
+class IsolatitudeAreaWeights(BaseNodeAttribute):
+    """Isolatitude area weights (newer anemoi-graphs releases; not in the pinned reference, upstream parity
+    unverified): every node gets the area of its latitude band over the number of nodes in its row - the band bounded
+    by the midpoints to the neighbouring rows and by the poles (``ops.isolatitude_areas``, DESIGN.md section 4).
+    Suits any node set laid out in latitude rows, limited-area ones included."""
+
+    def get_raw_values(self, nodes, **kwargs) -> torch.Tensor:
+        areas, n_rows = ops.isolatitude_areas(_device.node_state(nodes).x)
+        LOGGER.debug("%d nodes in %d latitude rows.", int(areas.shape[0]), n_rows)
+        return areas
+
+
 class BooleanBaseNodeAttribute(BaseNodeAttribute, ABC):
     """Base class for boolean node attributes."""
 

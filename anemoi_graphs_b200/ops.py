@@ -1085,12 +1085,27 @@ def voronoi_areas(x: torch.Tensor, radius: float = 1.0) -> torch.Tensor:
     )
 
 
+def isolatitude_areas(x: torch.Tensor) -> tuple[torch.Tensor, int]:
+    """float64 (n,) isolatitude area weights of a node set and its number of latitude rows (``agx_isolatitude_areas``):
+    every node gets the unit-sphere area of its latitude band - bounded by the midpoints to the neighbouring rows and by
+    the poles - over the number of nodes in its row, a row being one float32 latitude (-0.0 and +0.0 one row).
+    ValueError for a latitude that is NaN or beyond +-float32(pi/2)."""
+    xd = _dev_x(x)
+    n = int(xd.shape[0])
+    areas = torch.empty(n, dtype=torch.float64, device=xd.device)
+    n_rows = c_int32(0)
+    with _span("isolatitude_areas", n):
+        check(load_library().agx_isolatitude_areas(ptr(xd), n, ptr(areas), byref(n_rows), current_stream()))
+    return areas, int(n_rows.value)
+
+
 __all__ = [
     "multiscale_tri_edges_mapped",
     "relabel_rows",
     "output_maps",
     "DeferredEdgeAttributes",
     "voronoi_areas",
+    "isolatitude_areas",
     "HexCells",
     "hex_num_cells",
     "multiscale_adj_edges",

@@ -445,6 +445,17 @@ int agx_voronoi_areas(const float* latlon /*DEV n*2*/, int64_t n, const int32_t*
 int agx_voronoi_areas_small(const float* latlon /*DEV n*2*/, int64_t n, const int32_t* subset /*DEV m or NULL*/, int64_t m,
                             double radius, double* areas /*DEV n*/, int32_t* status /*DEV m*/, void* stream);
 
+/* ---- node attribute: isolatitude area weights (IsolatitudeAreaWeights of newer releases) --------------------------
+ * Not in the pinned reference; the rule this package commits to (DESIGN section 4, upstream parity unverified): a row
+ * is the set of nodes whose float32 latitudes are bit-equal, -0.0 and +0.0 one row.  With the R distinct latitudes
+ * phi_0 > ... > phi_{R-1} in float64, b_0 = pi/2, b_R = -pi/2 and b_r = (phi_{r-1} + phi_r) / 2, every node of row r
+ * weighs 4 pi cos((b_r + b_{r+1}) / 2) sin((b_r - b_{r+1}) / 2) / c_r (float64, unit sphere; c_r nodes in the row), so
+ * the weights sum to 4 pi.  Every input is sorted (radix sort of latitude keys, run-length encoding): no order assumed.
+ * *n_rows (HOST, may be NULL) receives R.  AGX_ERR_ARG for a latitude that is NaN or beyond +-float32(pi/2), for
+ * n outside [0, 2^31) and for a NULL buffer; n = 0 writes nothing.                                                   */
+int agx_isolatitude_areas(const float* latlon /*DEV n*2*/, int64_t n, double* areas /*DEV n*/, int32_t* n_rows /*HOST*/,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif
