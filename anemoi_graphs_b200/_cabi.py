@@ -122,6 +122,10 @@ SIGNATURES = {
         [c_void_p, c_int64, c_void_p, c_int, c_int, c_void_p, c_int64, c_double, c_void_p, c_void_p, c_void_p],
     ),
     "agx_voronoi_areas_small": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_double, c_void_p, c_void_p, c_void_p]),
+    "agx_voronoi_areas_wide": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int, c_double, c_void_p, POINTER(c_int64), c_void_p],
+    ),
     "agx_isolatitude_areas": (c_int, [c_void_p, c_int64, c_void_p, POINTER(c_int32), c_void_p]),
     "agx_healpix_nodes": (c_int, [c_int, c_void_p, c_void_p]),
     "agx_gaussian_latitudes": (c_int, [c_int, c_void_p, c_void_p]),

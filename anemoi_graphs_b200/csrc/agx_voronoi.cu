@@ -301,6 +301,464 @@ extern "C" int agx_voronoi_areas_small(const float* latlon, int64_t n, const int
 }
 
 // ------------------------------------------------------------------------------------------------------------------
+// Wide cells (DESIGN section 4, K9): the cells that k_voronoi_areas leaves open after its 63 nearest neighbours - a
+// coarse generator next to a much finer region, whose nearest neighbours all lie on one side of it - or that have
+// more than VOR_MAXV edges.  No radius sweep: a polygon built from a candidate set C is the true cell of g exactly
+// when no generator h has (h - g) . v > 0 at any of its vertices v (the corners of the initial square included),
+// because the polygon is the convex hull of its vertices.  So, in rounds over the cells still open:
+//   clip   one warp per cell clips the square with C in ascending (float64 rdist, index) order; the polygon lives in
+//          shared memory (VOR_WIDE_CAP edges) and the lanes split each clip's vertices;
+//   query  agx_knn of every vertex against the node set's index, VOR_WIDE_K neighbours;
+//   check  each (vertex, neighbour) pair in float64; the violators that are not candidates yet join C.
+// A cell without a violator whose vertices are certified (below) is final and gets its area as k_voronoi_areas
+// computes it; a cell that still touches the square then is not inside its open hemisphere.
+//
+// Certification of a vertex v: every generator h outside its VOR_WIDE_K nearest is at least as far from v (haversine
+// on the float32 (lat, lon)) as the K-th, a_K.  The float32 generator has |h| <= 1 + 2 VOR_NORM_SLACK and its
+// direction (and v's float32 query point) is within 2 VOR_NORM_SLACK rad of the exact one, so
+//     h . v <= (1 + 2 S) (cos a_K + 2 S sin a_K),   S = VOR_NORM_SLACK;
+// once that is below g . v, no generator outside the list can cut the cell at v.
+// ------------------------------------------------------------------------------------------------------------------
+#define VOR_WIDE_CAP 1024  /* polygon edges a warp holds in shared memory */
+#define VOR_WIDE_NEW 64    /* violators a cell takes per round; any others are found again in the next round */
+#define VOR_WIDE_K 32      /* neighbours of each vertex */
+#define VOR_WIDE_ROUNDS 32
+#define VOR_WIDE_OVERFLOW 5  /* more than VOR_WIDE_CAP edges */
+#define VOR_UNCERTIFIED 6    /* no violator, but VOR_WIDE_K neighbours do not certify a vertex */
+
+struct VorWideSmem {  // two polygons: each clip reads one and writes the other
+    double a[2][VOR_WIDE_CAP], b[2][VOR_WIDE_CAP], c[2][VOR_WIDE_CAP], u[2][VOR_WIDE_CAP], v[2][VOR_WIDE_CAP];
+    int id[2][VOR_WIDE_CAP];
+    unsigned in[VOR_WIDE_CAP / 32];  // bit j: vertex j is inside the clipping half-plane
+};
+
+// generator p (as given, float32-rounded), its unit direction and the tangent frame of k_voronoi_areas
+struct VorFrame {
+    double3 p, ph, e1, e2;
+};
+
+__device__ __forceinline__ VorFrame vor_frame(float2 ll) {
+    VorFrame f;
+    f.p = vor_xyz(ll);
+    f.ph = scale3(f.p, 1.0 / sqrt(dot3(f.p, f.p)));
+    const double3 axis = fabs(f.ph.x) <= fabs(f.ph.y) && fabs(f.ph.x) <= fabs(f.ph.z) ? make_double3(1, 0, 0)
+                         : (fabs(f.ph.y) <= fabs(f.ph.z) ? make_double3(0, 1, 0) : make_double3(0, 0, 1));
+    f.e1 = cross3(f.ph, axis);
+    f.e1 = scale3(f.e1, 1.0 / sqrt(dot3(f.e1, f.e1)));
+    f.e2 = cross3(f.ph, f.e1);
+    return f;
+}
+
+// One warp per open cell t (open[w], w < *n_open).  Candidates cand[off[t], off[t+1]) (self and -1 are skipped);
+// sorted receives them in clip order, key is scratch.  Vertex slots start at off[t] + 4 t (a polygon has at most
+// one edge per candidate plus the four of the square): unit xyz, float32 (lat, lon) to search with, and the
+// generator behind the edge that ends there (-1: the square).  nv[t] = vertex count, 0 if the cell failed.
+__global__ void __launch_bounds__(32) k_voronoi_wide_clip(const float2* __restrict__ latlon, const int32_t* __restrict__ wide,
+                                                          const int32_t* __restrict__ open, const int64_t* __restrict__ n_open,
+                                                          const int64_t* __restrict__ off, const int32_t* __restrict__ cand,
+                                                          double* __restrict__ key, int32_t* __restrict__ sorted,
+                                                          double* __restrict__ vxyz, float2* __restrict__ vll,
+                                                          int32_t* __restrict__ vid, int32_t* __restrict__ nv,
+                                                          unsigned long long* __restrict__ ctl) {
+    extern __shared__ __align__(16) unsigned char vor_smem[];
+    VorWideSmem& S = *reinterpret_cast<VorWideSmem*>(vor_smem);
+    const int lane = threadIdx.x;
+    const unsigned full = 0xffffffffu;
+    const int64_t count = *n_open;
+    for (int64_t w = blockIdx.x; w < count; w += gridDim.x) {
+        const int t = open[w];
+        const int i = wide[t];
+        const float2 gll = latlon[i];
+        const VorFrame F = vor_frame(gll);
+        const int64_t o0 = off[t];
+        const int L = (int)(off[t + 1] - o0);
+        // clip order: ascending (rdist, index), by rank counting (the lists are a few hundred long)
+        for (int j = lane; j < L; j += 32) {
+            const int q = cand[o0 + j];
+            key[o0 + j] = q >= 0 ? agx_rdist64(gll, latlon[q]) : HUGE_VAL;
+        }
+        __syncwarp();
+        for (int j = lane; j < L; j += 32) {
+            const double kj = key[o0 + j];
+            const int ij = cand[o0 + j];
+            int r = 0;
+            for (int x = 0; x < L; ++x) {
+                const double kx = key[o0 + x];
+                const int ix = cand[o0 + x];
+                r += kx < kj || (kx == kj && (ix < ij || (ix == ij && x < j)));
+            }
+            sorted[o0 + r] = ij;
+        }
+        __syncwarp();
+        const double B = VOR_BOX;
+        if (lane < 4) {  // the square of k_voronoi_areas: edge e is u <= B, v <= B, -u <= B, -v <= B
+            S.a[0][lane] = lane == 0 ? 1.0 : (lane == 2 ? -1.0 : 0.0);
+            S.b[0][lane] = lane == 1 ? 1.0 : (lane == 3 ? -1.0 : 0.0);
+            S.c[0][lane] = -B;
+            S.u[0][lane] = lane == 0 || lane == 3 ? B : -B;
+            S.v[0][lane] = lane < 2 ? B : -B;
+            S.id[0][lane] = -1;
+        }
+        __syncwarp();
+        int cur = 0, m = 4, st = VOR_OK;
+        for (int x = 0; x < L; ++x) {
+            const int q = sorted[o0 + x];
+            if (q == i || q < 0) continue;
+            const double3 nrm = sub3(vor_xyz(latlon[q]), F.p);
+            if (dot3(nrm, nrm) == 0.0) { st = VOR_DUPLICATE; break; }
+            const double A = dot3(nrm, F.e1), Bq = dot3(nrm, F.e2), C = dot3(nrm, F.ph);
+            int n_out = 0, first_in = -1;
+            for (int base = 0; base < m; base += 32) {
+                const int j = base + lane;
+                const bool out = j < m && A * S.u[cur][j] + Bq * S.v[cur][j] + C > 0.0;
+                const unsigned bo = __ballot_sync(full, out), bi = __ballot_sync(full, j < m && !out);
+                if (lane == 0) S.in[base >> 5] = bi;
+                n_out += __popc(bo);
+                if (bi && first_in < 0) first_in = base + __ffs(bi) - 1;
+            }
+            __syncwarp();
+            if (n_out == 0 || first_in < 0) continue;  // no vertex cut, or all of them (as vor_clip: keep the polygon)
+            // the edges in the order vor_clip visits them, j = (first_in + s) % m for s = 1..m: an edge inside at both
+            // ends is kept, one that leaves is kept up to the new line and followed by it, one that re-enters closes
+            // the new line (the output just before it) and is kept
+            const int nx = cur ^ 1;
+            int total = 0;
+            for (int base = 0; base < m; base += 32) {
+                const int s = base + lane + 1;
+                int cnt = 0, j = 0;
+                bool in_prev = false, in_cur = false;
+                if (s <= m) {
+                    j = (first_in + s) % m;
+                    const int jp = (j + m - 1) % m;
+                    in_prev = (S.in[jp >> 5] >> (jp & 31)) & 1u;
+                    in_cur = (S.in[j >> 5] >> (j & 31)) & 1u;
+                    cnt = in_cur ? 1 : (in_prev ? 2 : 0);
+                }
+                int incl = cnt;
+                for (int o = 1; o < 32; o <<= 1) {
+                    const int y = __shfl_up_sync(full, incl, o);
+                    if (lane >= o) incl += y;
+                }
+                const int pos = total + incl - cnt;
+                total += __shfl_sync(full, incl, 31);
+                if (cnt && pos + cnt <= VOR_WIDE_CAP) {
+                    const double pa = S.a[cur][j], pb = S.b[cur][j], pc = S.c[cur][j];
+                    S.a[nx][pos] = pa; S.b[nx][pos] = pb; S.c[nx][pos] = pc; S.id[nx][pos] = S.id[cur][j];
+                    if (in_cur) {
+                        S.u[nx][pos] = S.u[cur][j]; S.v[nx][pos] = S.v[cur][j];
+                        if (!in_prev) vor_meet(A, Bq, C, pa, pb, pc, S.u[nx][pos - 1], S.v[nx][pos - 1]);
+                    } else {
+                        vor_meet(pa, pb, pc, A, Bq, C, S.u[nx][pos], S.v[nx][pos]);
+                        S.a[nx][pos + 1] = A; S.b[nx][pos + 1] = Bq; S.c[nx][pos + 1] = C; S.id[nx][pos + 1] = q;
+                    }
+                }
+            }
+            __syncwarp();
+            // the polygon must fit shared memory and the cell's L + 4 vertex slots (in exact arithmetic a clip adds at
+            // most one edge, and the list holds the generator itself)
+            if (total > VOR_WIDE_CAP || total > L + 4) { st = VOR_WIDE_OVERFLOW; break; }
+            cur = nx;
+            m = total;
+        }
+        const int64_t vb = o0 + 4 * (int64_t)t;
+        if (st == VOR_OK) {
+            for (int j = lane; j < m; j += 32) {
+                const double u = S.u[cur][j], v = S.v[cur][j];
+                double3 w = make_double3(F.ph.x + u * F.e1.x + v * F.e2.x, F.ph.y + u * F.e1.y + v * F.e2.y,
+                                         F.ph.z + u * F.e1.z + v * F.e2.z);
+                w = scale3(w, 1.0 / sqrt(dot3(w, w)));
+                vxyz[3 * (vb + j)] = w.x; vxyz[3 * (vb + j) + 1] = w.y; vxyz[3 * (vb + j) + 2] = w.z;
+                vll[vb + j] = make_float2((float)atan2(w.z, hypot(w.x, w.y)), (float)atan2(w.y, w.x));
+                vid[vb + j] = S.id[cur][j];
+            }
+        } else if (lane == 0) {
+            atomicOr(ctl, 1ull << st);
+        }
+        if (lane == 0) nv[t] = st == VOR_OK ? m : 0;
+        __syncwarp();
+    }
+}
+
+// the vertices of the open cells, packed in open-list order for the search: q[voff[t] + j] = vll[off[t] + 4 t + j]
+__global__ void __launch_bounds__(32) k_voronoi_wide_pack(const int32_t* __restrict__ open, int64_t n_open,
+                                                          const int64_t* __restrict__ off, const int64_t* __restrict__ voff,
+                                                          const float2* __restrict__ vll, float2* __restrict__ q) {
+    for (int64_t w = blockIdx.x; w < n_open; w += gridDim.x) {
+        const int t = open[w];
+        const int64_t vb = off[t] + 4 * (int64_t)t;
+        for (int64_t j = threadIdx.x; j < voff[t + 1] - voff[t]; j += 32) q[voff[t] + j] = vll[vb + j];
+    }
+}
+
+// one warp per open cell: every (vertex, neighbour) pair.  A cell with violators stays open - flag[t] = 1,
+// grow[t] = its next candidate count, the violators (at most VOR_WIDE_NEW, first found first) in fresh[w * NEW ..] -
+// and any other cell is final: its area, or a failure bit in ctl[0].  ctl[1] / ctl[2]: largest / total candidate
+// count of the final cells; ctl[6]: cells that stay open and still touch the initial square.  flag, grow and ctl[6]
+// are zero on entry.
+__global__ void __launch_bounds__(32) k_voronoi_wide_check(const float2* __restrict__ latlon, const int32_t* __restrict__ wide,
+                                                           const int32_t* __restrict__ open, int64_t n_open,
+                                                           const int64_t* __restrict__ off, const int32_t* __restrict__ cand,
+                                                           const int64_t* __restrict__ voff, const double* __restrict__ vxyz,
+                                                           const int32_t* __restrict__ vid, const int32_t* __restrict__ nbr,
+                                                           const double* __restrict__ nrd, double radius,
+                                                           double* __restrict__ areas, uint8_t* __restrict__ flag,
+                                                           int32_t* __restrict__ grow, int32_t* __restrict__ fresh,
+                                                           unsigned long long* __restrict__ ctl) {
+    __shared__ int found[VOR_WIDE_NEW];
+    const int lane = threadIdx.x;
+    const unsigned full = 0xffffffffu;
+    const double S2 = 2.0 * VOR_NORM_SLACK;
+    for (int64_t w = blockIdx.x; w < n_open; w += gridDim.x) {
+        const int t = open[w];
+        const int nvt = (int)(voff[t + 1] - voff[t]);
+        if (nvt == 0) continue;  // failed in the clip
+        const int i = wide[t];
+        const double3 p = vor_xyz(latlon[i]);
+        const int64_t o0 = off[t], vb = o0 + 4 * (int64_t)t, q0 = voff[t];
+        const int L = (int)(off[t + 1] - o0);
+        bool boxed = false, uncertified = false;
+        int n_new = 0;
+        for (int base = 0; base < nvt * VOR_WIDE_K; base += 32) {
+            const int idx = base + lane;
+            bool viol = false;
+            int h = -1;
+            if (idx < nvt * VOR_WIDE_K) {
+                const int j = idx / VOR_WIDE_K, r = idx % VOR_WIDE_K;
+                const double3 v = make_double3(vxyz[3 * (vb + j)], vxyz[3 * (vb + j) + 1], vxyz[3 * (vb + j) + 2]);
+                const int ja = vid[vb + j], jb = vid[vb + (j + 1) % nvt];
+                boxed |= ja < 0;
+                h = nbr[(q0 + j) * VOR_WIDE_K + r];
+                if (r == VOR_WIDE_K - 1 && h >= 0) {
+                    const double ck = 1.0 - 2.0 * nrd[(q0 + j) * VOR_WIDE_K + r];
+                    const double sk = sqrt(fmax(0.0, 1.0 - ck * ck));
+                    uncertified |= (1.0 + S2) * (ck + S2 * sk) >= dot3(p, v);
+                }
+                if (h >= 0 && h != i && h != ja && h != jb) {
+                    viol = dot3(sub3(vor_xyz(latlon[h]), p), v) > 0.0;
+                    for (int x = 0; x < L && viol; ++x) viol = cand[o0 + x] != h;
+                    for (int x = 0; x < n_new && viol; ++x) viol = found[x] != h;
+                }
+            }
+            const unsigned vm = __ballot_sync(full, viol);
+            if (vm) {
+                bool keep = false;
+                if (viol) keep = __ffs(__match_any_sync(vm, h)) - 1 == lane;  // one lane per distinct violator
+                const unsigned km = __ballot_sync(full, keep);
+                const int at = n_new + __popc(km & ((1u << lane) - 1u));
+                if (keep && at < VOR_WIDE_NEW) found[at] = h;
+                n_new = min(n_new + __popc(km), VOR_WIDE_NEW);
+                __syncwarp();
+            }
+        }
+        boxed = __any_sync(full, boxed);
+        uncertified = __any_sync(full, uncertified);
+        if (n_new > 0) {
+            for (int x = lane; x < n_new; x += 32) fresh[w * VOR_WIDE_NEW + x] = found[x];
+            if (lane == 0) {
+                flag[t] = 1;
+                grow[t] = L + n_new;
+                if (boxed) atomicAdd(ctl + 6, 1ull);
+            }
+        } else if (lane == 0) {
+            if (boxed) atomicOr(ctl, 1ull << VOR_UNBOUNDED);
+            else if (uncertified) atomicOr(ctl, 1ull << VOR_UNCERTIFIED);
+            else {
+                // k_voronoi_areas' area: 3-D vertices from adjacent half-space normals, Van Oosterom - Strackee sum
+                const double3 ph = scale3(p, 1.0 / sqrt(dot3(p, p)));
+                double area = 0.0;
+                double3 first = make_double3(0, 0, 0), prev = make_double3(0, 0, 0);
+                for (int e = 0; e <= nvt; ++e) {
+                    double3 vtx;
+                    if (e < nvt) {
+                        const double3 n1 = sub3(vor_xyz(latlon[vid[vb + e]]), p);
+                        const double3 n2 = sub3(vor_xyz(latlon[vid[vb + (e + 1) % nvt]]), p);
+                        double3 cw = cross3(n1, n2);
+                        const double wn = sqrt(dot3(cw, cw));
+                        vtx = wn > 0.0 ? scale3(cw, (dot3(cw, ph) < 0.0 ? -1.0 : 1.0) / wn)
+                                       : make_double3(vxyz[3 * (vb + e)], vxyz[3 * (vb + e) + 1], vxyz[3 * (vb + e) + 2]);
+                        if (e == 0) first = vtx;
+                    } else {
+                        vtx = first;
+                    }
+                    if (e > 0) {
+                        const double num = dot3(p, cross3(prev, vtx));
+                        const double den = 1.0 + dot3(p, prev) + dot3(prev, vtx) + dot3(vtx, p);
+                        area += fabs(2.0 * atan2(num, den));
+                    }
+                    prev = vtx;
+                }
+                areas[i] = area * radius * radius;
+                atomicMax(ctl + 1, (unsigned long long)L);
+                atomicAdd(ctl + 2, (unsigned long long)L);
+            }
+        }
+        __syncwarp();
+    }
+}
+
+// next candidate lists: cand2[off2[t] ..] = the clip-ordered list, then the violators
+__global__ void __launch_bounds__(32) k_voronoi_wide_merge(const int32_t* __restrict__ open, int64_t n_open,
+                                                           const int64_t* __restrict__ off, const int32_t* __restrict__ sorted,
+                                                           const int32_t* __restrict__ grow, const int32_t* __restrict__ fresh,
+                                                           const int64_t* __restrict__ off2, int32_t* __restrict__ cand2) {
+    for (int64_t w = blockIdx.x; w < n_open; w += gridDim.x) {
+        const int t = open[w];
+        if (grow[t] == 0) continue;
+        const int L = (int)(off[t + 1] - off[t]);
+        for (int j = threadIdx.x; j < grow[t]; j += 32)
+            cand2[off2[t] + j] = j < L ? sorted[off[t] + j] : fresh[w * VOR_WIDE_NEW + j - L];
+    }
+}
+
+__global__ void k_voronoi_wide_seed_off(int64_t* off, int64_t m, int k) {
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t <= m; t += (int64_t)gridDim.x * blockDim.x) off[t] = t * k;
+}
+
+// ctl[3] = open cells, ctl[4] = vertices, ctl[5] = candidates: the one read-back of a round
+__global__ void k_voronoi_wide_sizes(const int64_t* n_open, const int64_t* voff, const int64_t* off, int64_t m,
+                                     unsigned long long* ctl) {
+    ctl[3] = (unsigned long long)*n_open;
+    ctl[4] = (unsigned long long)voff[m];
+    ctl[5] = (unsigned long long)off[m];
+}
+
+extern "C" int agx_voronoi_areas_wide(const agx_index_t* index, const float* latlon, int64_t n, const int32_t* wide,
+                                      int64_t m, const int32_t* seeds, int k_seed, double radius, double* areas,
+                                      int64_t* stats, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    AGX_REQUIRE(n >= 0 && n < (int64_t)2147483647 && m >= 0 && m <= n && k_seed > 0, AGX_ERR_ARG,
+                "agx_voronoi_areas_wide: bad sizes");
+    AGX_REQUIRE(index && latlon && areas && stats && (m == 0 || (wide && seeds)), AGX_ERR_ARG,
+                "agx_voronoi_areas_wide: NULL buffer");
+    for (int s = 0; s < 6; ++s) stats[s] = 0;
+    if (m == 0) return AGX_OK;
+    AGX_REQUIRE(n > VOR_WIDE_K, AGX_ERR_ARG, "agx_voronoi_areas_wide: needs more than %d generators", VOR_WIDE_K);
+    const size_t smem = sizeof(VorWideSmem);
+    AGX_CUDA_OK(cudaFuncSetAttribute(k_voronoi_wide_clip, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // per-round buffers are (re)allocated to the sizes the round's read-back gives; everything else lives throughout
+    unsigned long long* ctl = nullptr;  // [0] failure bits, [1] max and [2] total candidates of final cells, [3..5] sizes, [6] boxed open cells
+    int64_t *off = nullptr, *off2 = nullptr, *voff = nullptr, *n_open = nullptr;
+    int32_t *open = nullptr, *nv = nullptr, *grow = nullptr, *cand = nullptr, *cand2 = nullptr, *sorted = nullptr;
+    int32_t *fresh = nullptr, *vid = nullptr, *nbr = nullptr;
+    uint8_t* flag = nullptr;
+    double *key = nullptr, *vxyz = nullptr, *nrd = nullptr;
+    float2 *vll = nullptr, *q = nullptr;
+    int rc = AGX_OK;
+    cudaError_t e;
+#define WIDE_TRY(expr)                                                              \
+    if ((e = (expr)) != cudaSuccess) {                                              \
+        agx_set_error("%s failed: %s", #expr, cudaGetErrorString(e));               \
+        rc = AGX_ERR_CUDA;                                                          \
+        goto done;                                                                  \
+    }
+#define WIDE_CALL(expr) \
+    if ((rc = (expr)) != AGX_OK) goto done;
+#define WIDE_FREE(ptr_)                         \
+    do {                                        \
+        if (ptr_) cudaFreeAsync(ptr_, stream);  \
+        ptr_ = nullptr;                         \
+    } while (0)
+    {
+        agx_pool_keep_warm();
+        WIDE_TRY(cudaMallocAsync(&ctl, 8 * sizeof(unsigned long long), stream));
+        WIDE_TRY(cudaMemsetAsync(ctl, 0, 8 * sizeof(unsigned long long), stream));
+        WIDE_TRY(cudaMallocAsync(&off, (m + 1) * sizeof(int64_t), stream));
+        WIDE_TRY(cudaMallocAsync(&voff, (m + 1) * sizeof(int64_t), stream));
+        WIDE_TRY(cudaMallocAsync(&off2, (m + 1) * sizeof(int64_t), stream));
+        WIDE_TRY(cudaMallocAsync(&n_open, sizeof(int64_t), stream));
+        WIDE_TRY(cudaMallocAsync(&open, m * sizeof(int32_t), stream));
+        WIDE_TRY(cudaMallocAsync(&nv, m * sizeof(int32_t), stream));
+        WIDE_TRY(cudaMallocAsync(&grow, m * sizeof(int32_t), stream));
+        WIDE_TRY(cudaMallocAsync(&flag, (m + 3) / 4 * 4, stream));
+        // round 0: every cell open, its candidates the k_seed entries of its row of the last agx_knn pass
+        WIDE_TRY(cudaMemsetAsync(flag, 1, m, stream));
+        WIDE_CALL(agx_compact_flags(flag, m, open, n_open, stream));
+        WIDE_TRY(cudaMemsetAsync(nv, 0, m * sizeof(int32_t), stream));
+        WIDE_TRY(cudaMemsetAsync(grow, 0, m * sizeof(int32_t), stream));
+        WIDE_TRY(cudaMallocAsync(&cand, m * (int64_t)k_seed * sizeof(int32_t), stream));
+        WIDE_TRY(cudaMemcpyAsync(cand, seeds, m * (int64_t)k_seed * sizeof(int32_t), cudaMemcpyDeviceToDevice, stream));
+        k_voronoi_wide_seed_off<<<agx_grid(m + 1, 256, 4), 256, 0, stream>>>(off, m, k_seed);
+        WIDE_TRY(cudaGetLastError());
+        agx_note_launch(1);
+        int64_t n_open_h = m, n_cand_h = m * (int64_t)k_seed;
+        int round = 0;
+        for (;; ++round) {
+            // clip the open cells with their lists
+            WIDE_TRY(cudaMallocAsync(&key, n_cand_h * sizeof(double), stream));
+            WIDE_TRY(cudaMallocAsync(&sorted, n_cand_h * sizeof(int32_t), stream));
+            const int64_t slots = n_cand_h + 4 * m;
+            WIDE_TRY(cudaMallocAsync(&vxyz, 3 * slots * sizeof(double), stream));
+            WIDE_TRY(cudaMallocAsync(&vll, slots * sizeof(float2), stream));
+            WIDE_TRY(cudaMallocAsync(&vid, slots * sizeof(int32_t), stream));
+            WIDE_TRY(cudaMemsetAsync(nv, 0, m * sizeof(int32_t), stream));
+            if (n_open_h > 0) {
+                k_voronoi_wide_clip<<<(unsigned)n_open_h, 32, smem, stream>>>((const float2*)latlon, wide, open, n_open, off,
+                                                                              cand, key, sorted, vxyz, vll, vid, nv, ctl);
+                WIDE_TRY(cudaGetLastError());
+                agx_note_launch(1);
+            }
+            WIDE_CALL(agx_exclusive_scan(nv, m, voff, nullptr, stream));
+            k_voronoi_wide_sizes<<<1, 1, 0, stream>>>(n_open, voff, off, m, ctl);
+            WIDE_TRY(cudaGetLastError());
+            agx_note_launch(1);
+            unsigned long long h[7];
+            WIDE_CALL(agx_readback(h, ctl, 7, stream));
+            n_open_h = (int64_t)h[3];
+            n_cand_h = (int64_t)h[5];
+            const int64_t n_vert = (int64_t)h[4];
+            stats[0] = round;
+            stats[1] = n_open_h;
+            stats[2] = (int64_t)h[1];
+            stats[3] = (int64_t)h[2];
+            stats[4] = (int64_t)h[0];
+            stats[5] = (int64_t)h[6];
+            if (h[0] != 0 || n_open_h == 0 || round == VOR_WIDE_ROUNDS) break;
+            // search the vertices, check every (vertex, neighbour) pair
+            WIDE_TRY(cudaMallocAsync(&q, (n_vert > 0 ? n_vert : 1) * sizeof(float2), stream));
+            WIDE_TRY(cudaMallocAsync(&nbr, (n_vert > 0 ? n_vert : 1) * VOR_WIDE_K * sizeof(int32_t), stream));
+            WIDE_TRY(cudaMallocAsync(&nrd, (n_vert > 0 ? n_vert : 1) * VOR_WIDE_K * sizeof(double), stream));
+            WIDE_TRY(cudaMallocAsync(&fresh, n_open_h * VOR_WIDE_NEW * sizeof(int32_t), stream));
+            const unsigned grid = (unsigned)n_open_h;
+            k_voronoi_wide_pack<<<grid, 32, 0, stream>>>(open, n_open_h, off, voff, vll, q);
+            WIDE_TRY(cudaGetLastError());
+            agx_note_launch(1);
+            if (n_vert > 0)
+                WIDE_CALL(agx_knn(index, (const float*)q, n_vert, VOR_WIDE_K, 0.0, nbr, nullptr, 0, nrd, nullptr, stream));
+            WIDE_TRY(cudaMemsetAsync(flag, 0, m, stream));
+            WIDE_TRY(cudaMemsetAsync(ctl + 6, 0, sizeof(unsigned long long), stream));
+            WIDE_TRY(cudaMemsetAsync(grow, 0, m * sizeof(int32_t), stream));
+            k_voronoi_wide_check<<<grid, 32, 0, stream>>>((const float2*)latlon, wide, open, n_open_h, off, cand, voff, vxyz,
+                                                          vid, nbr, nrd, radius, areas, flag, grow, fresh, ctl);
+            WIDE_TRY(cudaGetLastError());
+            agx_note_launch(1);
+            // the lists of the cells that stay open: count (grow), scan, write
+            WIDE_CALL(agx_exclusive_scan(grow, m, off2, nullptr, stream));
+            WIDE_TRY(cudaMallocAsync(&cand2, (n_cand_h + n_open_h * VOR_WIDE_NEW) * sizeof(int32_t), stream));
+            k_voronoi_wide_merge<<<grid, 32, 0, stream>>>(open, n_open_h, off, sorted, grow, fresh, off2, cand2);
+            WIDE_TRY(cudaGetLastError());
+            agx_note_launch(1);
+            WIDE_CALL(agx_compact_flags(flag, m, open, n_open, stream));
+            n_cand_h += n_open_h * VOR_WIDE_NEW;  // a bound; the read-back of the next round gives the size
+            int64_t* to = off; off = off2; off2 = to;
+            WIDE_FREE(cand);
+            cand = cand2;
+            cand2 = nullptr;
+            WIDE_FREE(key); WIDE_FREE(sorted); WIDE_FREE(vxyz); WIDE_FREE(vll); WIDE_FREE(vid);
+            WIDE_FREE(q); WIDE_FREE(nbr); WIDE_FREE(nrd); WIDE_FREE(fresh);
+        }
+    }
+done:
+    WIDE_FREE(ctl); WIDE_FREE(off); WIDE_FREE(off2); WIDE_FREE(voff); WIDE_FREE(n_open); WIDE_FREE(open);
+    WIDE_FREE(nv); WIDE_FREE(grow); WIDE_FREE(flag); WIDE_FREE(cand); WIDE_FREE(cand2); WIDE_FREE(sorted);
+    WIDE_FREE(key); WIDE_FREE(vxyz); WIDE_FREE(vll); WIDE_FREE(vid); WIDE_FREE(q); WIDE_FREE(nbr); WIDE_FREE(nrd);
+    WIDE_FREE(fresh);
+#undef WIDE_TRY
+#undef WIDE_CALL
+#undef WIDE_FREE
+    return rc;
+}
+
+// ------------------------------------------------------------------------------------------------------------------
 // Isolatitude area weights (IsolatitudeAreaWeights of newer releases; DESIGN section 4).  A row is one float32
 // latitude (-0.0 and +0.0 one row); with the distinct latitudes phi_0 > ... > phi_{R-1} in float64, row r is the band
 // between b_r = (phi_{r-1} + phi_r) / 2 and b_{r+1}, b_0 = pi/2 and b_R = -pi/2, and each of its c_r nodes weighs

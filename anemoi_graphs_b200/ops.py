@@ -1028,12 +1028,19 @@ def octahedral_nodes(n: int, device=None) -> torch.Tensor:
 # ----------------------------------------------------------------------------------------------
 VORONOI_SMALL_N = 64  # up to this many generators unclosed cells go through the exhaustive spherical form
 VORONOI_K = (17, 33, 64)  # neighbours tried in turn (self included): a regular grid's cells close within the first 16
+VORONOI_WIDE_MAX_EDGES = 1024  # polygon capacity of the wide pass (agx_voronoi_areas_wide)
+# what the last voronoi_areas call handed to the wide pass: cells, rounds of vertex queries, candidates per final cell,
+# and the generator ids of those cells (CUDA int32, None when the pass did not run)
+voronoi_wide: dict = {}
 
 
 def voronoi_areas(x: torch.Tensor, radius: float = 1.0) -> torch.Tensor:
     """float64 (n,) areas of the spherical Voronoi cells of a node set - ``SphericalVoronoi(points, radius)
     .calculate_areas()`` of nodes/attributes.py:199-221 - on the device.  Generators whose cell is not closed by
-    their 16 nearest neighbours are retried with 32, then 63."""
+    their 16 nearest neighbours are retried with 32, then 63; the cells still open after that (a coarse generator
+    next to a much finer region) go through the wide pass, which grows each cell's candidates from the neighbours of
+    its vertices (``voronoi_wide`` records what it did)."""
+    voronoi_wide.update(cells=0, rounds=0, max_candidates=0, mean_candidates=0.0, generators=None)
     xd = _dev_x(x)
     n = int(xd.shape[0])
     lib = load_library()
@@ -1061,12 +1068,40 @@ def voronoi_areas(x: torch.Tensor, radius: float = 1.0) -> torch.Tensor:
                 return areas
             if worst == 3:
                 raise ValueError("Duplicate generators present.")  # scipy's message
-            if worst == 4:
-                raise NotImplementedError("a Voronoi cell with more than 32 edges is not built")
             retry = torch.nonzero(status > 0, as_tuple=False).squeeze(1).to(torch.int32)
             subset = retry if subset is None else subset[retry.long()]
             if k == n:
                 break
+        if n > VORONOI_SMALL_N:
+            # cells next to a much finer region: grown from their vertices' neighbours until certified
+            m = int(subset.numel())
+            seeds = knn.view(-1, k)[retry.long()].contiguous()
+            stats = (c_int64 * 6)()
+            with _span("voronoi_areas_wide", m):
+                check(
+                    lib.agx_voronoi_areas_wide(
+                        index.handle, ptr(xd), n, ptr(subset), m, ptr(seeds), k, float(radius), ptr(areas), stats,
+                        stream,
+                    )
+                )  # fmt: skip
+            voronoi_wide.update(
+                cells=m, rounds=stats[0], max_candidates=stats[2], mean_candidates=stats[3] / m, generators=subset
+            )
+            failed = stats[4]
+            if failed & (1 << 3):
+                raise ValueError("Duplicate generators present.")
+            if failed & (1 << 5):
+                raise NotImplementedError(f"a Voronoi cell with more than {VORONOI_WIDE_MAX_EDGES} edges is not built")
+            if failed & (1 << 6):
+                raise NotImplementedError(
+                    "a Voronoi vertex is not certified by its 32 nearest generators (float32 generators denser than "
+                    "~1e-3 rad around it)"
+                )
+            if stats[1] and not stats[5]:
+                raise NotImplementedError(f"{stats[1]} Voronoi cells are still open after {stats[0]} rounds of the wide pass")
+            if not failed and not stats[1]:
+                return areas
+            # a cell still touching the initial square: not inside its open hemisphere (a limited-area set on its own)
     if n <= VORONOI_SMALL_N:
         # a handful of generators: cells wider than a hemisphere do not fit the gnomonic plane - exhaustive form on the
         # sphere (every pair of bisector planes), the reference's range from 4 generators up

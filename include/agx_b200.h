@@ -444,6 +444,22 @@ int agx_voronoi_areas(const float* latlon /*DEV n*2*/, int64_t n, const int32_t*
  * half-space; vertices ordered by azimuth about the generator; the same solid-angle sum.  status as above.        */
 int agx_voronoi_areas_small(const float* latlon /*DEV n*2*/, int64_t n, const int32_t* subset /*DEV m or NULL*/, int64_t m,
                             double radius, double* areas /*DEV n*/, int32_t* status /*DEV m*/, void* stream);
+/* The cells agx_voronoi_areas leaves open after its k = 64 pass (status 1, 2 or 4) of a set whose cells all lie in
+ * the open hemisphere of their generator (DESIGN section 4, K9): wide[t] (t < m) are their generator ids, seeds[t *
+ * k_seed ..] the candidates each starts with (row 0 of that pass's agx_knn, self included), index the agx_index over
+ * the same n generators.  In rounds: one warp clips the cell with its candidates (up to 1024 edges in shared memory),
+ * agx_knn searches 32 neighbours of every vertex, and each neighbour h with (h - g) . v > 0 at a vertex v joins the
+ * candidates; a cell without one is final once every vertex is certified (no generator beyond the 32 can reach it).
+ * areas[wide[t]] is written for every final cell.  stats (HOST int64[6]) = {rounds of queries, cells still open after
+ * 32 rounds, largest candidate list of a final cell, candidates summed over the final cells, failure bits 1 << s, cells
+ * still open that touch the initial square}:
+ * s = 3 duplicate generators, 5 a cell with more than 1024 edges (or, through rounding, more than its candidates
+ * + 4), 2 a cell touching the initial square without a
+ * violator (not inside its open hemisphere), 6 a vertex the 32 neighbours do not certify.  One stream synchronisation
+ * per round.  AGX_ERR_ARG for NULL buffers, m < 0 or m > n, n past int32, k_seed < 1 and n <= 32 with m > 0.      */
+int agx_voronoi_areas_wide(const agx_index_t* index, const float* latlon /*DEV n*2*/, int64_t n,
+                           const int32_t* wide /*DEV m*/, int64_t m, const int32_t* seeds /*DEV m*k_seed*/, int k_seed,
+                           double radius, double* areas /*DEV n*/, int64_t* stats /*HOST 6*/, void* stream);
 
 /* ---- node attribute: isolatitude area weights (IsolatitudeAreaWeights of newer releases) --------------------------
  * Not in the pinned reference; the rule this package commits to (DESIGN section 4, upstream parity unverified): a row
