@@ -75,6 +75,10 @@ SIGNATURES = {
         c_int,
         [c_int, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int64), c_void_p, c_int64, c_void_p],
     ),
+    "agx_edges_to_csr": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, POINTER(c_int64), c_void_p],
+    ),
     "agx_set_output_maps": (None, [c_void_p, c_void_p]),
     "agx_concat_edges": (
         c_int,

@@ -650,6 +650,43 @@ def sort_permutation(key_row: torch.Tensor, other_row: torch.Tensor, n_key_nodes
     return perm
 
 
+CSR_VALUE_KINDS = {None: 0, torch.float32: 1, torch.bool: 2}
+
+
+def edges_to_csr(edge_index: torch.Tensor, n_dst_nodes: int, n_src_nodes: int,
+                 values: torch.Tensor | None = None) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:  # fmt: skip
+    """CUDA ``(indptr int64 (n_dst + 1,), indices int32 (nnz,), data (nnz,))``: the canonical CSR of the targets x
+    sources matrix ``M[edge_index[1, e], edge_index[0, e]] += values[e]`` of the CUDA int32 (2, E) ``edge_index``
+    (``agx_sort_edges`` by (target, source), then ``agx_edges_to_csr``; one read-back).  ``values``: CUDA float32 or
+    bool (E,), or None for float32 ones; duplicates are summed in column order (bool: OR).  ValueError for an endpoint
+    outside its node set and for E >= 2^31."""
+    assert edge_index.is_cuda and edge_index.dtype == torch.int32 and edge_index.dim() == 2 and edge_index.shape[0] == 2
+    edge_index = edge_index.contiguous()
+    n = int(edge_index.shape[1])
+    if n >= 2**31:
+        raise ValueError(f"edges_to_csr: {n} edges; an edge set must have fewer than 2^31 edges")
+    dtype = torch.float32 if values is None else values.dtype
+    assert values is None or (values.is_cuda and values.dtype in CSR_VALUE_KINDS and values.is_contiguous() and values.shape == (n,))
+    perm = sort_permutation(edge_index[1], edge_index[0], n_dst_nodes, n_src_nodes, descending=False)
+    dev = edge_index.device
+    indptr = torch.empty(int(n_dst_nodes) + 1, dtype=torch.int64, device=dev)
+    indices = torch.empty(n, dtype=torch.int32, device=dev)
+    data = torch.empty(n, dtype=dtype, device=dev)
+    nnz = c_int64(0)
+    with _span("edges_to_csr", n):
+        check(
+            load_library().agx_edges_to_csr(
+                ptr(edge_index[0]), ptr(edge_index[1]), n, int(n_dst_nodes), ptr(perm), ptr(values),
+                CSR_VALUE_KINDS[None if values is None else dtype], ptr(indptr), ptr(indices), ptr(data), byref(nnz),
+                current_stream(),
+            )
+        )  # fmt: skip
+    m = int(nnz.value)
+    if m < n:  # duplicate pairs: keep only the nnz entries
+        indices, data = indices[:m].clone(), data[:m].clone()
+    return indptr, indices, data
+
+
 def gather_rows(pairs: list[tuple[torch.Tensor, torch.Tensor]], index: torch.Tensor) -> None:
     """``dst[j] = src[index[j]]`` along dim 0 for every (src, dst) pair of contiguous CUDA tensors of one dtype and row
     shape, eight pairs per launch (``agx_gather_edge_columns``)."""

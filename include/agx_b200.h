@@ -219,6 +219,21 @@ int agx_gather_edge_columns(int n_arrays, const void* const* src /*HOST n_arrays
                             void* const* dst /*HOST n_arrays x DEV*/, const int64_t* row_bytes /*HOST n_arrays*/,
                             const int32_t* index /*DEV n_index*/, int64_t n_index, void* stream);
 
+/* ---- edge set as a sparse matrix (the export_to_sparse command of newer releases, as far as is known) -----------------
+ * agx_edges_to_csr: the canonical CSR of the (n_dst_nodes x n_src_nodes) matrix M[dst, src] += v_e over the E columns,
+ * rows = targets (the reference's get_adjacency_matrix layout, edges/builder.py:63): indptr (n_dst + 1 int64), indices
+ * (int32 sources, ascending within a row) and data; duplicate (dst, src) pairs are summed in column order.  perm must be
+ * agx_sort_edges(key = edge_dst, other = edge_src, ascending) of the same rows, which checks the endpoints.
+ * value_kind 0: v_e = 1 (values not read, data float32); 1: values / data float32, a run summed left to right from its
+ * first value in round-to-nearest adds; 2: values / data bytes, non-zero = true, a run is their OR (written as 0 / 1).
+ * indices and data have room for E entries; the first *nnz (HOST, one read-back) are written.  Scratch: 9 bytes per
+ * edge.  AGX_ERR_ARG for E >= 2^31, n_dst_nodes >= 2^31, edges into an empty target set, an unknown value_kind or a
+ * NULL buffer; E = 0 writes indptr = 0 and *nnz = 0 without a synchronisation.                                      */
+int agx_edges_to_csr(const int32_t* edge_src /*DEV E*/, const int32_t* edge_dst /*DEV E*/, int64_t n_edges,
+                     int64_t n_dst_nodes, const int32_t* perm /*DEV E*/, const void* values /*DEV E or NULL*/, int value_kind,
+                     int64_t* indptr /*DEV n_dst + 1*/, int32_t* indices /*DEV E*/, void* data /*DEV E*/,
+                     int64_t* nnz /*HOST*/, void* stream);
+
 /* ---- masked node sets -------------------------------------------------------------------------------------
  * NodeMaskingMixin.undo_masking (edges/builder.py:176-193: compact indices of the row-selected coordinates mapped back
  * to node indices through a python dict + np.vectorize) fused into the searches' writes: while maps are set (thread-
