@@ -19,7 +19,7 @@ CSRC = PKG / "csrc"
 LIB_DIR = PKG / "lib"
 LIB_PATH = LIB_DIR / "libagx_b200.so"
 OBJ_DIR = LIB_DIR / "obj"
-SOURCES = ["agx_util.cu", "agx_index.cu", "agx_knn.cu", "agx_radius.cu", "agx_attrs.cu", "agx_mesh.cu", "agx_hex.cu", "agx_voronoi.cu", "agx_concat.cu", "agx_postprocess.cu", "agx_sparse.cu", "agx_group_norm.cu"]
+SOURCES = ["agx_util.cu", "agx_index.cu", "agx_knn.cu", "agx_radius.cu", "agx_attrs.cu", "agx_mesh.cu", "agx_hex.cu", "agx_voronoi.cu", "agx_concat.cu", "agx_postprocess.cu", "agx_sparse.cu", "agx_spmm.cu", "agx_group_norm.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",

@@ -79,6 +79,7 @@ SIGNATURES = {
         c_int,
         [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, POINTER(c_int64), c_void_p],
     ),
+    "agx_csr_spmm": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "agx_set_output_maps": (None, [c_void_p, c_void_p]),
     "agx_concat_edges": (
         c_int,

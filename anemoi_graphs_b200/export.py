@@ -10,6 +10,7 @@ int64 ``indptr``, int32 ``indices`` ascending within each row, duplicate pairs s
 
 The CSR arrays are built on the GPU (``ops.edges_to_csr``: ``agx_sort_edges`` + ``agx_edges_to_csr``).  A
 device-resident graph gets a CUDA ``torch.sparse_csr_tensor``; a host-resident one a ``scipy.sparse.csr_matrix``.
+``EdgeSetOperator`` keeps the CUDA arrays and applies the matrix to node fields (``ops.csr_spmm``: ``agx_csr_spmm``).
 """
 
 from __future__ import annotations
@@ -17,6 +18,7 @@ from __future__ import annotations
 import logging
 import warnings
 from pathlib import Path
+from typing import NamedTuple
 
 import torch
 
@@ -54,6 +56,25 @@ def edge_set_to_sparse(graph, edges_name, edge_attribute_name: str | None = None
     outside its node set, ``NotImplementedError`` for a sharded block of a device-resident graph, ``KeyError`` for an
     edge set or attribute the graph does not have.
     """
+    csr = _device_csr(graph, edges_name, edge_attribute_name)
+    if csr.on_device:
+        return torch.sparse_csr_tensor(csr.indptr.to(torch.int32), csr.indices, csr.data, size=csr.shape, check_invariants=False)
+    from scipy.sparse import csr_matrix
+
+    return csr_matrix((csr.data.cpu().numpy(), csr.indices.cpu().numpy(), csr.indptr.cpu().numpy()), shape=csr.shape)
+
+
+class _DeviceCSR(NamedTuple):
+    name: tuple[str, str, str]
+    shape: tuple[int, int]  # (num target nodes, num source nodes)
+    indptr: torch.Tensor
+    indices: torch.Tensor
+    data: torch.Tensor
+    on_device: bool  # edge_index lives on the GPU
+
+
+def _device_csr(graph, edges_name, edge_attribute_name: str | None) -> _DeviceCSR:
+    """The CUDA CSR arrays of ``edge_set_to_sparse``, with its checks."""
     name = _edge_type(edges_name)
     if name not in graph.edge_types:
         raise KeyError(f"The graph has no edge set {name}; it has {graph.edge_types}.")
@@ -68,11 +89,59 @@ def edge_set_to_sparse(graph, edges_name, edge_attribute_name: str | None = None
     _device.flush()  # every node set in its final numbering, every pending copy and collective complete
     values = None if values is None else _device.to_device(values)
     indptr, indices, data = ops.edges_to_csr(_device.to_device(edge_index, torch.int32), n_dst, n_src, values)
-    if edge_index.is_cuda:
-        return torch.sparse_csr_tensor(indptr.to(torch.int32), indices, data, size=(n_dst, n_src), check_invariants=False)
-    from scipy.sparse import csr_matrix
+    return _DeviceCSR(name, (n_dst, n_src), indptr, indices, data, bool(edge_index.is_cuda))
 
-    return csr_matrix((data.cpu().numpy(), indices.cpu().numpy(), indptr.cpu().numpy()), shape=(n_dst, n_src))
+
+class EdgeSetOperator:
+    """The matrix of one edge set (``edge_set_to_sparse``) as an operator on node fields: ``op(x)`` maps a field on
+    the source nodes to one on the target nodes, ``y[t] = sum over the entries (t, s) of M[t, s] * x[s]``.  With
+    ``GaussianDistanceWeights`` on a KNN edge set the rows sum to 1 and ``op`` interpolates.
+
+    The CSR is built once on the GPU (``ops.edges_to_csr``) and kept there; every call is one ``agx_csr_spmm``.
+    Each element of ``y`` is a float32 sum over its row in ascending source order, ``acc = fmaf(M[t, s], x[s], acc)``
+    from +0, rounded once to x's dtype (float32 or bfloat16): bit-identical from call to call, and between host- and
+    device-resident graphs.  An empty row gives +0; NaN and inf reach only the rows that reference them.
+
+    Attributes
+    ----------
+    shape : tuple[int, int]
+        ``(num_nodes[target], num_nodes[source])``.
+
+    Raises ``ValueError`` for a bool attribute (a bool matrix is not an operator) and for the attribute errors of
+    ``edge_set_to_sparse``, ``KeyError`` for an edge set or attribute the graph does not have, ``NotImplementedError``
+    for a sharded block of a device-resident graph.
+    """
+
+    def __init__(self, graph, edges_name, edge_attribute_name: str | None = None) -> None:
+        csr = _device_csr(graph, edges_name, edge_attribute_name)
+        if csr.data.dtype == torch.bool:
+            raise ValueError(
+                f"The edge attribute '{edge_attribute_name}' of {csr.name} is bool: a bool matrix is not an operator; "
+                "use a float32 attribute."
+            )
+        self.name = csr.name
+        self.shape = csr.shape
+        self._indptr, self._indices, self._data = csr.indptr, csr.indices, csr.data
+
+    def __call__(self, x: torch.Tensor) -> torch.Tensor:
+        """``M x`` for a float32 or bfloat16 field ``x`` of shape (num_nodes[source], F) or (num_nodes[source],), on
+        the GPU or the host; ``y`` has shape (num_nodes[target], F) or (num_nodes[target],), x's dtype, and lives
+        where x lives (a host x is uploaded and the result copied back).  ValueError for an x of another dtype, of more
+        than two dimensions, or whose first dimension is not num_nodes[source]."""
+        if x.dim() not in (1, 2):
+            raise ValueError(f"{self.name}: a node field has shape (N,) or (N, F), got {tuple(x.shape)}.")
+        if x.dtype not in ops.SPMM_DTYPES:
+            raise ValueError(f"{self.name}: a node field must be float32 or bfloat16, got {x.dtype}.")
+        if x.shape[0] != self.shape[1]:
+            raise ValueError(f"{self.name}: x has {x.shape[0]} rows, the source node set has {self.shape[1]} nodes.")
+        y = ops.csr_spmm(self._indptr, self._indices, self._data, x.to(self._indptr.device), self.shape[0])
+        return y.to(x.device)
+
+
+def apply_edge_set(graph, edges_name, x: torch.Tensor, edge_attribute_name: str | None = None) -> torch.Tensor:
+    """``EdgeSetOperator(graph, edges_name, edge_attribute_name)(x)``: one field through an edge set's matrix.  To
+    apply one edge set to several fields, build the operator once."""
+    return EdgeSetOperator(graph, edges_name, edge_attribute_name)(x)
 
 
 def _edge_type(name) -> tuple[str, str, str]:

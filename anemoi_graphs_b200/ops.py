@@ -687,6 +687,36 @@ def edges_to_csr(edge_index: torch.Tensor, n_dst_nodes: int, n_src_nodes: int,
     return indptr, indices, data
 
 
+SPMM_DTYPES = {torch.float32: 0, torch.bfloat16: 1}  # AGX_SPMM_FLOAT32, AGX_SPMM_BFLOAT16
+
+
+def csr_spmm(indptr: torch.Tensor, indices: torch.Tensor, data: torch.Tensor, x: torch.Tensor, n_rows: int) -> torch.Tensor:
+    """``y = M x`` for the CSR ``(indptr, indices, data)`` of ``edges_to_csr`` (CUDA int64 / int32 / float32) and the
+    CUDA float32 or bfloat16 field ``x`` of shape (n_cols, F) or (n_cols,): ``y[t, f]`` is the float32 sum, left to
+    right in CSR order, of ``fmaf(data[j], x[indices[j], f], acc)`` from +0, rounded once to x's dtype
+    (``agx_csr_spmm``; one read-back, the index check).  ``y`` has shape (n_rows, F) or (n_rows,) and x's dtype.
+    ValueError for an index outside [0, n_cols)."""
+    assert indptr.is_cuda and indptr.dtype == torch.int64 and indptr.shape == (int(n_rows) + 1,)
+    assert indices.is_cuda and indices.dtype == torch.int32 and data.is_cuda and data.dtype == torch.float32
+    assert indices.dim() == 1 and indices.shape == data.shape
+    assert x.is_cuda and x.dtype in SPMM_DTYPES and x.dim() in (1, 2)
+    x = x.contiguous()
+    n_features = int(x.shape[1]) if x.dim() == 2 else 1
+    y = torch.empty((int(n_rows), *x.shape[1:]), dtype=x.dtype, device=x.device)
+    if y.numel() == 0:
+        return y
+    if indices.numel() == 0:  # no entries: every row is empty
+        return y.zero_()
+    with _span("csr_spmm", int(indices.numel()) * n_features):
+        check(
+            load_library().agx_csr_spmm(
+                ptr(indptr), ptr(indices), ptr(data), int(n_rows), int(x.shape[0]), ptr(x), n_features, SPMM_DTYPES[x.dtype],
+                ptr(y), current_stream(),
+            )
+        )  # fmt: skip
+    return y
+
+
 def gather_rows(pairs: list[tuple[torch.Tensor, torch.Tensor]], index: torch.Tensor) -> None:
     """``dst[j] = src[index[j]]`` along dim 0 for every (src, dst) pair of contiguous CUDA tensors of one dtype and row
     shape, eight pairs per launch (``agx_gather_edge_columns``)."""

@@ -234,6 +234,22 @@ int agx_edges_to_csr(const int32_t* edge_src /*DEV E*/, const int32_t* edge_dst 
                      int64_t* indptr /*DEV n_dst + 1*/, int32_t* indices /*DEV E*/, void* data /*DEV E*/,
                      int64_t* nnz /*HOST*/, void* stream);
 
+/* ---- edge set as an operator: y = M x for the CSR of agx_edges_to_csr (export.EdgeSetOperator) -------------------
+ * agx_csr_spmm: out[t, f] = sum over the entries j of row t, in CSR order, of data[j] * x[indices[j], f], for the
+ * n_rows x n_cols CSR (indptr, indices, data) and the row-major n_cols x n_features field x.  Each element is one
+ * float32 sum, acc = fmaf(data[j], x_j, acc) from acc = +0, left to right; an empty row gives +0.  dtype
+ * AGX_SPMM_FLOAT32: x and out float32; AGX_SPMM_BFLOAT16: x and out bf16 (raw 16-bit words), x widened exactly and
+ * the sum rounded once to nearest even.  No atomics: the result is bit-identical from run to run.  indptr must be a
+ * CSR row pointer (non-decreasing, indptr[0] = 0, indptr[n_rows] = the length of indices and data).  x and out may
+ * have any alignment of their elements.  One synchronisation (the index check).  AGX_ERR_ARG for a NULL buffer, a
+ * negative size, n_cols >= 2^31, an unknown dtype, a buffer not aligned to its elements and an index outside
+ * [0, n_cols) (never read); n_rows = 0 or n_features = 0 writes nothing and launches nothing.                    */
+#define AGX_SPMM_FLOAT32 0
+#define AGX_SPMM_BFLOAT16 1
+int agx_csr_spmm(const int64_t* indptr /*DEV n_rows + 1*/, const int32_t* indices /*DEV nnz*/, const float* data /*DEV nnz*/,
+                 int64_t n_rows, int64_t n_cols, const void* x /*DEV n_cols x n_features*/, int64_t n_features, int dtype,
+                 void* out /*DEV n_rows x n_features*/, void* stream);
+
 /* ---- masked node sets -------------------------------------------------------------------------------------
  * NodeMaskingMixin.undo_masking (edges/builder.py:176-193: compact indices of the row-selected coordinates mapped back
  * to node indices through a python dict + np.vectorize) fused into the searches' writes: while maps are set (thread-
